@@ -1904,6 +1904,15 @@ public:
         return touching;
     }
 
+    // b2DistanceProxy::Set of body b's shape (circle: its centre and radius; box: its 4 vertices and the polygon skin)
+    __device__ __forceinline__ Prox body_proxy(int b) {
+        Prox pb;
+        float hx = B(BF_HX, b), hy = B(BF_HY, b);
+        if (Bi(BF_FLAGS, b) & BFL_CIRCLE) { pb.count = 1; pb.radius = hx; pb.v[0] = mk(0.0f, 0.0f); pb.v[1] = pb.v[2] = pb.v[3] = pb.v[0]; }
+        else { pb.count = 4; pb.radius = RB_POLY_RADIUS; pb.v[0] = mk(-hx, -hy); pb.v[1] = mk(hx, -hy); pb.v[2] = mk(hx, hy); pb.v[3] = mk(-hx, hy); }
+        return pb;
+    }
+
     __device__ __forceinline__ void body_advance(int b, float alpha) {
         float alpha0 = B(BF_ALPHA0, b);
         float beta = (alpha - alpha0) / (1.0f - alpha0);
@@ -1941,10 +1950,7 @@ public:
             B(BF_C0X, b) = sw.c0.x; B(BF_C0Y, b) = sw.c0.y; B(BF_A0, b) = sw.a0; B(BF_ALPHA0, b) = alpha0;
         }
         V2 ev[2] = { mk(__ldg(&ter->v1x[e]), __ldg(&ter->v1y[e])), mk(__ldg(&ter->v2x[e]), __ldg(&ter->v2y[e])) };
-        Prox pb;
-        float hx = B(BF_HX, b), hy = B(BF_HY, b);
-        if (Bi(BF_FLAGS, b) & BFL_CIRCLE) { pb.count = 1; pb.radius = hx; pb.v[0] = mk(0.0f, 0.0f); pb.v[1] = pb.v[2] = pb.v[3] = pb.v[0]; }
-        else { pb.count = 4; pb.radius = RB_POLY_RADIUS; pb.v[0] = mk(-hx, -hy); pb.v[1] = mk(hx, -hy); pb.v[2] = mk(hx, hy); pb.v[3] = mk(-hx, hy); }
+        Prox pb = body_proxy(b);
         float t;
         bool touching = time_of_impact(ev, pb, sw, t);
         float alpha = 1.0f;

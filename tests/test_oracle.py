@@ -12,6 +12,7 @@ import json
 import math
 import os
 import random
+import sys
 
 import numpy as np
 import pytest
@@ -172,9 +173,16 @@ def test_sincos_modes_agree_over_100_ticks():
 
 
 def test_portable_float_sincos_is_accurate():
-    """rot_set mode 0 against float64 math over a wide angle range (via a free-spinning body's cached rotation is
-    not exposed, so the kernel is restated here in numpy float32 with the same operation order)."""
-    a = np.concatenate([np.linspace(-40, 40, 200001), np.linspace(-7000, 7000, 100001)]).astype(F32)
+    """rot_set mode 0 (the float kernel, used for |a| < 65536) restated in numpy float32 with the same operation order, against
+    float64 math over the whole range it serves. The restatement equals the device function bit for bit (the CPU build of
+    tests/probe). Its error grows with the quadrant count: 7.7e-8 below 8192, up to 9.6e-7 between 8192 and 65536
+    (measured on 4e6 random angles per band; tests/test_device_geometry.py states the same bounds for the device function)."""
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "probe"))
+    import probe
+    rng = np.random.default_rng(0)
+    small = np.concatenate([np.linspace(-40, 40, 200001), np.linspace(-8191.99, 8191.99, 100001), rng.uniform(-8192, 8192, 200000)])
+    large = rng.uniform(8192, 65535.99, 400000) * rng.choice([-1.0, 1.0], 400000)
+    a = np.concatenate([small, large]).astype(F32)
     kf = np.floor(a * F32(0.636619747) + F32(0.5)).astype(F32)
     r = ((a - kf * F32(1.5703125)) - kf * F32(4.837512969970703125e-4)) - kf * F32(7.54978995489188216e-8)
     z = r * r
@@ -183,8 +191,12 @@ def test_portable_float_sincos_is_accurate():
     n = kf.astype(np.int64) & 3
     s = np.where(n == 0, sr, np.where(n == 1, cr, np.where(n == 2, -sr, -cr)))
     c = np.where(n == 0, cr, np.where(n == 1, -sr, np.where(n == 2, -cr, sr)))
-    assert np.abs(s - np.sin(a.astype(np.float64))).max() < 2.5e-7
-    assert np.abs(c - np.cos(a.astype(np.float64))).max() < 2.5e-7
+    ds, dc = probe.rot_set(a)
+    assert np.array_equal(s.view(np.uint32), ds.view(np.uint32)) and np.array_equal(c.view(np.uint32), dc.view(np.uint32))
+    err = np.maximum(np.abs(s - np.sin(a.astype(np.float64))), np.abs(c - np.cos(a.astype(np.float64))))
+    band = np.abs(a) < 8192
+    assert err[band].max() < 1.0e-7
+    assert err[~band].max() < 1.2e-6
 
 
 def test_counters_and_threads_are_consistent():
