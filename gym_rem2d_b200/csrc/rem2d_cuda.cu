@@ -56,48 +56,6 @@ __global__ void roots_kernel(const float* state, const int* __restrict__ lane_cr
     alive[c] = __float_as_int(g[S_ALIVE * 32]);
 }
 
-// ---- survivor compaction between tick phases of the evaluate path -------------------------------------------------
-// plan: every lane whose episode ended (dead, tick budget reached, or a capacity overflow) writes its result; every
-// survivor gets a dense destination slot (order within the class is irrelevant for results).
-__global__ void compact_plan_kernel(const float* state, const int* __restrict__ lane_creature, int n_lanes, int words, int max_ticks,
-                                    double* fitness, int* ticks, int* alive, int* status, int* dst_slot, int* n_alive) {
-    int gl = blockIdx.x * blockDim.x + threadIdx.x;
-    if (gl >= n_lanes) return;
-    int c = lane_creature[gl];
-    int dst = -1;
-    if (c >= 0) {
-        const float* g = state + (size_t)(gl >> 5) * words * 32 + (gl & 31);
-        int a = __float_as_int(g[S_ALIVE * 32]), t = __float_as_int(g[S_TICKS * 32]), st = __float_as_int(g[S_STATUS * 32]);
-        if (!a || st || t >= max_ticks) {
-            fitness[c] = __hiloint2double(__float_as_int(g[S_FIT_HI * 32]), __float_as_int(g[S_FIT_LO * 32]));
-            ticks[c] = t; alive[c] = a; status[c] = st;
-        } else dst = atomicAdd(n_alive, 1);
-    }
-    dst_slot[gl] = dst;
-}
-// copy: one CTA per source lane moves the creature's column into its slot of the other (ping-pong) buffer
-__global__ void compact_copy_kernel(const float* src, float* dst, const int* __restrict__ dst_slot, const int* __restrict__ src_creature,
-                                    int* dst_creature, int words) {
-    int gl = blockIdx.x;
-    int d = dst_slot[gl];
-    if (d < 0) return;
-    const float* s = src + (size_t)(gl >> 5) * words * 32 + (gl & 31);
-    float* o = dst + (size_t)(d >> 5) * words * 32 + (d & 31);
-    for (int w = threadIdx.x; w < words; w += blockDim.x) o[w * 32] = s[w * 32];
-    if (threadIdx.x == 0) dst_creature[d] = src_creature[gl];
-}
-// pad: the unused lanes of the last destination batch become empty lanes
-__global__ void compact_pad_kernel(float* dst, int* dst_creature, int words, const int* n_alive) {
-    int n = *n_alive;
-    if (n == 0 || (n & 31) == 0) return;
-    int d = n + threadIdx.x;
-    if ((d >> 5) != ((n - 1) >> 5)) return;
-    float* o = dst + (size_t)(d >> 5) * words * 32 + (d & 31);
-    o[S_NB * 32] = __int_as_float(0);
-    o[S_ALIVE * 32] = __int_as_float(0);
-    dst_creature[d] = -1;
-}
-
 // FP32 issue-rate microbenchmark: 8 independent multiply / add chains per thread. The step kernel is built with
 // -fmad=false (parity), so its ceiling is the non-fused FMUL/FADD issue rate: 1 FLOP per lane per cycle.
 __global__ void fp32_issue_kernel(float* out, int iters, float b, float c) {
@@ -132,7 +90,7 @@ struct ClassState {
     int n_batches = 0;
     int n_members = 0;                  // creatures of this class (lane_creature[0..n_members) are real)
     int episode_grid = 0;               // resident warps of the persistent episode kernel
-    int grid2 = 0, gs2 = 0;             // second, wider-grouped launch for the creatures that do not fit in the first round
+    int grid2 = 0, gs2 = 0;             // overflow wave for the creatures that do not fit in the first round
     cudaStream_t stream2 = nullptr;
     cudaEvent_t done2 = nullptr;
     ParkPolicy park{};
@@ -140,20 +98,12 @@ struct ClassState {
     float* d_state = nullptr;
     int* d_lane_creature = nullptr;
     int* d_queue = nullptr;
-    Buf b_state, b_state2, b_lc, b_lcw0, b_lcw1, b_dst, b_small, b_trace, b_ttrace;   // backing storage (grow-only)
+    float* d_park_state = nullptr;      // columns of the parked creatures, by park slot
+    int* d_park_creature = nullptr;     // park slot -> creature + 1 (0: allocated, not yet published)
+    int* d_park_count = nullptr;        // park slots handed out
+    int* h_park_count = nullptr;        // pinned, see launch_episodes
+    Buf b_state, b_park_state, b_lc, b_park_creature, b_small, b_trace, b_ttrace;   // backing storage (grow-only)
     Buf b_redo_order, b_redo_slots;     // promotion re-runs (grow-only)
-    // phased evaluation with survivor compaction (ping-pong buffers)
-    float* d_state2 = nullptr;
-    int* d_lc_work[2] = {nullptr, nullptr};   // lane -> creature maps of the compacted phases (d_lane_creature stays the static map)
-    const int* lc_cur = nullptr;
-    int lc_next = 0;
-    int done_ticks = 0;
-    int* d_dst_slot = nullptr;
-    int* d_n_alive = nullptr;
-    int* h_n_alive = nullptr;            // pinned
-    int cur_lanes = 0;                  // lanes (padded to 32) of the current phase
-    int phase = 0;
-    bool active = false, pending = false;
     cudaStream_t stream = nullptr;
     cudaEvent_t done = nullptr;
     cudaEvent_t t_begin = nullptr, t_end = nullptr;     // per-class timeline of the last rem2d_run_episodes (diagnostics)
@@ -165,24 +115,13 @@ struct Options {
     int warp_mode_max = -1;      // largest population that runs one warp per creature from tick 0 (-1: 48 per SM)
     int park_ticks = -1;         // park threshold of the queue mode (-1: automatic, 0: never park)
     double park_cap = -1.0;      // fraction of a class that may be parked (-1: automatic)
-    int priority_mode = 1;       // rem2d_set_priority: 0 = expected lifetime >= 130 ticks first, 1 = and among those the longest first
     int overflow_wave = 1;       // queue the CTAs a class could not seat in its first wave behind the first launches (see choose_groups_and_grids)
     int image = -1;              // kernel image of the episode launches (-1: automatic, 0: ~200 registers, 1: 128 registers)
-    int park_late_ticks = -1;    // park threshold of creatures pulled after the first round (-1: same as park_ticks)
-    int park_lead = 0;           // park a creature as soon as its root is where the wall of death will be at the park threshold.
-                                 // Measured and rejected as default: more creatures are parked, and early, while the GPU is still full -
-                                 // the tail launches wait 100-300 ms for resources (950-1200 ms against 800 ms)
-    double smem_budget_kb = 227.0, small_weight = 1.0;
-    double wide_weight = 1.0;    // weight of the wide class next to one-lane classes in a throughput-bound mix (first wave)
-    int min_class = 0;
+    double smem_budget_kb = 227.0;
     int group_shift = -1;        // log2 lanes per creature in the queue / step kernels (-1: per class default)
     int class_gs[N_CLASSES] = {-1, -1, -1, -1, -1, -1, -1, -1, -1};   // per capacity class ("class_gs_<k>", -1: default)
     int tail_group_shift = 5;    // log2 lanes per creature of the tail launches (few creatures are parked by default: a warp each)
-    int second_group_shift = -1; // log2 lanes per creature of a second launch for the creatures a large class cannot seat in its first
-                                 // round (-1: off = refill the first launch's lanes). Measured and rejected as default: the GPU is
-                                 // still throughput-bound when the first round ends, wide groups only add issue load (+25 % run time)
     int trace = 0;
-    int phased = 0;              // tick phases with survivor compaction instead of the persistent queue kernel
 };
 
 struct rem2d_handle {
@@ -208,7 +147,6 @@ struct rem2d_handle {
     int max_warps_per_sm[2] = {8, 16};  // resident warps of the two episode kernel images per SM by registers (occupancy API)
     double first_wave_frac = 1.0;       // share of the shared memory the first-wave grids are sized for
     int prio_high = 0;                  // greatest stream priority of the device (tail pool)
-    bool overflow_wave = false;         // the second launches are overflow waves of the first (same width, both refill)
     int image = 0;                      // kernel image of the current population (0: 200 registers, 1: 128 registers)
     int n_edges = 0;
     // population
@@ -259,33 +197,24 @@ static bool set_option(Options& o, const char* name, double v) {
     if (n == "warp_mode_max") o.warp_mode_max = (int)v;
     else if (n == "park_ticks") o.park_ticks = (int)v;
     else if (n == "park_cap") o.park_cap = v;
-    else if (n == "park_late_ticks") o.park_late_ticks = (int)v;
-    else if (n == "park_lead") o.park_lead = (int)v;
     else if (n == "smem_budget_kb") o.smem_budget_kb = v;
-    else if (n == "small_weight") o.small_weight = v;
-    else if (n == "wide_weight") o.wide_weight = v;
-    else if (n == "min_class") o.min_class = std::max(0, std::min(N_CLASSES - 1, (int)v));
     else if (n == "group_shift") o.group_shift = (int)v;
     else if (n == "tail_group_shift") o.tail_group_shift = std::max(0, std::min(5, (int)v));
-    else if (n == "second_group_shift") o.second_group_shift = std::max(-1, std::min(5, (int)v));
     else if (n == "trace") o.trace = (int)v;
-    else if (n == "phased") o.phased = (int)v;
     else if (n == "image") o.image = std::max(-1, std::min(1, (int)v));
     else if (n == "overflow_wave") o.overflow_wave = (int)v != 0;
-    else if (n == "priority_mode") o.priority_mode = (int)v;
     else if (n.rfind("class_gs_", 0) == 0 && n.size() == 10 && n[9] >= '0' && n[9] < '0' + N_CLASSES) o.class_gs[n[9] - '0'] = (int)v;
     else return false;
     return true;
 }
 static void options_from_env(Options& o) {
-    static const char* names[] = {"warp_mode_max", "park_ticks", "park_cap", "park_late_ticks", "park_lead", "smem_budget_kb", "small_weight", "min_class",
-                                  "group_shift", "tail_group_shift", "second_group_shift", "trace", "image", "overflow_wave", "wide_weight", "priority_mode"};
+    static const char* names[] = {"warp_mode_max", "park_ticks", "park_cap", "smem_budget_kb",
+                                  "group_shift", "tail_group_shift", "trace", "image", "overflow_wave"};
     for (const char* n : names) {
         std::string env = "REM2D_";
         for (const char* q = n; *q; ++q) env += (char)toupper(*q);
         if (const char* e = getenv(env.c_str())) set_option(o, n, atof(e));
     }
-    if (const char* e = getenv("REM2D_EPISODE_MODE")) o.phased = !strcmp(e, "phased");
     if (const char* e = getenv("REM2D_CLASS_GS"))          // "0,0,1,2,2,2,2,3,3": group shift per capacity class
         for (int k = 0; k < N_CLASSES && *e; ++k) { o.class_gs[k] = atoi(e); while (*e && *e != ',') ++e; if (*e == ',') ++e; }
 }
@@ -297,11 +226,11 @@ static void free_population(rem2d_handle* h) {          // logical reset; the bu
 static void release_buffers(rem2d_handle* h) {
     for (auto& b : h->d_pop_mem) { if (b.p) cudaFree(b.p); b = Buf(); }
     for (auto& c : h->cls) {
-        Buf* bufs[] = {&c.b_state, &c.b_state2, &c.b_lc, &c.b_lcw0, &c.b_lcw1, &c.b_dst, &c.b_small, &c.b_trace, &c.b_ttrace,
+        Buf* bufs[] = {&c.b_state, &c.b_park_state, &c.b_lc, &c.b_park_creature, &c.b_small, &c.b_trace, &c.b_ttrace,
                        &c.b_redo_order, &c.b_redo_slots};
         for (Buf* b : bufs) { if (b->p) cudaFree(b->p); *b = Buf(); }
-        if (c.h_n_alive) cudaFreeHost(c.h_n_alive);
-        c.h_n_alive = nullptr;
+        if (c.h_park_count) cudaFreeHost(c.h_park_count);
+        c.h_park_count = nullptr;
     }
     if (h->b_results.p) cudaFree(h->b_results.p);
     h->b_results = Buf();
@@ -380,11 +309,10 @@ int rem2d_create(const rem2d_config* cfg, rem2d_handle** out) {
     if ((e = cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming)) != cudaSuccess) return fail("cudaEventCreate", e);
     cudaDeviceGetAttribute(&h->n_sms, cudaDevAttrMultiProcessorCount, cfg->device);
     {
-        int carve = cudaSharedmemCarveoutMaxShared, max_hot = 0;
-        if (const char* ev = getenv("REM2D_CARVEOUT")) carve = atoi(ev);      // experiment: percent of the unified L1/shared array
+        int max_hot = 0;
         for (int q = 0; q < N_CLASSES; ++q)
             for (int gs = 0; gs <= 5; ++gs) max_hot = std::max(max_hot, g_classes(q).hot_bytes(gs));
-        if ((e = rem2d_set_kernel_attributes(max_hot, carve)) != cudaSuccess) return fail("cudaFuncSetAttribute", e);
+        if ((e = rem2d_set_kernel_attributes(max_hot)) != cudaSuccess) return fail("cudaFuncSetAttribute", e);
         for (int im = 0; im < 2; ++im) h->max_warps_per_sm[im] = std::max(1, rem2d_episode_blocks_per_sm(im, 1024));
     }
     *out = h;
@@ -462,19 +390,17 @@ static int launch_reset(rem2d_handle* h);
 // others. Without this the largest class would occupy every SM until its last creature dies and the remaining classes would
 // run after it. Returns true iff EVERY creature of every class has a group from the start (one round, under-filled GPU).
 static bool size_grids(rem2d_handle* h, double warp_frac = 0.97) {
-    const double smem_kb = h->opt.smem_budget_kb, small_weight = h->opt.small_weight;
+    const double smem_kb = h->opt.smem_budget_kb;
     double budget = (double)h->n_sms * smem_kb * 1024.0 * 0.98 * h->first_wave_frac;
     double work[N_CLASSES], smem[N_CLASSES];
     bool fixed[N_CLASSES];
     for (int k = 0; k < N_CLASSES; ++k) {
         const int gs = h->cur_gs[k];
         work[k] = h->cls[k].work; fixed[k] = h->cls[k].n_members == 0; smem[k] = g_classes(k).hot_bytes(gs) + 1024.0;
-        if (g_classes(k).nb <= 8) work[k] *= small_weight;
         // a group of G lanes is one resident creature: G times the warps for the same residency, and the creature ticks
         // p(G) times faster (measured tick latencies, profiles/r2_timeline_*.txt)
         static const double speedup[6] = {1.0, 1.15, 1.5, 1.9, 2.2, 2.5};
         work[k] *= (double)(1 << gs) / speedup[gs];
-        if (gs > 0 && h->first_wave_frac < 1.0) work[k] *= h->opt.wide_weight;
         h->cls[k].episode_grid = 0;
     }
     // warps_k = W * work_k with W such that sum_k warps_k * smem_k = budget: every class then needs about the same
@@ -549,37 +475,21 @@ static void choose_groups_and_grids(rem2d_handle* h) {
         // EA-configured populations; all-one-lane populations (the bench) lose 4 % with it and keep the full first wave.
         bool mixed = false;
         for (int k = 0; k < N_CLASSES; ++k) mixed |= h->cls[k].n_members > 0 && h->cur_gs[k] > 0;
-        if (mixed && h->opt.overflow_wave && h->opt.second_group_shift < 0 && h->opt.smem_budget_kb > 226.0) {
+        if (mixed && h->opt.overflow_wave && h->opt.smem_budget_kb > 226.0) {
             h->first_wave_frac = 0.75;
             size_grids(h);
         }
     }
     for (int k = 0; k < N_CLASSES; ++k) { h->cls[k].grid2 = 0; h->cls[k].gs2 = 0; }
-    h->overflow_wave = false;
     if (!all_fit) {
-        // Throughput-bound population: one lane per creature, lanes refilled from the class queue. OPTION "second_group_shift"
-        // (off by default): the creatures of the large classes that do not get a lane in the first round are run by a second
-        // launch with wide groups (2-4x lower tick latency) whose CTAs become resident as the first launch's warps exit,
-        // instead of one more lap at the bulk tick latency. Measured on the bench population: the GPU is still
-        // throughput-bound when the first round ends (the small classes run until ~550 ms), so the wide groups only add issue
-        // load: 1050-1200 ms against 815-880 ms with refill.
-        const int gs2 = h->opt.second_group_shift;
-        for (int k = 0; k < N_CLASSES && gs2 >= 0; ++k) {
-            ClassState& cs = h->cls[k];
-            const int per1 = 32 >> h->cur_gs[k];
-            const int left = cs.n_members - cs.episode_grid * per1;
-            if (left <= 0 || g_classes(k).nb < 12 || forced[k]) continue;
-            cs.gs2 = std::max(gs2, h->cur_gs[k]);
-            cs.grid2 = (left + (32 >> cs.gs2) - 1) / (32 >> cs.gs2);
-        }
+        // Throughput-bound population: one lane per creature, lanes refilled from the class queue.
         // OVERFLOW WAVE (default): the first-wave grids above come from a static cost model; when it is off for a population -
         // measured on an EA-configured one: the 33-44 body class done after 1.9 s, the others at 3.1-3.6 s, with the freed 18 MB
         // of shared memory idle in between (profiles/r2_timeline_ea_gen2_before.txt) - nothing could use the resources of a
         // class that has finished. So every class also queues, BEHIND all first launches, the CTAs it could not seat: the
         // work distributor places them as earlier CTAs exit, they pull from the same class queue, and a CTA that finds its
         // queue empty exits at once. The hardware does the balancing.
-        if (gs2 < 0 && h->opt.overflow_wave) {
-            h->overflow_wave = true;
+        if (h->opt.overflow_wave) {
             for (int k = 0; k < N_CLASSES; ++k) {
                 ClassState& cs = h->cls[k];
                 const int per = 32 >> h->cur_gs[k];
@@ -616,12 +526,11 @@ static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_res
     h->creature_class.assign(n, -1);
     h->creature_lane.assign(n, -1);
     std::vector<std::vector<int>> members(N_CLASSES);
-    const int min_class = h->opt.min_class;      // experiment: force small creatures into a larger class
     for (int c = 0; c < n; ++c) {
         int nb = pop->body_off[c + 1] - pop->body_off[c];
         if (nb < 1) { h->err = "upload: creature without a root body"; return REM2D_E_INVALID; }
         int k = -1;
-        for (int q = min_class; q < N_CLASSES; ++q) if (nb <= g_classes(q).nb) { k = q; break; }
+        for (int q = 0; q < N_CLASSES; ++q) if (nb <= g_classes(q).nb) { k = q; break; }
         if (k < 0) { char buf[128]; snprintf(buf, sizeof(buf), "upload: creature %d has %d bodies (> %d supported)", c, nb, g_classes(N_CLASSES - 1).nb); h->err = buf; return REM2D_E_CAPACITY; }
         int j0 = pop->body_off[c] - c;
         for (int j = 0; j < nb - 1; ++j)
@@ -667,7 +576,7 @@ static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_res
         const float long_lived = (h->cfg.terminate && h->cfg.wod_speed > 0.0) ? (float)(5.2 / h->cfg.wod_speed) : 130.0f;
         std::stable_sort(m.begin(), m.end(), [&](int a, int b) {
             int la = prio && h->priority[a] >= long_lived, lb = prio && h->priority[b] >= long_lived;
-            if (prio && h->opt.priority_mode == 1) {      // ... and among those the longest expected lifetime first, in buckets of 32 ticks
+            if (prio) {      // ... and among those the longest expected lifetime first, in buckets of 32 ticks
                 la = la ? 1 + ((int)std::min(h->priority[a], 8192.0f) >> 5) : 0;
                 lb = lb ? 1 + ((int)std::min(h->priority[b], 8192.0f) >> 5) : 0;
             }
@@ -681,16 +590,15 @@ static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_res
         cs.lane_creature.assign((size_t)cs.n_batches * 32, -1);
         for (size_t i = 0; i < m.size(); ++i) { cs.lane_creature[i] = m[i]; h->creature_lane[m[i]] = (int)i; }
         const size_t lane_bytes = cs.lane_creature.size() * sizeof(int);
-        const size_t state_bytes = (size_t)(cs.n_batches + 2) * g_classes(k).words * 32 * sizeof(float);   // (+2: second launch's columns)
+        // (+2: the overflow wave's columns start at the block after the first launch's and end on a whole group)
+        const size_t state_bytes = (size_t)(cs.n_batches + 2) * g_classes(k).words * 32 * sizeof(float);
         CK(ensure(cs.b_lc, lane_bytes)); cs.d_lane_creature = (int*)cs.b_lc.p;
         CK(cudaMemcpy(cs.d_lane_creature, cs.lane_creature.data(), cs.lane_creature.size() * sizeof(int), cudaMemcpyHostToDevice));
         CK(ensure(cs.b_state, state_bytes)); cs.d_state = (float*)cs.b_state.p;
-        CK(ensure(cs.b_state2, state_bytes)); cs.d_state2 = (float*)cs.b_state2.p;
-        CK(ensure(cs.b_lcw0, lane_bytes)); cs.d_lc_work[0] = (int*)cs.b_lcw0.p;
-        CK(ensure(cs.b_lcw1, lane_bytes)); cs.d_lc_work[1] = (int*)cs.b_lcw1.p;
-        CK(ensure(cs.b_dst, lane_bytes)); cs.d_dst_slot = (int*)cs.b_dst.p;
-        CK(ensure(cs.b_small, 64)); cs.d_n_alive = (int*)cs.b_small.p; cs.d_queue = (int*)cs.b_small.p + 4;
-        if (!cs.h_n_alive) CK(cudaMallocHost(&cs.h_n_alive, sizeof(int)));
+        CK(ensure(cs.b_park_state, state_bytes)); cs.d_park_state = (float*)cs.b_park_state.p;
+        CK(ensure(cs.b_park_creature, lane_bytes)); cs.d_park_creature = (int*)cs.b_park_creature.p;
+        CK(ensure(cs.b_small, 64)); cs.d_park_count = (int*)cs.b_small.p; cs.d_queue = (int*)cs.b_small.p + 4;
+        if (!cs.h_park_count) CK(cudaMallocHost(&cs.h_park_count, sizeof(int)));
     }
     {   // per-creature cost ~ tick latency of its size: measured ~0.3 ms + 0.085 ms per body for a resident warp; lone bodies
         // fall asleep after landing and cost almost nothing
@@ -727,11 +635,6 @@ static int join_streams(rem2d_handle* h) {
         CK(cudaEventRecord(c.done, c.stream)); CK(cudaStreamWaitEvent(h->user_stream, c.done, 0));
         CK(cudaEventRecord(c.done2, c.stream2)); CK(cudaStreamWaitEvent(h->user_stream, c.done2, 0));
     }
-    return REM2D_OK;
-}
-
-static int join_streams_all(rem2d_handle* h) {
-    for (auto& c : h->cls) if (c.n_batches) { CK(cudaEventRecord(c.done, c.stream)); CK(cudaStreamWaitEvent(h->user_stream, c.done, 0)); }
     return REM2D_OK;
 }
 
@@ -789,92 +692,12 @@ static int promote_overflowed(rem2d_handle* h, int max_ticks) {
             CK(cudaMemsetAsync(d_queue, 0, sizeof(int), h->user_stream));
             g_classes(k).episode(h->image, gs, grid, h->user_stream, (float*)cs.b_redo_slots.p, d_order, (int)redo[k].size(), d_queue, h->dpop, h->d_ter,
                                  h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr}, nullptr, nullptr, nullptr, 1);
+                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr}, nullptr, nullptr, nullptr);
             h->launches++;
             CK(cudaGetLastError());
             CK(cudaStreamSynchronize(h->user_stream));      // redo[] (pageable source of the copy) goes out of scope
         }
     }
-    return REM2D_OK;
-}
-
-// Whole episodes in tick phases with survivor compaction (default evaluate path).
-// Every class advances independently on its own stream: step_kernel(phase ticks) -> plan (harvest finished creatures,
-// assign dense slots to survivors) -> copy columns into the other buffer -> the host reads the survivor count and
-// launches the next, smaller phase. Almost every creature of a random population dies when the wall of death reaches
-// the start pad (tick ~126), so the first phase is 128 ticks; afterwards the few survivors are repacked every 32 ticks
-// instead of keeping their original warps alive at 1-3 live lanes out of 32.
-static int launch_phased(rem2d_handle* h, int max_ticks) {
-    if (!h->have_terrain) { h->err = "run_episodes: no terrain set"; return REM2D_E_INVALID; }
-    CK(cudaEventRecord(h->ev_start, h->user_stream));
-    int rc = launch_reset(h);           // builds every world into the static batches (also zeroes the counters)
-    if (rc) return rc;
-    rc = fork_streams(h);
-    if (rc) return rc;
-    int n_active = 0;
-    for (int k = N_CLASSES - 1; k >= 0; --k) {
-        ClassState& cs = h->cls[k];
-        cs.active = cs.n_batches > 0; cs.pending = false; cs.phase = 0; cs.cur_lanes = cs.n_batches * 32;
-        cs.lc_cur = cs.d_lane_creature; cs.lc_next = 0; cs.done_ticks = 0;
-        if (cs.active) ++n_active;
-    }
-    const int first_phase = 128, next_phase = 32;
-    auto enqueue = [&](int k) -> int {
-        ClassState& cs = h->cls[k];
-        const int words = g_classes(k).words;
-        const int batches = cs.cur_lanes / 32;
-        int ticks = cs.phase == 0 ? first_phase : next_phase;
-        if (ticks > max_ticks - cs.done_ticks) ticks = max_ticks - cs.done_ticks;
-        cs.done_ticks += ticks;
-        int* lc_dst = cs.d_lc_work[cs.lc_next];
-        g_classes(k).step(step_gs(h, k), batches, cs.stream, cs.d_state, ticks, h->d_ter, h->d_consts, h->d_counters);
-        CK(cudaMemsetAsync(cs.d_n_alive, 0, sizeof(int), cs.stream));
-        compact_plan_kernel<<<(cs.cur_lanes + 127) / 128, 128, 0, cs.stream>>>(cs.d_state, cs.lc_cur, cs.cur_lanes, words, max_ticks,
-                                                                              h->d_fitness, h->d_ticks, h->d_alive, h->d_status,
-                                                                              cs.d_dst_slot, cs.d_n_alive);
-        compact_copy_kernel<<<cs.cur_lanes, 128, 0, cs.stream>>>(cs.d_state, cs.d_state2, cs.d_dst_slot, cs.lc_cur, lc_dst, words);
-        compact_pad_kernel<<<1, 32, 0, cs.stream>>>(cs.d_state2, lc_dst, words, cs.d_n_alive);
-        CK(cudaMemcpyAsync(cs.h_n_alive, cs.d_n_alive, sizeof(int), cudaMemcpyDeviceToHost, cs.stream));
-        CK(cudaGetLastError());
-        h->launches += 4;
-        cs.pending = true;
-        return REM2D_OK;
-    };
-    for (int k = N_CLASSES - 1; k >= 0; --k)
-        if (h->cls[k].active) { rc = enqueue(k); if (rc) return rc; }
-    while (n_active > 0) {
-        bool progressed = false;
-        for (int k = N_CLASSES - 1; k >= 0; --k) {
-            ClassState& cs = h->cls[k];
-            if (!cs.active || !cs.pending) continue;
-            cudaError_t q = cudaStreamQuery(cs.stream);
-            if (q == cudaErrorNotReady) continue;
-            if (q != cudaSuccess) { h->err = std::string("phase: ") + cudaGetErrorString(q); return REM2D_E_CUDA; }
-            progressed = true;
-            cs.pending = false;
-            std::swap(cs.d_state, cs.d_state2);
-            cs.lc_cur = cs.d_lc_work[cs.lc_next];
-            cs.lc_next ^= 1;
-            int alive = *cs.h_n_alive;
-            cs.phase++;
-            // creatures that reached the tick budget were harvested by the plan kernel, so alive == 0 ends the class
-            if (alive == 0) { cs.active = false; --n_active; continue; }
-            cs.cur_lanes = ((alive + 31) / 32) * 32;
-            rc = enqueue(k);
-            if (rc) return rc;
-        }
-        if (!progressed) {
-#if defined(__x86_64__)
-            __builtin_ia32_pause();
-#endif
-        }
-    }
-    rc = join_streams_all(h);
-    if (rc) return rc;
-    rc = promote_overflowed(h, max_ticks);
-    if (rc) return rc;
-    CK(cudaEventRecord(h->ev_stop, h->user_stream));
-    h->state_valid = false; h->results_valid = true;
     return REM2D_OK;
 }
 
@@ -897,9 +720,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
             const int per = 32 >> class_gs(h, k);
             if (h->cls[k].n_batches && h->cls[k].episode_grid * per < h->cls[k].n_members) single_round = false;
         }
-        bool second = false;
-        for (int k = 0; k < N_CLASSES; ++k) second |= h->cls[k].grid2 > 0 && !h->overflow_wave;
-        if (single_round || second) { park_ticks = 160; cap_frac = 0.25; }
+        if (single_round) { park_ticks = 160; cap_frac = 0.25; }
     }
     if (h->opt.park_ticks >= 0) park_ticks = h->opt.park_ticks;
     if (h->opt.park_cap >= 0.0) cap_frac = h->opt.park_cap;
@@ -935,23 +756,18 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         if (warp_mode) {      // queue mode with a whole warp per creature and one warp for every creature
             g_classes(k).episode(1, 5, cs.n_members, cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop, h->d_ter,
                                  h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr}, nullptr, nullptr, nullptr, 1);
+                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr}, nullptr, nullptr, nullptr);
             CK(cudaEventRecord(cs.t_end, cs.stream));
             h->launches++;
             continue;
         }
-        CK(cudaMemsetAsync(cs.d_n_alive, 0, sizeof(int), cs.stream));
-        CK(cudaMemsetAsync(cs.d_lc_work[0], 0, cs.lane_creature.size() * sizeof(int), cs.stream));     // "unpublished" markers
+        CK(cudaMemsetAsync(cs.d_park_count, 0, sizeof(int), cs.stream));
+        CK(cudaMemsetAsync(cs.d_park_creature, 0, cs.lane_creature.size() * sizeof(int), cs.stream));     // "unpublished" markers
         ParkPolicy park;
         park.ticks = park_ticks < max_ticks ? park_ticks : 0;
         park.cap = std::min(cs.n_members, std::max(32, std::min((int)(h->n_sms * 64 * cap_frac), (int)(cs.n_members * cap_frac))));
-        // late starters (pulled when a lane of the first round frees up): park right after the wall of death has passed the
-        // start pad (tick 126), so that the long-lived ones among them continue at the tail launches' tick latency
-        // a root that is already where the wall of death will be at the park threshold survives until then unless it walks back
-        park.lead_x = (h->opt.park_lead && h->cfg.terminate) ? (float)(park.ticks * h->cfg.wod_speed) : 0.0f;
-        park.lead_from = 32;
-        park.late_from = cs.episode_grid * (32 >> class_gs(h, k));
-        park.late_ticks = h->opt.park_late_ticks >= 0 ? std::min(h->opt.park_late_ticks, park.ticks) : park.ticks;
+        park.lead_x = 0.0f; park.lead_from = 0;
+        park.late_from = cs.n_members; park.late_ticks = park.ticks;
         park.trace = nullptr; park.tail_trace = nullptr;
         if (trace) {
             const size_t tb = (size_t)std::max(cs.n_members, 1) * 4 * sizeof(unsigned int);
@@ -967,13 +783,15 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         cs.park = park;
         g_classes(k).episode(h->image, class_gs(h, k), cs.episode_grid, cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop,
                              h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                             park, cs.d_state2, cs.d_lc_work[0], cs.d_n_alive, (cs.grid2 > 0 && !h->overflow_wave) ? 0 : 1);
-        CK(cudaMemcpyAsync(cs.h_n_alive, cs.d_n_alive, sizeof(int), cudaMemcpyDeviceToHost, cs.stream));
+                             park, cs.d_park_state, cs.d_park_creature, cs.d_park_count);
+        // Nothing reads this copy, but it shapes the tail launches: without it the bench population gets twice the tail
+        // launches and the second EA generation evaluates 40 % slower (3.1 s against 2.2 s; B200 at 1000 W).
+        CK(cudaMemcpyAsync(cs.h_park_count, cs.d_park_count, sizeof(int), cudaMemcpyDeviceToHost, cs.stream));
         CK(cudaEventRecord(cs.t_end, cs.stream));
         h->launches++;
     }
-    // second launches (after ALL first launches, so that their CTAs queue behind them): the creatures a class could not seat
-    // in its first round, in wide groups, on the columns behind the first launch's
+    // overflow waves (after ALL first launches, so that their CTAs queue behind them): the creatures a class could not seat
+    // in its first round, on the columns behind the first launch's
     for (int oi = 0; oi < N_CLASSES && !warp_mode; ++oi) {
         const int k = launch_order[oi];
         ClassState& cs = h->cls[k];
@@ -984,7 +802,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         park.trace = nullptr;
         g_classes(k).episode(h->image, cs.gs2, cs.grid2, cs.stream2, cs.d_state + first_block * g_classes(k).words * 32, cs.d_lane_creature, cs.n_members,
                              cs.d_queue, h->dpop, h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status,
-                             h->d_counters, park, cs.d_state2, cs.d_lc_work[0], cs.d_n_alive, 1);
+                             h->d_counters, park, cs.d_park_state, cs.d_park_creature, cs.d_park_count);
         h->launches++;
     }
     CK(cudaGetLastError());
@@ -1024,7 +842,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
                 if (q == cudaSuccess && h->cls[k].grid2 > 0) q = cudaStreamQuery(h->cls[k].stream2);
                 if (q == cudaSuccess) finished_now[k] = true;
                 else if (q != cudaErrorNotReady) { h->err = std::string("episode kernel: ") + cudaGetErrorString(q); return REM2D_E_CUDA; }
-                CK(cudaMemcpyAsync(&h->h_poll[k], h->cls[k].d_n_alive, sizeof(int), cudaMemcpyDeviceToHost, h->poll_stream));
+                CK(cudaMemcpyAsync(&h->h_poll[k], h->cls[k].d_park_count, sizeof(int), cudaMemcpyDeviceToHost, h->poll_stream));
             }
             CK(cudaStreamSynchronize(h->poll_stream));
             for (int k = N_CLASSES - 1; k >= 0; --k) {
@@ -1038,7 +856,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
                     // a handful of parked creatures (random populations): a warp each; dozens at once (evolved populations,
                     // where many creatures outlive the threshold): 8 lanes each - 4x fewer warps at nearly the same tick latency
                     const int tail_gs = (cnt - launched[k] >= 32) ? std::min(3, h->opt.tail_group_shift) : h->opt.tail_group_shift;
-                    g_classes(k).tail(h->image, tail_gs, idle_stream(), cs.d_state2, cs.d_lc_work[0], launched[k], cnt - launched[k],
+                    g_classes(k).tail(h->image, tail_gs, idle_stream(), cs.d_park_state, cs.d_park_creature, launched[k], cnt - launched[k],
                                       h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
                                       trace ? (unsigned int*)cs.b_ttrace.p : nullptr);
                     CK(cudaGetLastError());
@@ -1154,10 +972,7 @@ int rem2d_run_episodes(rem2d_handle* h, int32_t max_ticks) {
     if (!h) return REM2D_E_INVALID;
     if (!h->have_pop || max_ticks < 0) { h->err = "run_episodes: no population / negative tick count"; return REM2D_E_INVALID; }
     cudaSetDevice(h->cfg.device);
-    // Default: persistent kernel with per-lane refill. REM2D_EPISODE_MODE=phased selects tick phases with survivor
-    // compaction instead (measured slower at pop 65536: the run is bound by the sequential ticks of the longest-lived
-    // large creature, and phases add a launch/sync per 32 ticks to exactly that critical path).
-    int rc = h->opt.phased ? launch_phased(h, max_ticks) : launch_episodes(h, max_ticks);
+    int rc = launch_episodes(h, max_ticks);
     if (rc) return rc;
     CK(cudaEventSynchronize(h->ev_stop));
     CK(cudaEventElapsedTime(&h->last_ms, h->ev_start, h->ev_stop));
@@ -1250,7 +1065,7 @@ int rem2d_debug_tail_trace(rem2d_handle* h, int k, unsigned int* out, int64_t ma
     cudaSetDevice(h->cfg.device);
     cudaDeviceSynchronize();
     int parked = 0;
-    CK(cudaMemcpy(&parked, cs.d_n_alive, sizeof(int), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&parked, cs.d_park_count, sizeof(int), cudaMemcpyDeviceToHost));
     size_t words = (size_t)parked * 4;
     if ((int64_t)words > max_words) words = (size_t)max_words;
     CK(cudaMemcpy(out, cs.b_ttrace.p, words * sizeof(unsigned int), cudaMemcpyDeviceToHost));

@@ -84,9 +84,6 @@ void rem2d_launch_step(const Layout& L, int gs, int n_batches, cudaStream_t st, 
 // than the park threshold are parked for mode 1. With gs = 5 and one warp per creature this is the latency-oriented
 // execution of SMALL populations (every creature has its own warp from tick 0).
 //
-// `refill` = 0: every group pulls ONE creature and the warp exits when its creatures are done (primary launch of a class that
-// does not fit in one round: the leftover creatures are run by a second, wider-grouped launch as soon as CTAs exit).
-//
 // mode 1, tail: takes over parked creatures (one per group, normally gs = 5: a whole warp per creature) and finishes them:
 // the long-lived creatures bound the makespan, and a 32-lane schedule ticks a large creature several times faster than
 // the throughput-oriented groups of the queue mode.
@@ -101,7 +98,7 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
                                                         const Terrain* __restrict__ ter, const Consts* __restrict__ k, int max_ticks,
                                                         double* fitness, int* ticks, int* alive, int* status,
                                                         unsigned long long* counters, ParkPolicy park, float* park_state,
-                                                        int* park_creature, int* park_count, int first_slot, int n_slots, int refill) {
+                                                        int* park_creature, int* park_count, int first_slot, int n_slots) {
     extern __shared__ float hot[];
     const int lane = threadIdx.x;
     const bool tail = mode != 0;
@@ -146,7 +143,7 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
             if (sim.leader()) idx = atomicAdd(queue, 1);
             idx = sim.bcast(idx);
             if (idx < n_order) {
-                my = order[idx]; sim.build_world(p, my); snapshot = sim.cnt; exhausted = !refill;
+                my = order[idx]; sim.build_world(p, my); snapshot = sim.cnt;
                 park_at = idx >= park.late_from ? park.late_ticks : park.ticks;
             }
             else exhausted = true;
@@ -230,20 +227,20 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
 #define EPISODE_PARAMS const __grid_constant__ Layout L, int gs, int mode, float* slots, const int* __restrict__ order, int n_order, int* queue, \
                        DevPop p, const Terrain* __restrict__ ter, const Consts* __restrict__ k, int max_ticks, double* fitness, int* ticks, \
                        int* alive, int* status, unsigned long long* counters, ParkPolicy park, float* park_state, int* park_creature,      \
-                       int* park_count, int first_slot, int n_slots, int refill
+                       int* park_count, int first_slot, int n_slots
 #define EPISODE_ARGS L, gs, mode, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive, status, counters, park, park_state, \
-                     park_creature, park_count, first_slot, n_slots, refill
+                     park_creature, park_count, first_slot, n_slots
 __global__ void __launch_bounds__(32, 1) episode_kernel(EPISODE_PARAMS) { episode_body(EPISODE_ARGS); }
 __global__ void __launch_bounds__(32, 16) episode_kernel_r128(EPISODE_PARAMS) { episode_body(EPISODE_ARGS); }
 
 void rem2d_launch_episode(const Layout& L, int image, int gs, int grid, cudaStream_t st, float* slots, const int* order, int n_order, int* queue,
                           DevPop p, const Terrain* ter, const Consts* k, int max_ticks, double* fitness, int* ticks, int* alive, int* status,
-                          unsigned long long* counters, ParkPolicy park, float* park_state, int* park_creature, int* park_count, int refill) {
+                          unsigned long long* counters, ParkPolicy park, float* park_state, int* park_creature, int* park_count) {
     const int smem = make_hot_layout(L, gs).rows * 128;
     if (image) episode_kernel_r128<<<grid, 32, smem, st>>>(L, gs, 0, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive,
-                                                            status, counters, park, park_state, park_creature, park_count, 0, 0, refill);
+                                                            status, counters, park, park_state, park_creature, park_count, 0, 0);
     else episode_kernel<<<grid, 32, smem, st>>>(L, gs, 0, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive, status,
-                                                counters, park, park_state, park_creature, park_count, 0, 0, refill);
+                                                counters, park, park_state, park_creature, park_count, 0, 0);
 }
 // resident CTAs (= warps) of the episode kernel per SM for a given dynamic shared-memory size: registers AND shared memory
 int rem2d_episode_blocks_per_sm(int image, int dyn_smem_bytes) {
@@ -260,9 +257,9 @@ void rem2d_launch_tail(const Layout& L, int image, int gs, cudaStream_t st, floa
     const int per = 32 >> gs, grid = (n_parked + per - 1) / per, smem = make_hot_layout(L, gs).rows * 128;
     if (image) episode_kernel_r128<<<grid, 32, smem, st>>>(L, gs, 1, nullptr, nullptr, 0, nullptr, DevPop(), ter, k, max_ticks, fitness, ticks,
                                                             alive, status, counters, none, park_state, park_creature, nullptr, first_slot,
-                                                            n_parked, 0);
+                                                            n_parked);
     else episode_kernel<<<grid, 32, smem, st>>>(L, gs, 1, nullptr, nullptr, 0, nullptr, DevPop(), ter, k, max_ticks, fitness, ticks, alive, status,
-                                                counters, none, park_state, park_creature, nullptr, first_slot, n_parked, 0);
+                                                counters, none, park_state, park_creature, nullptr, first_slot, n_parked);
 }
 #endif
 
@@ -270,26 +267,26 @@ void rem2d_launch_tail(const Layout& L, int image, int gs, cudaStream_t st, floa
 // All kernels that can be resident together should agree on the shared-memory carve-out of the SM: a small-smem kernel
 // (tail) would otherwise pin its SMs in a large-L1 configuration and lock the big episode CTAs of other classes out
 // (measured: 1.4x slower whole run when a tail kernel was resident next to the episode kernels).
-cudaError_t rem2d_attr_step(int max_hot_bytes, int carve);
-cudaError_t rem2d_attr_episode(int max_hot_bytes, int carve);
+cudaError_t rem2d_attr_step(int max_hot_bytes);
+cudaError_t rem2d_attr_episode(int max_hot_bytes);
 #if REM2D_KERNEL_ID == 0
-cudaError_t rem2d_set_kernel_attributes(int max_hot_bytes, int carve) {
-    cudaError_t e = rem2d_attr_step(max_hot_bytes, carve);
+cudaError_t rem2d_set_kernel_attributes(int max_hot_bytes) {
+    cudaError_t e = rem2d_attr_step(max_hot_bytes);
     if (e != cudaSuccess) return e;
-    return rem2d_attr_episode(max_hot_bytes, carve);
+    return rem2d_attr_episode(max_hot_bytes);
 }
 #elif REM2D_KERNEL_ID == 1
-cudaError_t rem2d_attr_step(int max_hot_bytes, int carve) {
+cudaError_t rem2d_attr_step(int max_hot_bytes) {
     cudaError_t e = cudaFuncSetAttribute(step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes);
     if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(step_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
+    return cudaFuncSetAttribute(step_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
 }
 #elif REM2D_KERNEL_ID == 2
-cudaError_t rem2d_attr_episode(int max_hot_bytes, int carve) {
+cudaError_t rem2d_attr_episode(int max_hot_bytes) {
     cudaError_t e = cudaFuncSetAttribute(episode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes);
     if (e != cudaSuccess) return e;
-    if ((e = cudaFuncSetAttribute(episode_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carve)) != cudaSuccess) return e;
+    if ((e = cudaFuncSetAttribute(episode_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)) != cudaSuccess) return e;
     if ((e = cudaFuncSetAttribute(episode_kernel_r128, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes)) != cudaSuccess) return e;
-    return cudaFuncSetAttribute(episode_kernel_r128, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
+    return cudaFuncSetAttribute(episode_kernel_r128, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
 }
 #endif

@@ -167,7 +167,7 @@ int rem2d_measure_fp32_peak(rem2d_handle* h, double* gflops);
 /* Number of kernels this library launched since rem2d_create. */
 int64_t rem2d_launch_count(rem2d_handle* h);
 /* Tuning / diagnostic option by name (execution strategy only, never results): "warp_mode_max", "park_ticks", "park_cap",
- * "smem_budget_kb", "small_weight", "min_class", "group_shift", "tail_group_shift", "trace", "phased" (DESIGN.md section 4).
+ * "smem_budget_kb", "group_shift", "class_gs_<k>", "tail_group_shift", "overflow_wave", "image", "trace" (DESIGN.md section 4).
  * Unknown names return REM2D_E_INVALID. The oracle accepts the same names and ignores them. */
 int rem2d_set_option(rem2d_handle* h, const char* name, double value);
 /* Optional scheduling hint for the NEXT rem2d_upload / rem2d_evaluate: expected lifetime of every creature in ticks (an EA passes

@@ -2211,8 +2211,8 @@ float rem2d_last_step_ms(rem2d_handle* h) { (void)h; return 0.0f; }
 int64_t rem2d_launch_count(rem2d_handle* h) { (void)h; return 0; }
 /* execution-strategy options of the CUDA build: accepted and ignored (they never change results) */
 int rem2d_set_option(rem2d_handle* h, const char* name, double value) {
-    static const char* known[] = {"warp_mode_max", "park_ticks", "park_cap", "smem_budget_kb", "small_weight", "min_class",
-                                  "group_shift", "tail_group_shift", "second_group_shift", "park_late_ticks", "park_lead", "trace", "phased", "image", "overflow_wave", "wide_weight", "priority_mode"};
+    static const char* known[] = {"warp_mode_max", "park_ticks", "park_cap", "smem_budget_kb",
+                                  "group_shift", "tail_group_shift", "trace", "image", "overflow_wave"};
     (void)value;
     if (!h || !name) return REM2D_E_INVALID;
     for (size_t i = 0; i < sizeof(known) / sizeof(known[0]); ++i) if (!strcmp(known[i], name)) return REM2D_OK;

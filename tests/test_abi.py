@@ -65,7 +65,7 @@ def test_product_package_never_imports_the_oracle():
 
 def test_documented_options_are_the_implemented_ones():
     """DESIGN.md's option list, the names rem2d_set_option of the CUDA library parses (read from its source) and the names the
-    oracle's stub accepts are the same set; unknown names are an error."""
+    oracle's stub accepts are the same set; unknown names, and the names of removed execution strategies, are an error."""
     import ctypes
     import re
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -81,5 +81,9 @@ def test_documented_options_are_the_implemented_ones():
     e = OracleEngine()
     for name in sorted(implemented):
         e.set_option(name.replace("<k>", "3"), 1.0)
-    with pytest.raises(Exception):
-        e.set_option("no_such_option", 1.0)
+    removed = ("phased", "second_group_shift", "park_late_ticks", "park_lead", "priority_mode", "min_class", "small_weight",
+               "wide_weight")
+    for name in ("no_such_option",) + removed:
+        assert name not in implemented, name
+        with pytest.raises(Exception):
+            e.set_option(name, 1.0)
