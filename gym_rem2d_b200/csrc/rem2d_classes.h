@@ -1,27 +1,9 @@
-// rem2d_classes.h — capacity classes and the launch interface of the three kernels (rem2d_kernels.cu; one translation
-// unit per kernel so that they compile in parallel). All classes run the SAME code: the class only selects a Layout and
-// a default group size.
+// rem2d_classes.h — the launch interface of the three kernels (rem2d_kernels.cu; one translation unit per kernel so that
+// they compile in parallel) and the host's per-class view of it. All classes run the SAME code: the class only selects a
+// Layout (the capacity classes themselves are in rem2d_host_util.h).
 #pragma once
 #include <cuda_runtime.h>
 #include "rem2d_device.cuh"
-
-// NB bodies, NC contact-pool slots (fat-AABB overlaps), NT touching contacts staged in shared memory (further touching
-// contacts, up to NC, spill to the cold block: correct but slower), GS = largest log2(lanes per creature) the automatic choice
-// may give the class (rem2d_cuda.cu: choose_groups_and_grids; 1-2 body creatures have nothing to share). Hot words per creature
-// = 5*NB + 17*(NB-1) + 21*NT (+ schedule rows per warp when lanes are shared); shared memory, not registers, bounds the resident
-// creatures per SM, so lanes are the free resource: a group of 2^gs lanes shares one creature's solver sweeps (static modulo
-// schedule, rem2d_device.cuh) and its per-body / per-joint / per-contact loops.
-#define REM2D_CLASSES(X) \
-    X(0, 1, 10, 3, 0)    \
-    X(1, 2, 16, 4, 0)    \
-    X(2, 4, 28, 4, 1)    \
-    X(3, 8, 48, 6, 3)    \
-    X(4, 12, 64, 6, 5)   \
-    X(5, 16, 80, 6, 5)   \
-    X(6, 22, 104, 6, 5)  \
-    X(7, 32, 144, 8, 5)  \
-    X(8, 44, 192, 10, 5)
-#define N_CLASSES 9
 
 // When the queue-mode episode kernel hands a creature over to the tail mode (launches of the same kernel).
 struct ParkPolicy {
@@ -29,7 +11,7 @@ struct ParkPolicy {
     int cap;          // at most this many creatures of the class are parked
     // Always off (lead_x = 0, late_from = class size): the rejected lead and late-start park tests of the episode kernel.
     // Deleting them takes episode_kernel from 202 to 200 registers; at 200, 10 instead of 9 warps fit per SM, so the
-    // occupancy-based grid sizing (size_grids) hands out other first-wave grids.
+    // occupancy-based grid sizing (size_grids, rem2d_host_util.h) hands out other first-wave grids.
     float lead_x;     // > 0: park a creature whose root has reached x >= lead_x after lead_from ticks
     int lead_from;
     int late_from;    // creatures pulled from this position of the class queue on park after late_ticks ticks
@@ -58,12 +40,11 @@ void rem2d_launch_tail(const rem2d::Layout& L, int image, int gs, cudaStream_t s
 // Per-class view used by the host code.
 struct ClassOps {
     rem2d::Layout L;
-    int nb, nc, nt, nj, off_body, off_joint, off_cont, off_edge, words, hot_words, gs;
-    explicit ClassOps(int NB, int NC, int NT, int GS) : L(rem2d::make_layout(NB, NC, NT)) {
+    int nb, nc, nt, nj, off_body, off_joint, off_cont, off_edge, words, hot_words;
+    explicit ClassOps(int NB, int NC, int NT) : L(rem2d::make_layout(NB, NC, NT)) {
         nb = L.nb; nc = L.nc; nt = L.nt; nj = L.nj; off_body = rem2d::S_COUNT; off_joint = L.off_joint; off_cont = L.off_cont;
-        off_edge = L.off_edge; words = L.words; hot_words = L.hot_words; gs = GS;
+        off_edge = L.off_edge; words = L.words; hot_words = L.hot_words;
     }
-    int hot_bytes(int gshift) const { return rem2d::make_hot_layout(L, gshift).rows * 128; }
     template <class... A> void reset(A... a) const { rem2d_launch_reset(L, a...); }
     template <class... A> void step(A... a) const { rem2d_launch_step(L, a...); }
     template <class... A> void episode(A... a) const { rem2d_launch_episode(L, a...); }

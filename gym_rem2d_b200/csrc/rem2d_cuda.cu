@@ -21,13 +21,8 @@
 
 using namespace rem2d;
 
-// ------------------------------------------------------------------ capacity classes (rem2d_classes.h)
-static const ClassOps g_classes_tab[N_CLASSES] = {
-#define X(i, NB, NC, NT, GS) ClassOps(NB, NC, NT, GS),
-    REM2D_CLASSES(X)
-#undef X
-};
-#define g_classes(k) (g_classes_tab[k])
+// capacity class k (rem2d_host_util.h: class_dims)
+static ClassOps g_classes(int k) { return ClassOps(class_dims[k].nb, class_dims[k].nc, class_dims[k].nt); }
 
 // fitness / ticks / alive / status of every creature of a class -> creature-indexed outputs
 __global__ void gather_kernel(const float* state, const int* __restrict__ lane_creature, int n_lanes, int words,
@@ -89,12 +84,8 @@ struct ClassState {
     std::vector<int> lane_creature;     // host copy: [n_batches*32], -1 = padding lane
     int n_batches = 0;
     int n_members = 0;                  // creatures of this class (lane_creature[0..n_members) are real)
-    int episode_grid = 0;               // resident warps of the persistent episode kernel
-    int grid2 = 0, gs2 = 0;             // overflow wave for the creatures that do not fit in the first round
-    cudaStream_t stream2 = nullptr;
+    cudaStream_t stream2 = nullptr;     // overflow wave
     cudaEvent_t done2 = nullptr;
-    ParkPolicy park{};
-    double work = 0.0;                  // sum of the per-creature cost estimates (grid sizing)
     float* d_state = nullptr;
     int* d_lane_creature = nullptr;
     int* d_queue = nullptr;
@@ -109,25 +100,11 @@ struct ClassState {
     cudaEvent_t t_begin = nullptr, t_end = nullptr;     // per-class timeline of the last rem2d_run_episodes (diagnostics)
 };
 
-// Tuning / diagnostic options (rem2d_set_option; the REM2D_* environment variables of the same names are read ONCE, at
-// rem2d_create, as initial values - tools/sweep_groups.py, tools/ea_pop_sweep.py and the tests use them). Defaults are the measured optimum.
-struct Options {
-    int warp_mode_max = -1;      // largest population that runs one warp per creature from tick 0 (-1: 48 per SM)
-    int park_ticks = -1;         // park threshold of the queue mode (-1: automatic, 0: never park)
-    double park_cap = -1.0;      // fraction of a class that may be parked (-1: automatic)
-    int overflow_wave = 1;       // queue the CTAs a class could not seat in its first wave behind the first launches (see choose_groups_and_grids)
-    int image = -1;              // kernel image of the episode launches (-1: automatic, 0: ~200 registers, 1: 128 registers)
-    double smem_budget_kb = 227.0;
-    int group_shift = -1;        // log2 lanes per creature in the queue / step kernels (-1: per class default)
-    int class_gs[N_CLASSES] = {-1, -1, -1, -1, -1, -1, -1, -1, -1};   // per capacity class ("class_gs_<k>", -1: default)
-    int tail_group_shift = 5;    // log2 lanes per creature of the tail launches (few creatures are parked by default: a warp each)
-    int trace = 0;
-};
-
 struct rem2d_handle {
     rem2d_config cfg;
     Options opt;
-    int cur_gs[N_CLASSES] = {0, 0, 0, 0, 0, 0, 0, 0, 0};     // lanes per creature (log2) of the queue mode, per class
+    PlanInput load;                     // device and class sizes of the uploaded population, as the planner sees them
+    UploadPlan plan{};                  // group widths, grids and kernel image of the uploaded population (plan_upload)
     cudaStream_t user_stream = nullptr;
     Terrain* d_ter = nullptr;
     Consts* d_consts = nullptr;
@@ -143,11 +120,7 @@ struct rem2d_handle {
     bool have_terrain = false, have_pop = false;
     bool state_valid = false;           // per-creature state blocks hold a consistent snapshot (reset/step path)
     bool results_valid = false;         // d_fitness/d_ticks/... were written by the episode kernel
-    int n_sms = 0;
-    int max_warps_per_sm[2] = {8, 16};  // resident warps of the two episode kernel images per SM by registers (occupancy API)
-    double first_wave_frac = 1.0;       // share of the shared memory the first-wave grids are sized for
     int prio_high = 0;                  // greatest stream priority of the device (tail pool)
-    int image = 0;                      // kernel image of the current population (0: 200 registers, 1: 128 registers)
     int n_edges = 0;
     // population
     int n_creatures = 0, n_bodies = 0, n_joints = 0;
@@ -179,19 +152,6 @@ static thread_local std::string g_create_err;
         }                                                                                                \
     } while (0)
 
-// group shift of class k for the QUEUE mode of the uploaded population (choose_groups_and_grids)
-static int class_gs(const rem2d_handle* h, int k) { return h->cur_gs[k]; }
-// group shift of the stepping kernels (rem2d_reset / rem2d_step: static creature -> column mapping, no residency limit): the
-// option if given, else as wide as keeps all warps of the population resident at once (a single creature gets a whole warp)
-static int step_gs(const rem2d_handle* h, int k) {
-    const int o = h->opt.group_shift >= 0 ? h->opt.group_shift : h->opt.class_gs[k];
-    if (o >= 0) return std::min(5, o);
-    int total = 0;
-    for (int q = 0; q < N_CLASSES; ++q) total += h->cls[q].n_batches;
-    int gs = 0;
-    while (gs < 5 && (total << (gs + 1)) <= h->n_sms * 8) ++gs;
-    return g_classes(k).nb <= 2 ? 0 : gs;
-}
 static bool set_option(Options& o, const char* name, double v) {
     const std::string n(name);
     if (n == "warp_mode_max") o.warp_mode_max = (int)v;
@@ -307,13 +267,13 @@ int rem2d_create(const rem2d_config* cfg, rem2d_handle** out) {
     if ((e = cudaEventCreateWithFlags(&h->pool_done, cudaEventDisableTiming)) != cudaSuccess) return fail("cudaEventCreate", e);
     if ((e = cudaMallocHost(&h->h_poll, sizeof(int) * 16)) != cudaSuccess) return fail("cudaMallocHost", e);
     if ((e = cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming)) != cudaSuccess) return fail("cudaEventCreate", e);
-    cudaDeviceGetAttribute(&h->n_sms, cudaDevAttrMultiProcessorCount, cfg->device);
+    cudaDeviceGetAttribute(&h->load.n_sms, cudaDevAttrMultiProcessorCount, cfg->device);
     {
         int max_hot = 0;
         for (int q = 0; q < N_CLASSES; ++q)
-            for (int gs = 0; gs <= 5; ++gs) max_hot = std::max(max_hot, g_classes(q).hot_bytes(gs));
+            for (int gs = 0; gs <= 5; ++gs) max_hot = std::max(max_hot, class_hot_bytes(q, gs));
         if ((e = rem2d_set_kernel_attributes(max_hot)) != cudaSuccess) return fail("cudaFuncSetAttribute", e);
-        for (int im = 0; im < 2; ++im) h->max_warps_per_sm[im] = std::max(1, rem2d_episode_blocks_per_sm(im, 1024));
+        for (int im = 0; im < 2; ++im) h->load.max_warps_per_sm[im] = std::max(1, rem2d_episode_blocks_per_sm(im, 1024));
     }
     *out = h;
     return REM2D_OK;
@@ -384,136 +344,6 @@ static cudaError_t upload_array(rem2d_handle* h, int slot, const T* src, size_t 
 
 static int launch_reset(rem2d_handle* h);
 
-// Resident warps of the persistent episode kernels for the current group shifts (h->cur_gs). All classes run concurrently, so
-// the shared memory of the SMs (227 KB each) and the resident-warp limit set by the register file are divided among them in
-// proportion to their work; a class never gets more warps than it has creatures, and what it cannot use is handed to the
-// others. Without this the largest class would occupy every SM until its last creature dies and the remaining classes would
-// run after it. Returns true iff EVERY creature of every class has a group from the start (one round, under-filled GPU).
-static bool size_grids(rem2d_handle* h, double warp_frac = 0.97) {
-    const double smem_kb = h->opt.smem_budget_kb;
-    double budget = (double)h->n_sms * smem_kb * 1024.0 * 0.98 * h->first_wave_frac;
-    double work[N_CLASSES], smem[N_CLASSES];
-    bool fixed[N_CLASSES];
-    for (int k = 0; k < N_CLASSES; ++k) {
-        const int gs = h->cur_gs[k];
-        work[k] = h->cls[k].work; fixed[k] = h->cls[k].n_members == 0; smem[k] = g_classes(k).hot_bytes(gs) + 1024.0;
-        // a group of G lanes is one resident creature: G times the warps for the same residency, and the creature ticks
-        // p(G) times faster (measured tick latencies, profiles/r2_timeline_*.txt)
-        static const double speedup[6] = {1.0, 1.15, 1.5, 1.9, 2.2, 2.5};
-        work[k] *= (double)(1 << gs) / speedup[gs];
-        h->cls[k].episode_grid = 0;
-    }
-    // warps_k = W * work_k with W such that sum_k warps_k * smem_k = budget: every class then needs about the same
-    // number of sequential creature-lifetimes per group times its own tick latency, i.e. the classes finish together.
-    // The register file bounds the resident warps as well (h->max_warps_per_sm, from the occupancy API): a launch whose
-    // CTAs do not fit waits for the CTAs of the classes launched before it to EXIT, which serialises the classes
-    // (measured: the small classes started 400 ms late when 9 warps per SM fit and the grids asked for 9.7).
-    double warp_budget = (double)h->n_sms * h->max_warps_per_sm[h->image] * warp_frac;
-    bool all_fit = true;
-    for (int round = 0; round <= N_CLASSES; ++round) {
-        double denom = 0.0, wsum = 0.0;
-        for (int k = 0; k < N_CLASSES; ++k) if (!fixed[k]) { denom += work[k] * smem[k]; wsum += work[k]; }
-        if (denom <= 0.0) break;
-        const double W = std::max(0.0, std::min(budget / denom, warp_budget / wsum));
-        bool changed = false;
-        for (int k = 0; k < N_CLASSES; ++k) {
-            if (fixed[k]) continue;
-            const int per = 32 >> h->cur_gs[k], need = (h->cls[k].n_members + per - 1) / per;    // one group per creature
-            if ((int)(W * work[k]) >= need) {        // the class fits entirely: fix it and give the rest back
-                h->cls[k].episode_grid = need;
-                budget -= need * smem[k];
-                warp_budget -= need;
-                fixed[k] = true; changed = true;
-            }
-        }
-        if (!changed) {
-            for (int k = 0; k < N_CLASSES; ++k)
-                if (!fixed[k]) { h->cls[k].episode_grid = std::max(1, (int)(W * work[k])); all_fit = false; }
-            break;
-        }
-    }
-    for (int k = 0; k < N_CLASSES; ++k)
-        if (h->cls[k].n_members && h->cls[k].episode_grid < 1) h->cls[k].episode_grid = 1;
-    return all_fit;
-}
-
-// Lanes per creature of every class for the uploaded population, then the grids. Throughput and latency pull in opposite
-// directions: one lane per creature issues the fewest instructions per creature-tick, a group of G lanes ticks a creature
-// up to ~2x faster but spends more issue slots on it (idle lanes in the sweeps, leader sections). Measured on B200
-// (tools/sweep_groups.py): with 65536 creatures the GPU is throughput-bound and G = 1 everywhere is fastest; when the
-// population leaves the GPU under-filled (every creature resident from the start) the run time is one creature lifetime
-// times the tick latency, and wider groups win. So: start from G = 1 and widen the groups of the large classes (up to the
-// class table's value) as long as every creature of every class still has a group from the start. Explicit options
-// ("group_shift", "class_gs_<k>") override the choice.
-static void choose_groups_and_grids(rem2d_handle* h) {
-    bool forced[N_CLASSES];
-    for (int k = 0; k < N_CLASSES; ++k) {
-        const int o = h->opt.group_shift >= 0 ? h->opt.group_shift : h->opt.class_gs[k];
-        forced[k] = o >= 0;
-        h->cur_gs[k] = forced[k] ? std::min(5, o) : 0;
-    }
-    // under-filled GPU <=> everything fits with one lane per creature in the 128-register image: then widen (below)
-    h->image = 1;
-    h->first_wave_frac = 1.0;
-    bool all_fit = size_grids(h);
-    if (!all_fit) {
-        // Throughput-bound: one lane per creature - except the largest class (33-44 bodies): its 4.6 KB of solver state per
-        // creature make a 32-creature CTA 148 KB of shared memory, ONE resident warp per SM at a 5 ms tick. 8 lanes per creature
-        // (4 creatures, 19 KB per CTA) pack the same residency into warps that tick twice as fast and fit beside the other
-        // classes' CTAs. Measured on EA-configured populations (max_size 40; tools/ea_pop_sweep.py, profiles/r2_ea_pop_sweep.txt):
-        // 1.5-1.6x on the whole evaluation (1946 -> 1271 ms, 3311 -> 2112, 5925 -> 3676); widening the 23-32 body class as well
-        // gains nothing, the smaller classes lose (the bench population, <= 21 bodies, is unaffected).
-        for (int k = 0; k < N_CLASSES; ++k)
-            if (!forced[k]) h->cur_gs[k] = g_classes(k).nb > 32 ? 3 : 0;
-        h->image = h->opt.image >= 0 ? h->opt.image : 0;
-        size_grids(h);
-        // Mixed widths: the cost model's tick latencies are those of one-lane warps on moderately loaded SMs; next to
-        // hundreds of 8-lane warps the one-lane classes tick 2x slower than modelled (4.8 ms against 1.55 ms for the wide
-        // class) and a first wave that asks for all of the shared memory does not even fit (736 of 822 CTAs resident,
-        // the launches behind them held back). With an overflow wave it is better to seat 75 % statically and let the
-        // queued CTAs take the rest as it frees up: 3560 -> 2610 ms, 1930 -> 1600, 1155 -> 1130 ms on the three
-        // EA-configured populations; all-one-lane populations (the bench) lose 4 % with it and keep the full first wave.
-        bool mixed = false;
-        for (int k = 0; k < N_CLASSES; ++k) mixed |= h->cls[k].n_members > 0 && h->cur_gs[k] > 0;
-        if (mixed && h->opt.overflow_wave && h->opt.smem_budget_kb > 226.0) {
-            h->first_wave_frac = 0.75;
-            size_grids(h);
-        }
-    }
-    for (int k = 0; k < N_CLASSES; ++k) { h->cls[k].grid2 = 0; h->cls[k].gs2 = 0; }
-    if (!all_fit) {
-        // Throughput-bound population: one lane per creature, lanes refilled from the class queue.
-        // OVERFLOW WAVE (default): the first-wave grids above come from a static cost model; when it is off for a population -
-        // measured on an EA-configured one: the 33-44 body class done after 1.9 s, the others at 3.1-3.6 s, with the freed 18 MB
-        // of shared memory idle in between (profiles/r2_timeline_ea_gen2_before.txt) - nothing could use the resources of a
-        // class that has finished. So every class also queues, BEHIND all first launches, the CTAs it could not seat: the
-        // work distributor places them as earlier CTAs exit, they pull from the same class queue, and a CTA that finds its
-        // queue empty exits at once. The hardware does the balancing.
-        if (h->opt.overflow_wave) {
-            for (int k = 0; k < N_CLASSES; ++k) {
-                ClassState& cs = h->cls[k];
-                const int per = 32 >> h->cur_gs[k];
-                const int left = cs.n_members - cs.episode_grid * per;
-                if (!cs.n_members || left <= 0) continue;
-                cs.gs2 = h->cur_gs[k];
-                cs.grid2 = (left + per - 1) / per;
-            }
-        }
-        return;
-    }
-    // widest uniform group width (capped per class) with which every creature has a group from the start AND the warps fill
-    // at most 60 % of the resident-warp limit: wide groups are issue-bound before the SMs are full. Measured optimum
-    // (tools/small_pop.py): 16384 creatures -> 4 lanes, 8192 -> 8, 4096 -> 8-16, <= 1024 -> 32
-    for (int gs = 5; gs >= 1; --gs) {
-        for (int k = 0; k < N_CLASSES; ++k)
-            if (!forced[k]) h->cur_gs[k] = std::min(gs, g_classes(k).gs);
-        if (size_grids(h, 0.6)) { size_grids(h); return; }
-    }
-    for (int k = 0; k < N_CLASSES; ++k)
-        if (!forced[k]) h->cur_gs[k] = 0;
-    size_grids(h);
-}
-
 static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_reset) {
     if (!h || !pop) return REM2D_E_INVALID;
     if (pop->n_creatures < 0 || pop->n_joints != pop->n_bodies - pop->n_creatures) { h->err = "upload: inconsistent counts"; return REM2D_E_INVALID; }
@@ -530,8 +360,8 @@ static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_res
         int nb = pop->body_off[c + 1] - pop->body_off[c];
         if (nb < 1) { h->err = "upload: creature without a root body"; return REM2D_E_INVALID; }
         int k = -1;
-        for (int q = 0; q < N_CLASSES; ++q) if (nb <= g_classes(q).nb) { k = q; break; }
-        if (k < 0) { char buf[128]; snprintf(buf, sizeof(buf), "upload: creature %d has %d bodies (> %d supported)", c, nb, g_classes(N_CLASSES - 1).nb); h->err = buf; return REM2D_E_CAPACITY; }
+        for (int q = 0; q < N_CLASSES; ++q) if (nb <= class_dims[q].nb) { k = q; break; }
+        if (k < 0) { char buf[128]; snprintf(buf, sizeof(buf), "upload: creature %d has %d bodies (> %d supported)", c, nb, class_dims[N_CLASSES - 1].nb); h->err = buf; return REM2D_E_CAPACITY; }
         int j0 = pop->body_off[c] - c;
         for (int j = 0; j < nb - 1; ++j)
             if (pop->joint_parent[j0 + j] < 0 || pop->joint_parent[j0 + j] > j) { h->err = "upload: joint parent must precede its child"; return REM2D_E_INVALID; }
@@ -586,7 +416,6 @@ static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_res
         ClassState& cs = h->cls[k];
         cs.n_batches = (int)((m.size() + 31) / 32);
         cs.n_members = (int)m.size();
-        cs.episode_grid = cs.n_batches;     // sized below once every class is known
         cs.lane_creature.assign((size_t)cs.n_batches * 32, -1);
         for (size_t i = 0; i < m.size(); ++i) { cs.lane_creature[i] = m[i]; h->creature_lane[m[i]] = (int)i; }
         const size_t lane_bytes = cs.lane_creature.size() * sizeof(int);
@@ -600,14 +429,14 @@ static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_res
         CK(ensure(cs.b_small, 64)); cs.d_park_count = (int*)cs.b_small.p; cs.d_queue = (int*)cs.b_small.p + 4;
         if (!cs.h_park_count) CK(cudaMallocHost(&cs.h_park_count, sizeof(int)));
     }
-    {   // per-creature cost ~ tick latency of its size: measured ~0.3 ms + 0.085 ms per body for a resident warp; lone bodies
-        // fall asleep after landing and cost almost nothing
-        for (int k = 0; k < N_CLASSES; ++k) {
-            h->cls[k].work = 0.0;
-            for (int c : members[k]) { int nbc = pop->body_off[c + 1] - pop->body_off[c]; h->cls[k].work += nbc == 1 ? 1.0 : 3.5 + nbc; }
-        }
-        choose_groups_and_grids(h);
+    // per-creature cost ~ tick latency of its size: measured ~0.3 ms + 0.085 ms per body for a resident warp; lone bodies
+    // fall asleep after landing and cost almost nothing
+    for (int k = 0; k < N_CLASSES; ++k) {
+        h->load.members[k] = h->cls[k].n_members;
+        h->load.work[k] = 0.0;
+        for (int c : members[k]) { int nbc = pop->body_off[c + 1] - pop->body_off[c]; h->load.work[k] += nbc == 1 ? 1.0 : 3.5 + nbc; }
     }
+    h->plan = plan_upload(h->load, h->opt);
     {
         const size_t nn = (size_t)std::max(n, 1);
         CK(ensure(h->b_results, nn * (sizeof(double) + 3 * sizeof(int))));
@@ -645,7 +474,7 @@ static int launch_reset(rem2d_handle* h) {
     for (int k = N_CLASSES - 1; k >= 0; --k) {
         ClassState& cs = h->cls[k];
         if (!cs.n_batches) continue;
-        g_classes(k).reset(step_gs(h, k), cs.n_batches, cs.stream, cs.d_state, cs.d_lane_creature, h->dpop);
+        g_classes(k).reset(step_group_shift(h->load, k, h->opt), cs.n_batches, cs.stream, cs.d_state, cs.d_lane_creature, h->dpop);
         h->launches++;
     }
     CK(cudaGetLastError());
@@ -682,7 +511,7 @@ static int promote_overflowed(rem2d_handle* h, int max_ticks) {
         for (int k = 0; k < N_CLASSES; ++k) {
             if (redo[k].empty()) continue;
             ClassState& cs = h->cls[k];
-            const int gs = class_gs(h, k), per = 32 >> gs;
+            const int gs = h->plan.gs[k], per = 32 >> gs;
             const int grid = (int)((redo[k].size() + per - 1) / per), batches = (int)((redo[k].size() + 31) / 32);
             CK(ensure(cs.b_redo_order, sizeof(int) * (redo[k].size() + 1)));
             CK(ensure(cs.b_redo_slots, (size_t)batches * g_classes(k).words * 32 * sizeof(float)));
@@ -690,7 +519,7 @@ static int promote_overflowed(rem2d_handle* h, int max_ticks) {
             int* d_queue = d_order + redo[k].size();
             CK(cudaMemcpyAsync(d_order, redo[k].data(), sizeof(int) * redo[k].size(), cudaMemcpyHostToDevice, h->user_stream));
             CK(cudaMemsetAsync(d_queue, 0, sizeof(int), h->user_stream));
-            g_classes(k).episode(h->image, gs, grid, h->user_stream, (float*)cs.b_redo_slots.p, d_order, (int)redo[k].size(), d_queue, h->dpop, h->d_ter,
+            g_classes(k).episode(h->plan.image, gs, grid, h->user_stream, (float*)cs.b_redo_slots.p, d_order, (int)redo[k].size(), d_queue, h->dpop, h->d_ter,
                                  h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
                                  ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr}, nullptr, nullptr, nullptr);
             h->launches++;
@@ -704,56 +533,23 @@ static int promote_overflowed(rem2d_handle* h, int max_ticks) {
 // Whole episodes for the uploaded population on the persistent episode kernels (one per class, concurrent).
 static int launch_episodes(rem2d_handle* h, int max_ticks) {
     if (!h->have_terrain) { h->err = "run_episodes: no terrain set"; return REM2D_E_INVALID; }
-    // creatures still alive after park_ticks are finished by tail-mode launches (REM2D_PARK_TICKS=0 disables parking)
-    // Measured on B200 (tools/sweep_groups.py, 65536 L-system creatures): parking at 200-256 ticks (~0.5-1.4 % of the creatures)
-    // is the best trade: a tail warp finishes a creature 3-4x sooner than its bulk lane would, but it occupies a whole warp, so
-    // earlier thresholds (thousands of parked creatures) slow the bulk down more than they shorten the critical path; later
-    // ones leave the longest-lived creatures on the slow path. Drain / late-start parking never paid off. The number of
-    // parked creatures per class is bounded (a quarter of the class, at most 16 per SM): in an evolved population where most creatures live
-    // long, the rest simply stay on their lanes.
-    int park_ticks = 200;            // measured (tools/sweep_groups.py, 65536 creatures): 256 -> 820 ms, 200 -> 790 ms, 160 -> 930 ms
-    double cap_frac = 0.25;
-    {   // Under-filled GPU (every creature of every class has a group from the start, e.g. 16384 creatures): tail warps find
-        // free SM resources, so parking earlier pays (16384 creatures: 450 -> 413 ms with 160 ticks and a quarter of a class).
-        bool single_round = true;
-        for (int k = 0; k < N_CLASSES; ++k) {
-            const int per = 32 >> class_gs(h, k);
-            if (h->cls[k].n_batches && h->cls[k].episode_grid * per < h->cls[k].n_members) single_round = false;
-        }
-        if (single_round) { park_ticks = 160; cap_frac = 0.25; }
-    }
-    if (h->opt.park_ticks >= 0) park_ticks = h->opt.park_ticks;
-    if (h->opt.park_cap >= 0.0) cap_frac = h->opt.park_cap;
+    const LaunchPlan lp = plan_launch(h->load, h->plan, max_ticks, h->opt);
+    const bool trace = h->opt.trace != 0;
+    auto park_policy = [&](int k) {
+        return ParkPolicy{lp.park_ticks, lp.park_cap[k], 0.0f, 0, h->cls[k].n_members, lp.park_ticks, nullptr,
+                          trace ? (unsigned int*)h->cls[k].b_ttrace.p : nullptr};
+    };
     CK(cudaMemsetAsync(h->d_counters, 0, sizeof(unsigned long long) * N_COUNTER_WORDS, h->user_stream));
     CK(cudaEventRecord(h->ev_start, h->user_stream));
     int rc = fork_streams(h);
     if (rc) return rc;
-    // Small populations: one warp per creature from tick 0 (mode 2). All creatures then advance at the low tail-mode tick
-    // latency and the run takes about one creature lifetime. Measured (tools/small_pop.py, L-system creatures): 2.4x faster
-    // than the bulk mode at 128 creatures, 1.9x at 1024, 1.2x at 6144, break-even near 10^4, 0.6x at 16384 (the bulk mode has
-    // 32x the lane efficiency).
-    const int warp_mode_max = h->opt.warp_mode_max >= 0 ? h->opt.warp_mode_max : h->n_sms * 48;
-    const bool warp_mode = h->n_creatures <= warp_mode_max;
-    if (warp_mode) park_ticks = 0;
-    const bool trace = h->opt.trace != 0;
-    // Launch order = decreasing shared memory per CTA (first-fit decreasing): the work distributor places the CTAs of the
-    // launches in order, and a CTA that finds no SM with enough free shared memory holds back every launch behind it.
-    // Measured (profiles/r2_timeline_ea_gen2_before.txt): with the 33-44 body class at 8 lanes per creature (22 KB per CTA)
-    // launched first, its 822 CTAs left < 109 KB free on every SM, the 23-32 body class (109 KB per CTA) could not start, and
-    // all seven smaller classes waited behind it until the first launch had finished (1.3 s of a 3.8 s evaluation).
-    int launch_order[N_CLASSES];
-    for (int k = 0; k < N_CLASSES; ++k) launch_order[k] = k;
-    std::stable_sort(launch_order, launch_order + N_CLASSES, [&](int a, int b) {
-        const size_t sa = g_classes(a).hot_bytes(warp_mode ? 5 : class_gs(h, a)), sb = g_classes(b).hot_bytes(warp_mode ? 5 : class_gs(h, b));
-        return sa != sb ? sa > sb : a > b;
-    });
     for (int oi = 0; oi < N_CLASSES; ++oi) {
-        const int k = launch_order[oi];
+        const int k = lp.order[oi];
         ClassState& cs = h->cls[k];
         if (!cs.n_batches) continue;
         CK(cudaMemsetAsync(cs.d_queue, 0, sizeof(int), cs.stream));
         CK(cudaEventRecord(cs.t_begin, cs.stream));
-        if (warp_mode) {      // queue mode with a whole warp per creature and one warp for every creature
+        if (lp.warp_mode) {      // queue mode with a whole warp per creature and one warp for every creature
             g_classes(k).episode(1, 5, cs.n_members, cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop, h->d_ter,
                                  h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
                                  ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr}, nullptr, nullptr, nullptr);
@@ -763,25 +559,18 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         }
         CK(cudaMemsetAsync(cs.d_park_count, 0, sizeof(int), cs.stream));
         CK(cudaMemsetAsync(cs.d_park_creature, 0, cs.lane_creature.size() * sizeof(int), cs.stream));     // "unpublished" markers
-        ParkPolicy park;
-        park.ticks = park_ticks < max_ticks ? park_ticks : 0;
-        park.cap = std::min(cs.n_members, std::max(32, std::min((int)(h->n_sms * 64 * cap_frac), (int)(cs.n_members * cap_frac))));
-        park.lead_x = 0.0f; park.lead_from = 0;
-        park.late_from = cs.n_members; park.late_ticks = park.ticks;
-        park.trace = nullptr; park.tail_trace = nullptr;
         if (trace) {
             const size_t tb = (size_t)std::max(cs.n_members, 1) * 4 * sizeof(unsigned int);
             CK(ensure(cs.b_ttrace, tb));
             CK(cudaMemsetAsync(cs.b_ttrace.p, 0, tb, cs.stream));
-            park.tail_trace = (unsigned int*)cs.b_ttrace.p;
-            const size_t bytes = (size_t)cs.episode_grid * REM2D_TRACE_SAMPLES * 2 * sizeof(unsigned int);
+            const size_t bytes = (size_t)h->plan.grid[k] * REM2D_TRACE_SAMPLES * 2 * sizeof(unsigned int);
             CK(ensure(cs.b_trace, bytes));
             CK(cudaMemsetAsync(cs.b_trace.p, 0, bytes, cs.stream));
-            park.trace = (unsigned int*)cs.b_trace.p;
         }
-        if (cs.grid2 > 0) { CK(cudaEventRecord(cs.done2, cs.stream)); CK(cudaStreamWaitEvent(cs.stream2, cs.done2, 0)); }   // queue / park counters are reset
-        cs.park = park;
-        g_classes(k).episode(h->image, class_gs(h, k), cs.episode_grid, cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop,
+        ParkPolicy park = park_policy(k);
+        if (trace) park.trace = (unsigned int*)cs.b_trace.p;
+        if (h->plan.grid2[k] > 0) { CK(cudaEventRecord(cs.done2, cs.stream)); CK(cudaStreamWaitEvent(cs.stream2, cs.done2, 0)); }   // queue / park counters are reset
+        g_classes(k).episode(h->plan.image, h->plan.gs[k], h->plan.grid[k], cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop,
                              h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
                              park, cs.d_park_state, cs.d_park_creature, cs.d_park_count);
         // Nothing reads this copy, but it shapes the tail launches: without it the bench population gets twice the tail
@@ -792,21 +581,19 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
     }
     // overflow waves (after ALL first launches, so that their CTAs queue behind them): the creatures a class could not seat
     // in its first round, on the columns behind the first launch's
-    for (int oi = 0; oi < N_CLASSES && !warp_mode; ++oi) {
-        const int k = launch_order[oi];
+    for (int oi = 0; oi < N_CLASSES && !lp.warp_mode; ++oi) {
+        const int k = lp.order[oi];
         ClassState& cs = h->cls[k];
-        if (!cs.n_batches || cs.grid2 <= 0) continue;
-        const int per1 = 32 >> class_gs(h, k);
-        const size_t first_block = ((size_t)cs.episode_grid * per1 + 31) / 32;
-        ParkPolicy park = cs.park;
-        park.trace = nullptr;
-        g_classes(k).episode(h->image, cs.gs2, cs.grid2, cs.stream2, cs.d_state + first_block * g_classes(k).words * 32, cs.d_lane_creature, cs.n_members,
+        if (!cs.n_batches || h->plan.grid2[k] <= 0) continue;
+        const int gs = h->plan.gs[k];
+        const size_t first_block = ((size_t)h->plan.grid[k] * (32 >> gs) + 31) / 32;
+        g_classes(k).episode(h->plan.image, gs, h->plan.grid2[k], cs.stream2, cs.d_state + first_block * g_classes(k).words * 32, cs.d_lane_creature, cs.n_members,
                              cs.d_queue, h->dpop, h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status,
-                             h->d_counters, park, cs.d_park_state, cs.d_park_creature, cs.d_park_count);
+                             h->d_counters, park_policy(k), cs.d_park_state, cs.d_park_creature, cs.d_park_count);
         h->launches++;
     }
     CK(cudaGetLastError());
-    if (park_ticks > 0 && park_ticks < max_ticks) {
+    if (lp.park_ticks > 0) {
         // Tail: while the episode kernels run, poll their park counters and hand newly parked creatures to the
         // warp-per-creature tail mode right away (pool of streams), so the sequential ticks of the longest-lived
         // creatures overlap the bulk instead of extending the run; the last launch of a class happens when its episode
@@ -839,7 +626,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
                 finished_now[k] = false;
                 if (!running[k]) continue;
                 cudaError_t q = cudaStreamQuery(h->cls[k].stream);       // BEFORE reading the counter: no slot can be missed
-                if (q == cudaSuccess && h->cls[k].grid2 > 0) q = cudaStreamQuery(h->cls[k].stream2);
+                if (q == cudaSuccess && h->plan.grid2[k] > 0) q = cudaStreamQuery(h->cls[k].stream2);
                 if (q == cudaSuccess) finished_now[k] = true;
                 else if (q != cudaErrorNotReady) { h->err = std::string("episode kernel: ") + cudaGetErrorString(q); return REM2D_E_CUDA; }
                 CK(cudaMemcpyAsync(&h->h_poll[k], h->cls[k].d_park_count, sizeof(int), cudaMemcpyDeviceToHost, h->poll_stream));
@@ -856,7 +643,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
                     // a handful of parked creatures (random populations): a warp each; dozens at once (evolved populations,
                     // where many creatures outlive the threshold): 8 lanes each - 4x fewer warps at nearly the same tick latency
                     const int tail_gs = (cnt - launched[k] >= 32) ? std::min(3, h->opt.tail_group_shift) : h->opt.tail_group_shift;
-                    g_classes(k).tail(h->image, tail_gs, idle_stream(), cs.d_park_state, cs.d_park_creature, launched[k], cnt - launched[k],
+                    g_classes(k).tail(h->plan.image, tail_gs, idle_stream(), cs.d_park_state, cs.d_park_creature, launched[k], cnt - launched[k],
                                       h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
                                       trace ? (unsigned int*)cs.b_ttrace.p : nullptr);
                     CK(cudaGetLastError());
@@ -929,7 +716,7 @@ int rem2d_step(rem2d_handle* h, int32_t n_ticks) {
     for (int k = N_CLASSES - 1; k >= 0; --k) {        // most expensive class first
         ClassState& cs = h->cls[k];
         if (!cs.n_batches) continue;
-        g_classes(k).step(step_gs(h, k), cs.n_batches, cs.stream, cs.d_state, n_ticks, h->d_ter, h->d_consts, h->d_counters);
+        g_classes(k).step(step_group_shift(h->load, k, h->opt), cs.n_batches, cs.stream, cs.d_state, n_ticks, h->d_ter, h->d_consts, h->d_counters);
         h->launches++;
     }
     CK(cudaGetLastError());
@@ -1036,7 +823,7 @@ int rem2d_debug_class_timeline(rem2d_handle* h, float* out) {
         ClassState& cs = h->cls[k];
         float b = -1.0f, e = -1.0f;
         if (cs.n_batches) { cudaEventElapsedTime(&b, h->ev_start, cs.t_begin); cudaEventElapsedTime(&e, h->ev_start, cs.t_end); }
-        out[5 * k] = (float)g_classes(k).nb; out[5 * k + 1] = (float)cs.n_members; out[5 * k + 2] = (float)cs.episode_grid;
+        out[5 * k] = (float)class_dims[k].nb; out[5 * k + 1] = (float)cs.n_members; out[5 * k + 2] = (float)h->plan.grid[k];
         out[5 * k + 3] = b; out[5 * k + 4] = e;
     }
     cudaGetLastError();
@@ -1051,10 +838,10 @@ int rem2d_debug_trace(rem2d_handle* h, int k, unsigned int* out, int64_t max_wor
     if (!cs.b_trace.p || !cs.n_batches) return 0;
     cudaSetDevice(h->cfg.device);
     cudaDeviceSynchronize();
-    size_t words = (size_t)cs.episode_grid * REM2D_TRACE_SAMPLES * 2;
+    size_t words = (size_t)h->plan.grid[k] * REM2D_TRACE_SAMPLES * 2;
     if ((int64_t)words > max_words) words = (size_t)max_words;
     CK(cudaMemcpy(out, cs.b_trace.p, words * sizeof(unsigned int), cudaMemcpyDeviceToHost));
-    return cs.episode_grid;
+    return h->plan.grid[k];
 }
 
 // Diagnostics: per park slot {us parked, us tail start, us tail end, tail ticks} of class k (REM2D_TRACE=1). Returns #slots.

@@ -9,7 +9,6 @@ from gym_rem2d_b200.capi import Config, Engine, Population, load_library, N_COUN
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB = os.path.join(HERE, "librem2d_emu.so")
-CLASSES = [(1, 10, 3), (2, 16, 4), (4, 28, 4), (8, 48, 6), (12, 64, 6), (16, 80, 6), (22, 104, 6), (32, 144, 8), (44, 192, 10)]
 
 
 class EmuOut(C.Structure):
@@ -33,14 +32,54 @@ def lib():
         _lib = C.CDLL(build())
         _lib.rem2d_emu_run.argtypes = [C.POINTER(Population), C.c_void_p, C.c_int, C.c_double, C.POINTER(Config), C.c_int, C.c_int,
                                        C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.POINTER(EmuOut)]
+        _lib.rem2d_emu_classes.argtypes = [C.c_void_p]
+        _lib.rem2d_emu_plan.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
     return _lib
 
 
+_classes = None
+
+
+def classes():
+    """The capacity classes of the CUDA library: (bodies, contact-pool slots, staged touching contacts, widest group shift)."""
+    global _classes
+    if _classes is None:
+        out = np.zeros((64, 4), np.int32)
+        n = lib().rem2d_emu_classes(out.ctypes.data)
+        _classes = [tuple(int(v) for v in row) for row in out[:n]]
+    return _classes
+
+
 def class_of(nb):
-    for cl in CLASSES:
+    for cl in classes():
         if nb <= cl[0]:
             return cl
     raise ValueError(nb)
+
+
+# the Options fields the planner reads, in the order rem2d_emu_plan takes them (rem2d_set_option names)
+PLAN_OPTIONS = ("warp_mode_max", "park_ticks", "park_cap", "overflow_wave", "image", "smem_budget_kb", "group_shift")
+
+
+def plan(members, work, options=None, max_ticks=10000, n_sms=148, max_warps_per_sm=(9, 16)):
+    """The CUDA library's episode plan for a population with `members` creatures and a cost estimate of `work` per capacity
+    class, on `n_sms` SMs with `max_warps_per_sm` resident warps per SM for the two kernel images, with the planner options
+    `options` (a dict: PLAN_OPTIONS and "class_gs_<k>"; the library's defaults for the rest)."""
+    L, n = lib(), len(classes())
+    members, work = np.ascontiguousarray(members, np.int32), np.ascontiguousarray(work, np.float64)
+    assert members.shape == (n,) and work.shape == (n,)
+    warps = np.ascontiguousarray(max_warps_per_sm, np.int32)
+    names = PLAN_OPTIONS + tuple("class_gs_%d" % k for k in range(n))
+    unknown = set(options or {}) - set(names)
+    if unknown:
+        raise ValueError("not a planner option: %s" % sorted(unknown))
+    opt = np.array([(options or {}).get(k, np.nan) for k in names], np.float64)
+    out = np.zeros(4 + 6 * n, np.int32)
+    L.rem2d_emu_plan(n_sms, warps.ctypes.data, members.ctypes.data, work.ctypes.data, opt.ctypes.data, int(max_ticks),
+                     out.ctypes.data)
+    cols = out[4:].reshape(6, n)
+    return dict(image=int(out[0]), all_fit=bool(out[1]), warp_mode=bool(out[2]), park_ticks=int(out[3]),
+                **{k: cols[i].tolist() for i, k in enumerate(("gs", "grid", "grid2", "park_cap", "order", "step_gs"))})
 
 
 def run(pop, ys, step, creatures, gs, n_ticks, max_pairs=24, klass=None, **cfg_over):

@@ -1,7 +1,8 @@
 // rem2d_emu.cpp — TEST INFRASTRUCTURE: runs gym_rem2d_b200/csrc/rem2d_device.cuh (the device code of the CUDA kernels) on
 // the CPU, one host thread per lane of a warp (see rem2d_emu_shim.h), so that the lane-group logic can be compared with the
 // oracle without a GPU. One call = one warp: up to 32 >> gs creatures, each owned by a group of 1 << gs lanes, stepped like
-// rem2d_step (reset + n ticks). Build: make -C tests/emu. Used by tests/test_emu.py only.
+// rem2d_step (reset + n ticks). Also exports the capacity classes and the episode planner of rem2d_host_util.h. Build:
+// make -C tests/emu. Used by tests/emu/emu.py only.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -26,6 +27,40 @@ struct EmuOut {                  // caller-allocated, concatenated over the crea
 };
 
 extern "C" int rem2d_emu_hot_rows(int NB, int NC, int NT, int gs) { return make_hot_layout(make_layout(NB, NC, NT), gs).rows; }
+
+// The capacity classes of the CUDA library: out[4 * k ..] = {nb, nc, nt, gs} of class k. Returns the number of classes.
+extern "C" int rem2d_emu_classes(int32_t* out) {
+    for (int k = 0; k < N_CLASSES; ++k) {
+        out[4 * k] = class_dims[k].nb; out[4 * k + 1] = class_dims[k].nc; out[4 * k + 2] = class_dims[k].nt; out[4 * k + 3] = class_dims[k].gs;
+    }
+    return N_CLASSES;
+}
+
+// The episode planner of the CUDA library (plan_upload, plan_launch, step_group_shift) for the given device and class sizes.
+// opt[] holds the Options fields the planner reads, in the order warp_mode_max, park_ticks, park_cap, overflow_wave, image,
+// smem_budget_kb, group_shift, class_gs[0..N_CLASSES); NaN keeps the default. out = {image, all_fit, warp_mode, park_ticks}
+// followed by N_CLASSES values each of gs, grid, grid2, park_cap, order and the stepping kernels' group shift.
+extern "C" int rem2d_emu_plan(int n_sms, const int32_t* max_warps_per_sm, const int32_t* members, const double* work,
+                              const double* opt, int max_ticks, int32_t* out) {
+    PlanInput in;
+    in.n_sms = n_sms;
+    for (int i = 0; i < 2; ++i) in.max_warps_per_sm[i] = max_warps_per_sm[i];
+    for (int k = 0; k < N_CLASSES; ++k) { in.members[k] = members[k]; in.work[k] = work[k]; }
+    Options o;
+    auto set = [&](int i, auto& field) { if (!std::isnan(opt[i])) field = opt[i]; };
+    set(0, o.warp_mode_max); set(1, o.park_ticks); set(2, o.park_cap); set(3, o.overflow_wave); set(4, o.image);
+    set(5, o.smem_budget_kb); set(6, o.group_shift);
+    for (int k = 0; k < N_CLASSES; ++k) set(7 + k, o.class_gs[k]);
+    const UploadPlan up = plan_upload(in, o);
+    const LaunchPlan lp = plan_launch(in, up, max_ticks, o);
+    out[0] = up.image; out[1] = up.all_fit; out[2] = lp.warp_mode; out[3] = lp.park_ticks;
+    for (int k = 0; k < N_CLASSES; ++k) {
+        int32_t* col = out + 4 + k;
+        col[0] = up.gs[k]; col[N_CLASSES] = up.grid[k]; col[2 * N_CLASSES] = up.grid2[k]; col[3 * N_CLASSES] = lp.park_cap[k];
+        col[4 * N_CLASSES] = lp.order[k]; col[5 * N_CLASSES] = step_group_shift(in, k, o);
+    }
+    return 0;
+}
 
 extern "C" int rem2d_emu_run(const rem2d_population* pop, const double* terrain_y, int n_vertices, double step, const rem2d_config* cfg,
                              int NB, int NC, int NT, int gs, const int32_t* creatures, int n, int n_ticks, EmuOut* out) {

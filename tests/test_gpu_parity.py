@@ -200,7 +200,7 @@ def test_inclined_terrain_and_no_sleep_bit_exact(tan_slope):
 
 # ---------------------------------------------------------------------------------------------------------------------
 # The PRODUCTION execution path at test size (VERDICT r1, item 1): persistent bulk warps whose lanes are REFILLED from the
-# class queue (episode_grid < n_batches), parking at 256 ticks with a 1/16 cap and on-demand tail launches that see
+# class queue (first-wave grid < n_batches), parking at 256 ticks with a 1/16 cap and on-demand tail launches that see
 # late-parked creatures. A small shared-memory budget forces several refill rounds with a few thousand creatures.
 def _oracle_eval(pop, ys, steps=K.EVALUATION_STEPS, **cfg):
     o = OracleEngine(threads=max(8, (__import__("os").cpu_count() or 8)), **cfg)
