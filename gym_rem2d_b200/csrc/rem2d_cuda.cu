@@ -519,9 +519,9 @@ static int promote_overflowed(rem2d_handle* h, int max_ticks) {
             int* d_queue = d_order + redo[k].size();
             CK(cudaMemcpyAsync(d_order, redo[k].data(), sizeof(int) * redo[k].size(), cudaMemcpyHostToDevice, h->user_stream));
             CK(cudaMemsetAsync(d_queue, 0, sizeof(int), h->user_stream));
-            g_classes(k).episode(h->plan.image, gs, grid, h->user_stream, (float*)cs.b_redo_slots.p, d_order, (int)redo[k].size(), d_queue, h->dpop, h->d_ter,
+            g_classes(k).episode(h->plan.image, gs, widest_group_shift(k, gs), grid, h->user_stream, (float*)cs.b_redo_slots.p, d_order, (int)redo[k].size(), d_queue, h->dpop, h->d_ter,
                                  h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr}, nullptr, nullptr, nullptr);
+                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr, 0}, nullptr, nullptr, nullptr);
             h->launches++;
             CK(cudaGetLastError());
             CK(cudaStreamSynchronize(h->user_stream));      // redo[] (pageable source of the copy) goes out of scope
@@ -537,7 +537,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
     const bool trace = h->opt.trace != 0;
     auto park_policy = [&](int k) {
         return ParkPolicy{lp.park_ticks, lp.park_cap[k], 0.0f, 0, h->cls[k].n_members, lp.park_ticks, nullptr,
-                          trace ? (unsigned int*)h->cls[k].b_ttrace.p : nullptr};
+                          trace ? (unsigned int*)h->cls[k].b_ttrace.p : nullptr, h->opt.tail_group_shift};
     };
     CK(cudaMemsetAsync(h->d_counters, 0, sizeof(unsigned long long) * N_COUNTER_WORDS, h->user_stream));
     CK(cudaEventRecord(h->ev_start, h->user_stream));
@@ -550,9 +550,9 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         CK(cudaMemsetAsync(cs.d_queue, 0, sizeof(int), cs.stream));
         CK(cudaEventRecord(cs.t_begin, cs.stream));
         if (lp.warp_mode) {      // queue mode with a whole warp per creature and one warp for every creature
-            g_classes(k).episode(1, 5, cs.n_members, cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop, h->d_ter,
+            g_classes(k).episode(1, 5, 5, cs.n_members, cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop, h->d_ter,
                                  h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr}, nullptr, nullptr, nullptr);
+                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr, 0}, nullptr, nullptr, nullptr);
             CK(cudaEventRecord(cs.t_end, cs.stream));
             h->launches++;
             continue;
@@ -570,7 +570,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         ParkPolicy park = park_policy(k);
         if (trace) park.trace = (unsigned int*)cs.b_trace.p;
         if (h->plan.grid2[k] > 0) { CK(cudaEventRecord(cs.done2, cs.stream)); CK(cudaStreamWaitEvent(cs.stream2, cs.done2, 0)); }   // queue / park counters are reset
-        g_classes(k).episode(h->plan.image, h->plan.gs[k], h->plan.grid[k], cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop,
+        g_classes(k).episode(h->plan.image, h->plan.gs[k], widest_group_shift(k, h->plan.gs[k]), h->plan.grid[k], cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop,
                              h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
                              park, cs.d_park_state, cs.d_park_creature, cs.d_park_count);
         // Nothing reads this copy, but it shapes the tail launches: without it the bench population gets twice the tail
@@ -587,7 +587,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         if (!cs.n_batches || h->plan.grid2[k] <= 0) continue;
         const int gs = h->plan.gs[k];
         const size_t first_block = ((size_t)h->plan.grid[k] * (32 >> gs) + 31) / 32;
-        g_classes(k).episode(h->plan.image, gs, h->plan.grid2[k], cs.stream2, cs.d_state + first_block * g_classes(k).words * 32, cs.d_lane_creature, cs.n_members,
+        g_classes(k).episode(h->plan.image, gs, widest_group_shift(k, gs), h->plan.grid2[k], cs.stream2, cs.d_state + first_block * g_classes(k).words * 32, cs.d_lane_creature, cs.n_members,
                              cs.d_queue, h->dpop, h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status,
                              h->d_counters, park_policy(k), cs.d_park_state, cs.d_park_creature, cs.d_park_count);
         h->launches++;
@@ -643,7 +643,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
                     // a handful of parked creatures (random populations): a warp each; dozens at once (evolved populations,
                     // where many creatures outlive the threshold): 8 lanes each - 4x fewer warps at nearly the same tick latency
                     const int tail_gs = (cnt - launched[k] >= 32) ? std::min(3, h->opt.tail_group_shift) : h->opt.tail_group_shift;
-                    g_classes(k).tail(h->plan.image, tail_gs, idle_stream(), cs.d_park_state, cs.d_park_creature, launched[k], cnt - launched[k],
+                    g_classes(k).tail(h->plan.image, tail_gs, widest_group_shift(k, tail_gs), idle_stream(), cs.d_park_state, cs.d_park_creature, launched[k], cnt - launched[k],
                                       h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
                                       trace ? (unsigned int*)cs.b_ttrace.p : nullptr);
                     CK(cudaGetLastError());

@@ -25,6 +25,9 @@
 #pragma once
 #ifdef REM2D_EMU
 #include "rem2d_emu_shim.h"      // tests/emu: lanes are host threads (test infrastructure, never a product path)
+// the two atomics of the park hand-over in Sim::episodes, which the emulation (parking off) compiles but never executes
+inline int atomicCAS(int* p, int cmp, int v) { __atomic_compare_exchange_n(p, &cmp, v, false, __ATOMIC_ACQ_REL, __ATOMIC_ACQUIRE); return cmp; }
+inline int atomicExch(int* p, int v) { return __atomic_exchange_n(p, v, __ATOMIC_ACQ_REL); }
 #else
 #include <cuda_runtime.h>
 #endif
@@ -206,6 +209,32 @@ struct DevPop {
 };
 // work counters kept in registers and flushed once per launch
 struct Cnt { unsigned int c[REM2D_N_COUNTERS]; };   // per lane per launch; summed into 64-bit totals
+
+// When the queue-mode episode kernel hands a creature over to the tail mode (launches of the same kernel).
+struct ParkPolicy {
+    int ticks;        // park a creature that is still alive after this many ticks (0: never park)
+    int cap;          // at most this many creatures of the class are parked
+    // Always off (lead_x = 0, late_from = class size): the rejected lead and late-start park tests of the episode kernel.
+    // Deleting them takes episode_kernel from 202 to 200 registers; at 200, 10 instead of 9 warps fit per SM, so the
+    // occupancy-based grid sizing (size_grids, rem2d_host_util.h) hands out other first-wave grids.
+    float lead_x;     // > 0: park a creature whose root has reached x >= lead_x after lead_from ticks
+    int lead_from;
+    int late_from;    // creatures pulled from this position of the class queue on park after late_ticks ticks
+    int late_ticks;
+    // diagnostics (trace option): every 4th tick lane 0 of each warp records {globaltimer us, live creatures | tick << 8 |
+    // smid << 24}; REM2D_TRACE_SAMPLES entries per warp. Null in production.
+    unsigned int* trace;
+    unsigned int* tail_trace;   // per park slot: {us parked, us tail warp started, us finished, ticks run by the tail warp}
+    int wide_gs;      // a creature whose group already has this many lanes (log2) is not parked: the tail launch is no wider
+};
+#define REM2D_TRACE_SAMPLES 1024
+
+// The class queue of an episode launch and where finished creatures are written (indexed by creature).
+struct EpisodeQueue {
+    const int* __restrict__ order; int n_order; int* queue;      // creatures in pull order; pull counter
+    DevPop p; int max_ticks;
+    double* fitness; int* ticks; int* alive; int* status;
+};
 
 // Capacities and section offsets of one capacity class. The layout is a RUN-TIME value (kernel parameter, i.e. constant
 // bank): all classes execute the SAME code image. With one template instantiation per class, warps of 7 different
@@ -2163,6 +2192,127 @@ public:
         bool solved = tick_pre(nt);
         if (solved) solve_velocity(nt);
         tick_post(solved, nt);
+    }
+
+    // ---- whole episodes: the loop of the episode kernel (rem2d_kernels.cu) in both modes, WARP-cooperative.
+    // Queue mode: every group without a creature pulls the next one of the class queue, builds its world in the group's column
+    // and ticks it until its episode ends; long-lived creatures are parked for the tail mode. Tail mode (tail = true): the groups
+    // start with their parked creatures (my, column g) and nothing to pull. `tslot` is the park slot of a tail creature (-1:
+    // none). Hooks: sample(sim, iteration, live lanes) before every iteration, regrouped(sim, old gs) after a regroup,
+    // finished(sim, creature, tslot, iterations) on the leader of a group whose creature ended, now_us() for the park trace.
+    //
+    // Regrouping: once the queue is empty (some group of the warp failed a pull; pulls are monotone, so every later pull fails
+    // too), the warp's dead groups would idle until the last live creature ends. Instead the warp packs its n live creatures onto
+    // groups 0..n-1, in order, with the largest width 2^gs' <= 32 / n (at most max_gs), and repeats that as more creatures end.
+    // Exact: every width runs the same code on the creature's own cold column, the hot block is staged from it at every tick
+    // (solve_pre) and written back (solve_post), and make_hot_layout(L, gs').rows never exceeds the rows at a narrower gs, so
+    // the widened groups fit in the shared memory the warp was launched with (tests/test_regroup.py).
+    template <class Hooks>
+    __device__ __forceinline__ void episodes(const int lane, const bool tail, const int max_gs, float* hot, const EpisodeQueue& Q,
+                                             const ParkPolicy& park, float* park_state, int* park_creature, int* park_count,
+                                             int my, int tslot, Hooks& hooks) {
+        int loop_iter = 0, park_at = park.ticks;
+        bool exhausted = tail, drained = tail;
+        Cnt snapshot = cnt;
+        for (;;) {
+            if (my < 0 && !exhausted) {
+                int idx = 0;
+                if (leader()) idx = atomicAdd(Q.queue, 1);
+                idx = bcast(idx);
+                if (idx < Q.n_order) {
+                    my = Q.order[idx]; build_world(Q.p, my); snapshot = cnt;
+                    park_at = idx >= park.late_from ? park.late_ticks : park.ticks;
+                }
+                else exhausted = true;
+            }
+            const unsigned live = __ballot_sync(0xffffffffu, my >= 0);
+            hooks.sample(*this, loop_iter, live);
+            ++loop_iter;
+            if (!live) break;
+            if (!drained) drained = __any_sync(0xffffffffu, exhausted);
+            if (drained && gs < max_gs && (__popc(live) >> gs) << (gs + 1) <= 32) {
+                const int old = gs;
+                regroup(lane, live, max_gs, hot, my, park_at, tslot, snapshot);
+                exhausted = true;
+                hooks.regrouped(*this, old);
+            }
+            if (my >= 0) {                                            // group-uniform
+                tick();
+                PHASE(PH_PARK);
+                const int t = Si(S_TICKS), st = Si(S_STATUS), al = Si(S_ALIVE);    // (written before tick()'s last group barrier)
+                if (!al || t >= Q.max_ticks || st) {
+                    if (leader()) {
+                        Q.fitness[my] = Sd(S_FIT_LO); Q.ticks[my] = t; Q.alive[my] = al; Q.status[my] = st;
+                        hooks.finished(*this, my, tslot, loop_iter);
+                    }
+                    // a creature that outgrew a capacity of this class is re-run by the host in the next class up:
+                    // its partial work must not be counted
+                    if (st) cnt = snapshot;
+                    my = -1;
+                } else if (!tail && park.ticks > 0 && gs < park.wide_gs &&
+                           (t >= park_at || (park.lead_x > 0.0f && t >= park.lead_from && B(BF_CX, 0) >= park.lead_x))) {
+                    // long-lived creature: park its state; the latency-oriented tail mode (one warp per creature) finishes it.
+                    // (the counter never exceeds the cap: the host hands every counted slot to a tail launch)
+                    int slot = -1;
+                    if (leader()) {
+                        int seen = *(volatile int*)park_count;
+                        while (seen < park.cap) {
+                            const int prev = atomicCAS(park_count, seen, seen + 1);
+                            if (prev == seen) { slot = seen; break; }
+                            seen = prev;
+                        }
+                    }
+                    slot = bcast(slot);
+                    if (slot >= 0) {
+                        float* dst = park_state + (size_t)(slot >> 5) * L.words * 32 + (slot & 31);
+                        for (int w = sub; w < L.words; w += G) dst[w * 32] = g[w * 32];
+                        __threadfence();                                 // the column is visible before the slot is published
+                        gsync();
+                        if (leader()) {
+                            if (park.tail_trace) park.tail_trace[slot * 4] = hooks.now_us();
+                            __threadfence();
+                            atomicExch(&park_creature[slot], my + 1);    // 0 = allocated but not yet published
+                        }
+                        my = -1;
+                    }
+                }
+                gsync();          // the leader's reads of this creature's scalars are done before the column is rebuilt
+                PHASE(PH_LOOP);
+            }
+        }
+    }
+    // Packs the live creatures of the warp onto the first groups, widened to the largest gs' <= max_gs with n_live << gs' <= 32
+    // (see episodes). Each creature takes its id, cold column, park threshold and park slot along. Its work so far, summed over
+    // the lanes of its old group, moves to the counters of its new leader lane, so that `cnt = snapshot` after an overflow still
+    // removes all of it.
+    __device__ __forceinline__ void regroup(const int lane, const unsigned live, const int max_gs, float* hot, int& my, int& park_at,
+                                            int& tslot, Cnt& snapshot) {
+        const int n = __popc(live) >> gs;
+        int ngs = gs + 1;
+        while (ngs < max_gs && n << (ngs + 1) <= 32) ++ngs;
+        __syncwarp();                      // hot columns and cold columns change owners: earlier accesses are done
+        const unsigned leads = __ballot_sync(0xffffffffu, my >= 0 && leader());
+        unsigned m = leads;
+        for (int i = lane >> ngs; i > 0 && m; --i) m &= m - 1;       // the (lane >> ngs)-th live creature, in lane order
+        const bool has = m != 0u;
+        const int src = has ? __ffs((int)m) - 1 : lane;
+        const bool new_leader = has && (lane & ((1 << ngs) - 1)) == 0;
+#pragma unroll
+        for (int i = 0; i < REM2D_N_COUNTERS; ++i) {
+            unsigned w = my >= 0 ? cnt.c[i] - snapshot.c[i] : 0u;
+            for (int o = G >> 1; o > 0; o >>= 1) w += __shfl_xor_sync(gmask, w, o);
+            if (my >= 0) cnt.c[i] = snapshot.c[i];
+            w = __shfl_sync(0xffffffffu, w, src);
+            snapshot.c[i] = cnt.c[i];
+            if (new_leader) cnt.c[i] += w;
+        }
+        my = __shfl_sync(0xffffffffu, my, src);
+        park_at = __shfl_sync(0xffffffffu, park_at, src);
+        tslot = __shfl_sync(0xffffffffu, tslot, src);
+        const unsigned long long col = __shfl_sync(0xffffffffu, (unsigned long long)g, src);
+        set_group(ngs, lane, hot);
+        if (has) { g = (float*)col; nb = Si(S_NB); nj = nb - 1; }
+        else { my = -1; tslot = -1; nb = nj = 0; }
     }
 };
 

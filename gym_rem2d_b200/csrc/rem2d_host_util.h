@@ -18,6 +18,9 @@ static const ClassDims class_dims[N_CLASSES] = {
     {1, 10, 3, 0}, {2, 16, 4, 0}, {4, 28, 4, 1}, {8, 48, 6, 3}, {12, 64, 6, 5}, {16, 80, 6, 5}, {22, 104, 6, 5}, {32, 144, 8, 5},
     {44, 192, 10, 5},
 };
+// Widest group shift a draining episode warp of class k launched at group shift gs regroups its survivors to (Sim::episodes):
+// the class's automatic cap, or the launch's own width if that was forced wider.
+static inline int widest_group_shift(int k, int gs) { return std::max(gs, class_dims[k].gs); }
 static inline int class_hot_bytes(int k, int gs) {      // shared memory of a warp (CTA) of class k, groups of 2^gs lanes
     return rem2d::make_hot_layout(rem2d::make_layout(class_dims[k].nb, class_dims[k].nc, class_dims[k].nt), gs).rows * 128;
 }

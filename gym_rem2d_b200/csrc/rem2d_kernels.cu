@@ -87,13 +87,56 @@ void rem2d_launch_step(const Layout& L, int gs, int n_batches, cudaStream_t st, 
 // mode 1, tail: takes over parked creatures (one per group, normally gs = 5: a whole warp per creature) and finishes them:
 // the long-lived creatures bound the makespan, and a 32-lane schedule ticks a large creature several times faster than
 // the throughput-oriented groups of the queue mode.
-// Dynamic shared memory: make_hot_layout(L, gs).rows * 128 B.
+// The loop of both modes is Sim::episodes (rem2d_device.cuh, shared with the CPU emulation); once its class queue is empty, a
+// warp regroups its surviving creatures into wider groups, up to the class's widest group shift (max_gs).
+
+// Hooks of Sim::episodes: the trace samples, the phase-timing flush on a regroup and the tail traces.
+struct KernelHooks {
+    const ParkPolicy& park;
+    unsigned long long* counters;
+    int lane, mode;
+    __device__ __forceinline__ unsigned now_us() {
+        unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+        return (unsigned)(t / 1000ull);
+    }
+    __device__ __forceinline__ void sample(Sim& sim, int loop_iter, unsigned live) {
+        if (park.trace && lane == 0 && (loop_iter & 3) == 0 && (loop_iter >> 2) < REM2D_TRACE_SAMPLES) {
+            unsigned smid;
+            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+            unsigned int* tr = park.trace + ((size_t)blockIdx.x * REM2D_TRACE_SAMPLES + (loop_iter >> 2)) * 2;
+            tr[0] = now_us();
+            tr[1] = (unsigned)(__popc(live) >> sim.gs) | ((unsigned)(loop_iter & 0xffff) << 8) | (smid << 24);
+        }
+    }
+    // warp-cycles per phase as seen by lane 0, per (mode, group shift): counters[REM2D_N_COUNTERS + ((mode * 6 + gs) * 16 + phase)]
+    __device__ __forceinline__ void flush_phases(Sim& sim, int gs) {
+#ifdef REM2D_PHASE_TIMING
+        if (lane == 0) {
+            PHASE(PH_LOOP);
+            for (int i = 0; i < REM2D_N_PHASES; ++i) {
+                if (sim.ph[i] > 0) atomicAdd(&counters[REM2D_N_COUNTERS + (mode * 6 + gs) * REM2D_N_PHASES + i], (unsigned long long)sim.ph[i]);
+                sim.ph[i] = 0;
+            }
+        }
+#endif
+    }
+    __device__ __forceinline__ void regrouped(Sim& sim, int old_gs) { flush_phases(sim, old_gs); }
+    __device__ __forceinline__ void finished(Sim&, int, int tslot, int loop_iter) {
+        if (tslot >= 0 && park.tail_trace) {
+            park.tail_trace[tslot * 4 + 2] = now_us();
+            park.tail_trace[tslot * 4 + 3] = (unsigned)loop_iter;
+        }
+    }
+};
+
+// Dynamic shared memory: make_hot_layout(L, gs).rows * 128 B (gs = the launch's group shift; regrouping only widens, and
+// never needs more rows).
 // Two images of the same code that differ only in their register cap (__launch_bounds__): IMAGE 0, 200 registers (<= 9 warps per
 // SM), for throughput-bound populations - every class runs one lane per creature, shared memory allows 3-12 warps per SM anyway
 // and the uncapped code is ~3 % faster; IMAGE 1, 128 registers (16 warps per SM, no spills), for under-filled GPUs - the creatures
 // are spread over wide lane groups and the resident-warp limit is what bounds how wide. All launches of one evaluation (queue
 // and tail) use the same image, so co-resident warps still share one code image in the instruction cache.
-static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int mode, float* slots,
+static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int max_gs, int mode, float* slots,
                                                         const int* __restrict__ order, int n_order, int* queue, DevPop p,
                                                         const Terrain* __restrict__ ter, const Consts* __restrict__ k, int max_ticks,
                                                         double* fitness, int* ticks, int* alive, int* status,
@@ -107,12 +150,12 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
     sim.ter = ter; sim.k = k;
 #pragma unroll
     for (int i = 0; i < REM2D_N_COUNTERS; ++i) sim.cnt.c[i] = 0u;
-    int my = -1, loop_iter = 0, park_at = park.ticks;
-    bool exhausted = false;
+    int my = -1, tslot = -1;
 #ifdef REM2D_PHASE_TIMING
     for (int i = 0; i < REM2D_N_PHASES; ++i) sim.ph[i] = 0;
     sim.phase_t0 = clock64(); sim.phase_cur = PH_LOOP;
 #endif
+    KernelHooks hooks{park, counters, lane, tail ? 1 : 0};
     const int q = blockIdx.x * (32 >> gs) + (lane >> gs);           // my group's column / park slot index
     if (tail) {
         // the slot was allocated by a queue-mode warp that may still be running: wait until its column has been published
@@ -125,98 +168,18 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
                 __threadfence();
             }
             my = sim.bcast(my);
-            if (park.tail_trace && sim.leader()) {
-                unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-                park.tail_trace[slot * 4 + 1] = (unsigned)(t / 1000ull);
-            }
+            tslot = slot;
+            if (park.tail_trace && sim.leader()) park.tail_trace[slot * 4 + 1] = hooks.now_us();
             sim.g = park_state + (size_t)(slot >> 5) * L.words * 32 + (slot & 31);
             sim.nb = sim.Si(S_NB); sim.nj = sim.nb - 1;
         } else { sim.g = nullptr; sim.nb = sim.nj = 0; }
-        exhausted = true;
     } else {
         sim.g = slots + (size_t)(q >> 5) * L.words * 32 + (q & 31);
     }
-    Cnt snapshot = sim.cnt;
-    for (;;) {
-        if (my < 0 && !exhausted) {
-            int idx = 0;
-            if (sim.leader()) idx = atomicAdd(queue, 1);
-            idx = sim.bcast(idx);
-            if (idx < n_order) {
-                my = order[idx]; sim.build_world(p, my); snapshot = sim.cnt;
-                park_at = idx >= park.late_from ? park.late_ticks : park.ticks;
-            }
-            else exhausted = true;
-        }
-        const unsigned live = __ballot_sync(0xffffffffu, my >= 0);
-        if (park.trace && lane == 0 && (loop_iter & 3) == 0 && (loop_iter >> 2) < REM2D_TRACE_SAMPLES) {
-            unsigned long long t; unsigned smid;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-            unsigned int* tr = park.trace + ((size_t)blockIdx.x * REM2D_TRACE_SAMPLES + (loop_iter >> 2)) * 2;
-            tr[0] = (unsigned)(t / 1000ull);
-            tr[1] = (unsigned)(__popc(live) >> gs) | ((unsigned)(loop_iter & 0xffff) << 8) | (smid << 24);
-        }
-        ++loop_iter;
-        if (!live) break;
-        if (my >= 0) {                                            // group-uniform
-            sim.tick();
-            PHASE(PH_PARK);
-            const int t = sim.Si(S_TICKS), st = sim.Si(S_STATUS), al = sim.Si(S_ALIVE);    // (written before tick()'s last group barrier)
-            if (!al || t >= max_ticks || st) {
-                if (sim.leader()) { fitness[my] = sim.Sd(S_FIT_LO); ticks[my] = t; alive[my] = al; status[my] = st; }
-                // a creature that outgrew a capacity of this class is re-run by the host in the next class up:
-                // its partial work must not be counted
-                if (st) sim.cnt = snapshot;
-                my = -1;
-            } else if (!tail && park.ticks > 0 &&
-                       (t >= park_at || (park.lead_x > 0.0f && t >= park.lead_from && sim.B(BF_CX, 0) >= park.lead_x))) {
-                // long-lived creature: park its state; the latency-oriented tail mode (one warp per creature) finishes it.
-                // (the counter never exceeds the cap: the host hands every counted slot to a tail launch)
-                int slot = -1;
-                if (sim.leader()) {
-                    int seen = *(volatile int*)park_count;
-                    while (seen < park.cap) {
-                        const int prev = atomicCAS(park_count, seen, seen + 1);
-                        if (prev == seen) { slot = seen; break; }
-                        seen = prev;
-                    }
-                }
-                slot = sim.bcast(slot);
-                if (slot >= 0) {
-                    float* dst = park_state + (size_t)(slot >> 5) * L.words * 32 + (slot & 31);
-                    for (int w = sim.sub; w < L.words; w += sim.G) dst[w * 32] = sim.g[w * 32];
-                    __threadfence();                                 // the column is visible before the slot is published
-                    sim.gsync();
-                    if (sim.leader()) {
-                        if (park.tail_trace) {
-                            unsigned long long tt; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tt));
-                            park.tail_trace[slot * 4] = (unsigned)(tt / 1000ull);
-                        }
-                        __threadfence();
-                        atomicExch(&park_creature[slot], my + 1);    // 0 = allocated but not yet published
-                    }
-                    my = -1;
-                }
-            }
-            sim.gsync();          // the leader's reads of this creature's scalars are done before the column is rebuilt
-            PHASE(PH_LOOP);
-        }
-    }
-    if (tail && park.tail_trace && sim.leader() && q < n_slots) {
-        unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        park.tail_trace[(first_slot + q) * 4 + 2] = (unsigned)(t / 1000ull);
-        park.tail_trace[(first_slot + q) * 4 + 3] = (unsigned)loop_iter - 1u;
-    }
+    const EpisodeQueue Q{order, n_order, queue, p, max_ticks, fitness, ticks, alive, status};
+    sim.episodes(lane, tail, max_gs, hot, Q, park, park_state, park_creature, park_count, my, tslot, hooks);
     __syncwarp();
-#ifdef REM2D_PHASE_TIMING
-    // warp-cycles per phase as seen by lane 0, per (mode, group shift): counters[REM2D_N_COUNTERS + ((mode * 6 + gs) * 16 + phase)]
-    if (lane == 0) {
-        PHASE(PH_LOOP);
-        for (int i = 0; i < REM2D_N_PHASES; ++i)
-            if (sim.ph[i] > 0) atomicAdd(&counters[REM2D_N_COUNTERS + ((tail ? 6 : 0) + gs) * REM2D_N_PHASES + i], (unsigned long long)sim.ph[i]);
-    }
-#endif
+    hooks.flush_phases(sim, sim.gs);
 #pragma unroll
     for (int i = 0; i < REM2D_N_COUNTERS; ++i) {
         unsigned long long v = sim.cnt.c[i];
@@ -224,22 +187,22 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
         if (lane == 0 && v) atomicAdd(&counters[i], v);
     }
 }
-#define EPISODE_PARAMS const __grid_constant__ Layout L, int gs, int mode, float* slots, const int* __restrict__ order, int n_order, int* queue, \
+#define EPISODE_PARAMS const __grid_constant__ Layout L, int gs, int max_gs, int mode, float* slots, const int* __restrict__ order, int n_order, int* queue, \
                        DevPop p, const Terrain* __restrict__ ter, const Consts* __restrict__ k, int max_ticks, double* fitness, int* ticks, \
                        int* alive, int* status, unsigned long long* counters, ParkPolicy park, float* park_state, int* park_creature,      \
                        int* park_count, int first_slot, int n_slots
-#define EPISODE_ARGS L, gs, mode, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive, status, counters, park, park_state, \
+#define EPISODE_ARGS L, gs, max_gs, mode, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive, status, counters, park, park_state, \
                      park_creature, park_count, first_slot, n_slots
 __global__ void __launch_bounds__(32, 1) episode_kernel(EPISODE_PARAMS) { episode_body(EPISODE_ARGS); }
 __global__ void __launch_bounds__(32, 16) episode_kernel_r128(EPISODE_PARAMS) { episode_body(EPISODE_ARGS); }
 
-void rem2d_launch_episode(const Layout& L, int image, int gs, int grid, cudaStream_t st, float* slots, const int* order, int n_order, int* queue,
+void rem2d_launch_episode(const Layout& L, int image, int gs, int max_gs, int grid, cudaStream_t st, float* slots, const int* order, int n_order, int* queue,
                           DevPop p, const Terrain* ter, const Consts* k, int max_ticks, double* fitness, int* ticks, int* alive, int* status,
                           unsigned long long* counters, ParkPolicy park, float* park_state, int* park_creature, int* park_count) {
     const int smem = make_hot_layout(L, gs).rows * 128;
-    if (image) episode_kernel_r128<<<grid, 32, smem, st>>>(L, gs, 0, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive,
+    if (image) episode_kernel_r128<<<grid, 32, smem, st>>>(L, gs, max_gs, 0, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive,
                                                             status, counters, park, park_state, park_creature, park_count, 0, 0);
-    else episode_kernel<<<grid, 32, smem, st>>>(L, gs, 0, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive, status,
+    else episode_kernel<<<grid, 32, smem, st>>>(L, gs, max_gs, 0, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive, status,
                                                 counters, park, park_state, park_creature, park_count, 0, 0);
 }
 // resident CTAs (= warps) of the episode kernel per SM for a given dynamic shared-memory size: registers AND shared memory
@@ -250,15 +213,15 @@ int rem2d_episode_blocks_per_sm(int image, int dyn_smem_bytes) {
     if (e != cudaSuccess) { cudaGetLastError(); return 0; }
     return n;
 }
-void rem2d_launch_tail(const Layout& L, int image, int gs, cudaStream_t st, float* park_state, int* park_creature, int first_slot, int n_parked,
+void rem2d_launch_tail(const Layout& L, int image, int gs, int max_gs, cudaStream_t st, float* park_state, int* park_creature, int first_slot, int n_parked,
                        const Terrain* ter, const Consts* k, int max_ticks, double* fitness, int* ticks, int* alive, int* status,
                        unsigned long long* counters, unsigned int* tail_trace) {
-    ParkPolicy none = {0, 0, 0.0f, 0, 0, 0, nullptr, tail_trace};
+    ParkPolicy none = {0, 0, 0.0f, 0, 0, 0, nullptr, tail_trace, 0};
     const int per = 32 >> gs, grid = (n_parked + per - 1) / per, smem = make_hot_layout(L, gs).rows * 128;
-    if (image) episode_kernel_r128<<<grid, 32, smem, st>>>(L, gs, 1, nullptr, nullptr, 0, nullptr, DevPop(), ter, k, max_ticks, fitness, ticks,
+    if (image) episode_kernel_r128<<<grid, 32, smem, st>>>(L, gs, max_gs, 1, nullptr, nullptr, 0, nullptr, DevPop(), ter, k, max_ticks, fitness, ticks,
                                                             alive, status, counters, none, park_state, park_creature, nullptr, first_slot,
                                                             n_parked);
-    else episode_kernel<<<grid, 32, smem, st>>>(L, gs, 1, nullptr, nullptr, 0, nullptr, DevPop(), ter, k, max_ticks, fitness, ticks, alive, status,
+    else episode_kernel<<<grid, 32, smem, st>>>(L, gs, max_gs, 1, nullptr, nullptr, 0, nullptr, DevPop(), ter, k, max_ticks, fitness, ticks, alive, status,
                                                 counters, none, park_state, park_creature, nullptr, first_slot, n_parked);
 }
 #endif
