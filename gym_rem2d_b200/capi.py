@@ -50,6 +50,16 @@ class StateView(C.Structure):
                 ("reserved", C.c_int32)]
 
 
+class EpisodeStats(C.Structure):
+    _fields_ = [("end_reason", C.c_void_p), ("max_x", C.c_void_p), ("joint_work", C.c_void_p),
+                ("airborne_ticks", C.c_void_p), ("ground_ticks", C.c_void_p)]
+
+
+# rem2d_episode_stats.end_reason values (include/rem2d_stats.h)
+END_RUNNING, END_ORIGIN, END_WALL, END_GOAL, END_STEPS = 0, 1, 2, 3, 4
+END_REASONS = {END_RUNNING: "running", END_ORIGIN: "origin", END_WALL: "wall", END_GOAL: "goal", END_STEPS: "steps"}
+
+
 class Rem2dError(RuntimeError):
     pass
 
@@ -93,6 +103,9 @@ def load_library(path=None):
     lib.rem2d_set_option.argtypes = [H, C.c_char_p, C.c_double]
     lib.rem2d_read_roots.argtypes = [H, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.rem2d_set_priority.argtypes = [H, C.c_void_p, C.c_int32]
+    if hasattr(lib, "rem2d_read_stats"):          # the episode statistics extension (include/rem2d_stats.h)
+        lib.rem2d_set_stats.argtypes = [H, C.c_int32]
+        lib.rem2d_read_stats.argtypes = [H, C.POINTER(EpisodeStats)]
     _LIBS[path] = lib
     return lib
 
@@ -254,4 +267,30 @@ class Engine:
             setattr(v, k, a.ctypes.data)
         v.max_pairs = max_pairs
         self._check(self.lib.rem2d_read_state(self.h, C.byref(v)), "rem2d_read_state")
+        return st
+
+    def _require_stats(self):
+        if not hasattr(self.lib, "rem2d_read_stats"):
+            raise Rem2dError("%s does not record episode statistics (include/rem2d_stats.h)" % self.backend)
+
+    def set_stats(self, on=True):
+        """Record episode statistics in the whole-episode runs of every later upload / evaluate (never changes results)."""
+        self._require_stats()
+        self._check(self.lib.rem2d_set_stats(self.h, 1 if on else 0), "rem2d_set_stats")
+
+    def read_stats(self):
+        """Episode statistics of the last run_episodes / evaluate of a population uploaded with set_stats(True): a dict of
+        end_reason int32[n] (END_*), max_x float32[n], joint_work float64[n], airborne_ticks int32[n] and ground_ticks
+        int32[n_bodies] (aligned with the table's bodies). Definitions: include/rem2d_stats.h."""
+        self._require_stats()
+        pop = self.pop
+        if pop is None:
+            raise Rem2dError("rem2d_read_stats: no population uploaded")
+        nc, nb = pop.n_creatures, pop.n_bodies
+        st = dict(end_reason=np.zeros(nc, np.int32), max_x=np.zeros(nc, np.float32), joint_work=np.zeros(nc, np.float64),
+                  airborne_ticks=np.zeros(nc, np.int32), ground_ticks=np.zeros(nb, np.int32))
+        v = EpisodeStats()
+        for k, a in st.items():
+            setattr(v, k, a.ctypes.data)
+        self._check(self.lib.rem2d_read_stats(self.h, C.byref(v)), "rem2d_read_stats")
         return st

@@ -1,5 +1,5 @@
 // rem2d_classes.h — the launch interface of the three kernels (rem2d_kernels.cu; one translation unit per kernel so that
-// they compile in parallel) and the host's per-class view of it. All classes run the SAME code: the class only selects a
+// they compile in parallel, and one more for the episode kernel with statistics) and the host's per-class view of it. All classes run the SAME code: the class only selects a
 // Layout (the capacity classes themselves are in rem2d_host_util.h).
 #pragma once
 #include <cuda_runtime.h>
@@ -7,19 +7,30 @@
 
 using rem2d::ParkPolicy;
 
-// Launchers (rem2d_kernels.cu).
+// Launchers (rem2d_kernels.cu). The episode and tail launchers take the statistics' destinations: nullptr launches the
+// images without statistics, anything else the statistics images (rem2d_launch_*_stats, called through them).
 cudaError_t rem2d_set_kernel_attributes(int max_hot_bytes);
+// image 0 / 1: the episode kernel images without statistics, 2 / 3: the statistics images with the same register caps
 int rem2d_episode_blocks_per_sm(int image, int dyn_smem_bytes);
+int rem2d_episode_blocks_per_sm_stats(int image, int dyn_smem_bytes);
 void rem2d_launch_reset(const rem2d::Layout& L, int gs, int n_batches, cudaStream_t st, float* state, const int* lane_creature, rem2d::DevPop p);
 void rem2d_launch_step(const rem2d::Layout& L, int gs, int n_batches, cudaStream_t st, float* state, int n_ticks, const rem2d::Terrain* ter,
                        const rem2d::Consts* k, unsigned long long* counters);
 void rem2d_launch_episode(const rem2d::Layout& L, int image, int gs, int max_gs, int grid, cudaStream_t st, float* slots, const int* order, int n_order, int* queue,
                           rem2d::DevPop p, const rem2d::Terrain* ter, const rem2d::Consts* k, int max_ticks, double* fitness,
                           int* ticks, int* alive, int* status, unsigned long long* counters, ParkPolicy park, float* park_state,
-                          int* park_creature, int* park_count);
+                          int* park_creature, int* park_count, const rem2d::EpisodeStats* stats);
+void rem2d_launch_episode_stats(const rem2d::Layout& L, int image, int gs, int max_gs, int grid, cudaStream_t st, float* slots, const int* order,
+                                int n_order, int* queue, rem2d::DevPop p, const rem2d::Terrain* ter, const rem2d::Consts* k, int max_ticks,
+                                double* fitness, int* ticks, int* alive, int* status, unsigned long long* counters, ParkPolicy park,
+                                float* park_state, int* park_creature, int* park_count, const rem2d::EpisodeStats* stats);
 void rem2d_launch_tail(const rem2d::Layout& L, int image, int gs, int max_gs, cudaStream_t st, float* park_state, int* park_creature, int first_slot,
                        int n_parked, const rem2d::Terrain* ter, const rem2d::Consts* k, int max_ticks, double* fitness, int* ticks,
-                       int* alive, int* status, unsigned long long* counters, unsigned int* tail_trace);
+                       int* alive, int* status, unsigned long long* counters, unsigned int* tail_trace, const rem2d::EpisodeStats* stats);
+void rem2d_launch_tail_stats(const rem2d::Layout& L, int image, int gs, int max_gs, cudaStream_t st, float* park_state, int* park_creature,
+                             int first_slot, int n_parked, const rem2d::Terrain* ter, const rem2d::Consts* k, int max_ticks, double* fitness,
+                             int* ticks, int* alive, int* status, unsigned long long* counters, unsigned int* tail_trace,
+                             const rem2d::EpisodeStats* stats);
 
 // Per-class view used by the host code.
 struct ClassOps {

@@ -1,4 +1,4 @@
-// rem2d_cuda.cu — host side + C-ABI (include/rem2d.h) of the CUDA build, sm_100a only (kernels: rem2d_kernels.cu).
+// rem2d_cuda.cu — host side + C-ABI (include/rem2d.h, include/rem2d_stats.h) of the CUDA build, sm_100a only (kernels: rem2d_kernels.cu).
 //
 // Sorts creatures into capacity classes (by body count), keeps one lane-interleaved state block per 32 creatures in
 // HBM, and runs every class on its own stream so small and large classes overlap on the 148 SMs: rem2d_step on a
@@ -120,6 +120,12 @@ struct rem2d_handle {
     bool have_terrain = false, have_pop = false;
     bool state_valid = false;           // per-creature state blocks hold a consistent snapshot (reset/step path)
     bool results_valid = false;         // d_fitness/d_ticks/... were written by the episode kernel
+    // episode statistics (rem2d_set_stats): the flag, its value at the upload (selects the statistics images for the runs of
+    // that upload), and whether the statistics buffers hold those of the last run
+    bool stats_on = false, upload_stats = false, stats_valid = false;
+    Buf b_stats;
+    EpisodeStats dstats{};
+    int warps_per_sm[4] = {};           // rem2d_episode_blocks_per_sm of the four episode images (plan_upload input)
     int prio_high = 0;                  // greatest stream priority of the device (tail pool)
     int n_edges = 0;
     // population
@@ -181,7 +187,7 @@ static void options_from_env(Options& o) {
 
 static void free_population(rem2d_handle* h) {          // logical reset; the buffers stay allocated for reuse
     for (auto& c : h->cls) { c.n_batches = 0; c.n_members = 0; c.lane_creature.clear(); }
-    h->have_pop = false; h->state_valid = false; h->results_valid = false;
+    h->have_pop = false; h->state_valid = false; h->results_valid = false; h->stats_valid = false;
 }
 static void release_buffers(rem2d_handle* h) {
     for (auto& b : h->d_pop_mem) { if (b.p) cudaFree(b.p); b = Buf(); }
@@ -196,6 +202,8 @@ static void release_buffers(rem2d_handle* h) {
     h->b_results = Buf();
     if (h->b_roots.p) cudaFree(h->b_roots.p);
     h->b_roots = Buf();
+    if (h->b_stats.p) cudaFree(h->b_stats.p);
+    h->b_stats = Buf();
 }
 
 extern "C" {
@@ -273,7 +281,8 @@ int rem2d_create(const rem2d_config* cfg, rem2d_handle** out) {
         for (int q = 0; q < N_CLASSES; ++q)
             for (int gs = 0; gs <= 5; ++gs) max_hot = std::max(max_hot, class_hot_bytes(q, gs));
         if ((e = rem2d_set_kernel_attributes(max_hot)) != cudaSuccess) return fail("cudaFuncSetAttribute", e);
-        for (int im = 0; im < 2; ++im) h->load.max_warps_per_sm[im] = std::max(1, rem2d_episode_blocks_per_sm(im, 1024));
+        for (int im = 0; im < 4; ++im) h->warps_per_sm[im] = std::max(1, rem2d_episode_blocks_per_sm(im, 1024));
+        for (int im = 0; im < 2; ++im) h->load.max_warps_per_sm[im] = h->warps_per_sm[im];
     }
     *out = h;
     return REM2D_OK;
@@ -436,7 +445,21 @@ static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_res
         h->load.work[k] = 0.0;
         for (int c : members[k]) { int nbc = pop->body_off[c + 1] - pop->body_off[c]; h->load.work[k] += nbc == 1 ? 1.0 : 3.5 + nbc; }
     }
+    // statistics runs launch the statistics images: the planner sees their occupancy
+    h->upload_stats = h->stats_on;
+    for (int im = 0; im < 2; ++im) h->load.max_warps_per_sm[im] = h->warps_per_sm[im + (h->upload_stats ? 2 : 0)];
     h->plan = plan_upload(h->load, h->opt);
+    if (h->upload_stats) {
+        const size_t nn = (size_t)std::max(n, 1), nbod = (size_t)std::max(pop->n_bodies, 1);
+        CK(ensure(h->b_stats, nn * (sizeof(double) + sizeof(float) + 2 * sizeof(int32_t)) + nbod * sizeof(int32_t) + 64));
+        EpisodeStats& d = h->dstats;
+        d.joint_work = (double*)h->b_stats.p;
+        d.max_x = (float*)(d.joint_work + nn);
+        d.end_reason = (int32_t*)(d.max_x + nn);
+        d.airborne_ticks = d.end_reason + nn;
+        d.ground_ticks = d.airborne_ticks + nn;
+        d.body_off = h->dpop.body_off;
+    }
     {
         const size_t nn = (size_t)std::max(n, 1);
         CK(ensure(h->b_results, nn * (sizeof(double) + 3 * sizeof(int))));
@@ -481,12 +504,15 @@ static int launch_reset(rem2d_handle* h) {
     rc = join_streams(h);
     if (rc) return rc;
     CK(cudaMemsetAsync(h->d_counters, 0, sizeof(unsigned long long) * N_COUNTER_WORDS, h->user_stream));
-    h->state_valid = true; h->results_valid = false;
+    h->state_valid = true; h->results_valid = false; h->stats_valid = false;
     return REM2D_OK;
 }
 
 // Promotion: creatures that exceeded a capacity of their class (contact pool) are re-run from tick 0 on the refill
 // episode kernel of the next larger class until they fit. Rare (very fine terrains, pile-ups).
+// destinations of the episode statistics of the uploaded population (nullptr: it was uploaded with statistics off)
+static const EpisodeStats* stats_dest(const rem2d_handle* h) { return h->upload_stats ? &h->dstats : nullptr; }
+
 static int promote_overflowed(rem2d_handle* h, int max_ticks) {
     const int n = h->n_creatures;
     std::vector<int> cls_of(h->creature_class);
@@ -521,7 +547,7 @@ static int promote_overflowed(rem2d_handle* h, int max_ticks) {
             CK(cudaMemsetAsync(d_queue, 0, sizeof(int), h->user_stream));
             g_classes(k).episode(h->plan.image, gs, widest_group_shift(k, gs), grid, h->user_stream, (float*)cs.b_redo_slots.p, d_order, (int)redo[k].size(), d_queue, h->dpop, h->d_ter,
                                  h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr, 0}, nullptr, nullptr, nullptr);
+                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr, 0}, nullptr, nullptr, nullptr, stats_dest(h));
             h->launches++;
             CK(cudaGetLastError());
             CK(cudaStreamSynchronize(h->user_stream));      // redo[] (pageable source of the copy) goes out of scope
@@ -533,6 +559,7 @@ static int promote_overflowed(rem2d_handle* h, int max_ticks) {
 // Whole episodes for the uploaded population on the persistent episode kernels (one per class, concurrent).
 static int launch_episodes(rem2d_handle* h, int max_ticks) {
     if (!h->have_terrain) { h->err = "run_episodes: no terrain set"; return REM2D_E_INVALID; }
+    h->stats_valid = false;
     const LaunchPlan lp = plan_launch(h->load, h->plan, max_ticks, h->opt);
     const bool trace = h->opt.trace != 0;
     auto park_policy = [&](int k) {
@@ -552,7 +579,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         if (lp.warp_mode) {      // queue mode with a whole warp per creature and one warp for every creature
             g_classes(k).episode(1, 5, 5, cs.n_members, cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop, h->d_ter,
                                  h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr, 0}, nullptr, nullptr, nullptr);
+                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr, 0}, nullptr, nullptr, nullptr, stats_dest(h));
             CK(cudaEventRecord(cs.t_end, cs.stream));
             h->launches++;
             continue;
@@ -572,7 +599,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         if (h->plan.grid2[k] > 0) { CK(cudaEventRecord(cs.done2, cs.stream)); CK(cudaStreamWaitEvent(cs.stream2, cs.done2, 0)); }   // queue / park counters are reset
         g_classes(k).episode(h->plan.image, h->plan.gs[k], widest_group_shift(k, h->plan.gs[k]), h->plan.grid[k], cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop,
                              h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                             park, cs.d_park_state, cs.d_park_creature, cs.d_park_count);
+                             park, cs.d_park_state, cs.d_park_creature, cs.d_park_count, stats_dest(h));
         // Nothing reads this copy, but it shapes the tail launches: without it the bench population gets twice the tail
         // launches and the second EA generation evaluates 40 % slower (3.1 s against 2.2 s; B200 at 1000 W).
         CK(cudaMemcpyAsync(cs.h_park_count, cs.d_park_count, sizeof(int), cudaMemcpyDeviceToHost, cs.stream));
@@ -589,7 +616,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         const size_t first_block = ((size_t)h->plan.grid[k] * (32 >> gs) + 31) / 32;
         g_classes(k).episode(h->plan.image, gs, widest_group_shift(k, gs), h->plan.grid2[k], cs.stream2, cs.d_state + first_block * g_classes(k).words * 32, cs.d_lane_creature, cs.n_members,
                              cs.d_queue, h->dpop, h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status,
-                             h->d_counters, park_policy(k), cs.d_park_state, cs.d_park_creature, cs.d_park_count);
+                             h->d_counters, park_policy(k), cs.d_park_state, cs.d_park_creature, cs.d_park_count, stats_dest(h));
         h->launches++;
     }
     CK(cudaGetLastError());
@@ -645,7 +672,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
                     const int tail_gs = (cnt - launched[k] >= 32) ? std::min(3, h->opt.tail_group_shift) : h->opt.tail_group_shift;
                     g_classes(k).tail(h->plan.image, tail_gs, widest_group_shift(k, tail_gs), idle_stream(), cs.d_park_state, cs.d_park_creature, launched[k], cnt - launched[k],
                                       h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                                      trace ? (unsigned int*)cs.b_ttrace.p : nullptr);
+                                      trace ? (unsigned int*)cs.b_ttrace.p : nullptr, stats_dest(h));
                     CK(cudaGetLastError());
                     h->launches++;
                     launched[k] = cnt;
@@ -665,7 +692,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
     rc = promote_overflowed(h, max_ticks);
     if (rc) return rc;
     CK(cudaEventRecord(h->ev_stop, h->user_stream));
-    h->state_valid = false; h->results_valid = true;
+    h->state_valid = false; h->results_valid = true; h->stats_valid = h->upload_stats;
     return REM2D_OK;
 }
 
@@ -710,6 +737,7 @@ int rem2d_step(rem2d_handle* h, int32_t n_ticks) {
     if (!h->have_pop || n_ticks < 0) { h->err = "step: no population / negative tick count"; return REM2D_E_INVALID; }
     if (!h->state_valid) { h->err = "step: per-creature state was consumed by rem2d_run_episodes/rem2d_evaluate; call rem2d_reset first"; return REM2D_E_INVALID; }
     cudaSetDevice(h->cfg.device);
+    h->stats_valid = false;                      // the stepping path records no statistics
     CK(cudaEventRecord(h->ev_start, h->user_stream));
     int rc = fork_streams(h);
     if (rc) return rc;
@@ -857,6 +885,33 @@ int rem2d_debug_tail_trace(rem2d_handle* h, int k, unsigned int* out, int64_t ma
     if ((int64_t)words > max_words) words = (size_t)max_words;
     CK(cudaMemcpy(out, cs.b_ttrace.p, words * sizeof(unsigned int), cudaMemcpyDeviceToHost));
     return parked;
+}
+
+int rem2d_set_stats(rem2d_handle* h, int32_t on) {
+    if (!h) return REM2D_E_INVALID;
+    h->stats_on = on != 0;
+    return REM2D_OK;
+}
+
+int rem2d_read_stats(rem2d_handle* h, rem2d_episode_stats* out) {
+    if (!h || !out) return REM2D_E_INVALID;
+    if (!h->stats_valid) {
+        h->err = "read_stats: no statistics: run rem2d_run_episodes / rem2d_evaluate on a population uploaded with rem2d_set_stats(1)";
+        return REM2D_E_INVALID;
+    }
+    cudaSetDevice(h->cfg.device);
+    const size_t n = (size_t)h->n_creatures, nb = (size_t)h->n_bodies;
+    const EpisodeStats& d = h->dstats;
+    auto copy = [&](void* dst, const void* src, size_t bytes) {
+        return dst && bytes ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, h->user_stream) : cudaSuccess;
+    };
+    CK(copy(out->end_reason, d.end_reason, n * sizeof(int32_t)));
+    CK(copy(out->max_x, d.max_x, n * sizeof(float)));
+    CK(copy(out->joint_work, d.joint_work, n * sizeof(double)));
+    CK(copy(out->airborne_ticks, d.airborne_ticks, n * sizeof(int32_t)));
+    CK(copy(out->ground_ticks, d.ground_ticks, nb * sizeof(int32_t)));
+    CK(cudaStreamSynchronize(h->user_stream));
+    return REM2D_OK;
 }
 
 int rem2d_set_priority(rem2d_handle* h, const float* expected_ticks, int32_t n) {

@@ -35,6 +35,7 @@ inline int atomicExch(int* p, int v) { return __atomic_exchange_n(p, v, __ATOMIC
 #include <float.h>
 
 #include "../../include/rem2d.h"
+#include "../../include/rem2d_stats.h"
 
 namespace rem2d {
 
@@ -236,6 +237,13 @@ struct EpisodeQueue {
     double* fitness; int* ticks; int* alive; int* status;
 };
 
+// Episode statistics (include/rem2d_stats.h, rem2d_episode_stats), accumulated by the statistics images of the episode kernel only
+// (-DREM2D_STATS): indexed by creature, ground_ticks by global body index body_off[c] + b. Zeroed when a creature is pulled.
+struct EpisodeStats {
+    int32_t* end_reason; float* max_x; double* joint_work; int32_t* airborne_ticks; int32_t* ground_ticks;
+    const int32_t* body_off;
+};
+
 // Capacities and section offsets of one capacity class. The layout is a RUN-TIME value (kernel parameter, i.e. constant
 // bank): all classes execute the SAME code image. With one template instantiation per class, warps of 7 different
 // 365 KB kernels shared each SM's instruction cache and every class ran 1.4-5x slower than alone (measured, DESIGN.md).
@@ -308,6 +316,10 @@ public:
     int nb, nj;
     // schedule of the current tick (group-uniform): period (slots), largest iteration skew; sched_P == 0: sequential fallback
     int sched_P, sched_smax;
+#ifdef REM2D_STATS
+    EpisodeStats st;          // where the statistics go, and the creature this group is ticking (set before every tick)
+    int st_c;
+#endif
 
     // ---- accessors
     __device__ __forceinline__ float& S(int f) { return g[f * 32]; }
@@ -2185,8 +2197,72 @@ public:
                 if (i + 1 >= k->evaluation_steps) setSi(S_ALIVE, 0);
             } else if (reward > 0.0) setSd(S_FIT_LO, reward);
         }
+#ifdef REM2D_STATS
+        stats_tick();
+#endif
         gsync();
     }
+#ifdef REM2D_STATS
+    // ---- episode statistics (statistics images only). Each is defined by the state at the end of the tick, as
+    // rem2d_read_state / rem2d_read_roots report it, and accumulated in the order of oracle/rem2d_oracle.c:tick().
+    // Zero the statistics of creature c, pulled into this group (after build_world: nb is set).
+    __device__ void stats_begin(int c) {
+        const int b0 = st.body_off[c];
+        for (int b = sub; b < nb; b += G) st.ground_ticks[b0 + b] = 0;
+        if (leader()) {
+            st.end_reason[c] = REM2D_END_RUNNING;
+            st.max_x[c] = __int_as_float((int)0xff800000);       // -inf
+            st.joint_work[c] = 0.0;
+            st.airborne_ticks[c] = 0;
+        }
+    }
+    __device__ void stats_tick() {
+        gsync();                                         // the tick's writes to bodies, joints and contacts are done
+        const int c = st_c, b0 = st.body_off[c];
+        // bodies with a touching terrain contact: a mask over the pool (order-free, strided over the group)
+        unsigned long long m = 0ull;
+        const int n_pool = Si(S_NC);
+        for (int q = sub; q < n_pool; q += G) {
+            const int key = Ci(CF_KEY, q);
+            if (key_flags(key) & CK_TOUCHING) m |= 1ull << key_body(key);
+        }
+        for (int o = G >> 1; o > 0; o >>= 1) m |= __shfl_xor_sync(gmask, m, o);
+        for (int b = sub; b < nb; b += G)
+            if ((m >> b) & 1ull) st.ground_ticks[b0 + b] += 1;
+        // joint work: the group computes the terms, the leader adds them to the running sum in joint order
+        double work = 0.0;
+        if (leader()) work = st.joint_work[c];
+        for (int base = 0; base < nj; base += G) {
+            const int j = base + sub;
+            double t = 0.0;
+            if (j < nj) {
+                const int a = Ji(JF_META, j) & 0xff;
+                t = fabs((double)J(JF_MIMP, j) * ((double)B(BF_W, j + 1) - (double)B(BF_W, a)));
+            }
+            const int n = nj - base < G ? nj - base : G;
+            for (int i = 0; i < n; ++i) {
+                const double v = gs ? __shfl_sync(gmask, t, lead + i) : t;
+                if (leader()) work += v;
+            }
+        }
+        if (leader()) {
+            st.joint_work[c] = work;
+            if (m == 0ull) st.airborne_ticks[c] += 1;
+            const float x = B(BF_CX, 0);
+            if (x > st.max_x[c]) st.max_x[c] = x;
+            // the comparisons of the termination rule above, in its precedence
+            const double wod = Sd(S_WOD_LO);
+            int why = REM2D_END_RUNNING;
+            if (k->terminate) {
+                if (x < 0.0f) why = REM2D_END_ORIGIN;
+                else if (wod > (double)x) why = REM2D_END_WALL;
+                else if ((double)x > k->env_length) why = REM2D_END_GOAL;
+                else if (Si(S_TICKS) >= k->evaluation_steps) why = REM2D_END_STEPS;
+            }
+            if (why != REM2D_END_RUNNING) st.end_reason[c] = why;
+        }
+    }
+#endif
     __device__ void tick() {
         int nt;
         bool solved = tick_pre(nt);
@@ -2221,6 +2297,9 @@ public:
                 idx = bcast(idx);
                 if (idx < Q.n_order) {
                     my = Q.order[idx]; build_world(Q.p, my); snapshot = cnt;
+#ifdef REM2D_STATS
+                    stats_begin(my);
+#endif
                     park_at = idx >= park.late_from ? park.late_ticks : park.ticks;
                 }
                 else exhausted = true;
@@ -2237,6 +2316,9 @@ public:
                 hooks.regrouped(*this, old);
             }
             if (my >= 0) {                                            // group-uniform
+#ifdef REM2D_STATS
+                st_c = my;
+#endif
                 tick();
                 PHASE(PH_PARK);
                 const int t = Si(S_TICKS), st = Si(S_STATUS), al = Si(S_ALIVE);    // (written before tick()'s last group barrier)

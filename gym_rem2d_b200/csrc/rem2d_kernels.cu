@@ -1,10 +1,15 @@
 // rem2d_kernels.cu — the three kernels of the hot path (reset, step, episode with its queue and tail modes). Compiled once per
 // kernel (-DREM2D_KERNEL_ID=0..2) so the translation units build in parallel; every capacity class and every group size runs the
-// same code with its own Layout and group shift (kernel parameters).
+// same code with its own Layout and group shift (kernel parameters). REM2D_KERNEL_ID=3 compiles the episode kernel once more
+// with the episode statistics (REM2D_STATS): two more images, launched only by evaluations that record statistics, so that
+// the images of every other evaluation stay exactly what they are without them.
 //
 // Lane mapping (all kernels): a warp holds 32 >> gs creatures, each owned by a group of G = 1 << gs lanes (rem2d_device.cuh).
 // Cold state: blocks of 32 creature columns; creature column q lives in block q >> 5, column q & 31.
 #include <cstdlib>
+#if REM2D_KERNEL_ID == 3
+#define REM2D_STATS 1
+#endif
 #include "rem2d_classes.h"
 
 using namespace rem2d;
@@ -74,7 +79,7 @@ void rem2d_launch_step(const Layout& L, int gs, int n_batches, cudaStream_t st, 
 }
 #endif
 
-#if REM2D_KERNEL_ID == 2
+#if REM2D_KERNEL_ID == 2 || REM2D_KERNEL_ID == 3
 // Whole episodes, two modes of ONE kernel (one code image: co-resident warps of both modes share the instruction cache).
 //
 // mode 0, queue: every group pulls the next creature of its class from a queue (big creatures first), builds its world in
@@ -141,13 +146,20 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
                                                         const Terrain* __restrict__ ter, const Consts* __restrict__ k, int max_ticks,
                                                         double* fitness, int* ticks, int* alive, int* status,
                                                         unsigned long long* counters, ParkPolicy park, float* park_state,
-                                                        int* park_creature, int* park_count, int first_slot, int n_slots) {
+                                                        int* park_creature, int* park_count, int first_slot, int n_slots
+#ifdef REM2D_STATS
+                                                        , const EpisodeStats& stats
+#endif
+                                                        ) {
     extern __shared__ float hot[];
     const int lane = threadIdx.x;
     const bool tail = mode != 0;
     Sim sim;
     sim.L = L; sim.set_group(gs, lane, hot);
     sim.ter = ter; sim.k = k;
+#ifdef REM2D_STATS
+    sim.st = stats; sim.st_c = -1;
+#endif
 #pragma unroll
     for (int i = 0; i < REM2D_N_COUNTERS; ++i) sim.cnt.c[i] = 0u;
     int my = -1, tslot = -1;
@@ -193,36 +205,75 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
                        int* park_count, int first_slot, int n_slots
 #define EPISODE_ARGS L, gs, max_gs, mode, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive, status, counters, park, park_state, \
                      park_creature, park_count, first_slot, n_slots
+#ifndef REM2D_STATS
 __global__ void __launch_bounds__(32, 1) episode_kernel(EPISODE_PARAMS) { episode_body(EPISODE_ARGS); }
 __global__ void __launch_bounds__(32, 16) episode_kernel_r128(EPISODE_PARAMS) { episode_body(EPISODE_ARGS); }
-
-void rem2d_launch_episode(const Layout& L, int image, int gs, int max_gs, int grid, cudaStream_t st, float* slots, const int* order, int n_order, int* queue,
-                          DevPop p, const Terrain* ter, const Consts* k, int max_ticks, double* fitness, int* ticks, int* alive, int* status,
-                          unsigned long long* counters, ParkPolicy park, float* park_state, int* park_creature, int* park_count) {
-    const int smem = make_hot_layout(L, gs).rows * 128;
-    if (image) episode_kernel_r128<<<grid, 32, smem, st>>>(L, gs, max_gs, 0, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive,
-                                                            status, counters, park, park_state, park_creature, park_count, 0, 0);
-    else episode_kernel<<<grid, 32, smem, st>>>(L, gs, max_gs, 0, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive, status,
-                                                counters, park, park_state, park_creature, park_count, 0, 0);
+#define EPISODE_IMAGE0 episode_kernel
+#define EPISODE_IMAGE1 episode_kernel_r128
+#define EPISODE_FN(name) name
+#define STATS_ARG
+#else
+// the statistics images: the same code and register caps, the statistics' destinations as a trailing parameter
+__global__ void __launch_bounds__(32, 1) episode_kernel_stats(EPISODE_PARAMS, const __grid_constant__ EpisodeStats stats) {
+    episode_body(EPISODE_ARGS, stats);
 }
-// resident CTAs (= warps) of the episode kernel per SM for a given dynamic shared-memory size: registers AND shared memory
-int rem2d_episode_blocks_per_sm(int image, int dyn_smem_bytes) {
+__global__ void __launch_bounds__(32, 16) episode_kernel_stats_r128(EPISODE_PARAMS, const __grid_constant__ EpisodeStats stats) {
+    episode_body(EPISODE_ARGS, stats);
+}
+#define EPISODE_IMAGE0 episode_kernel_stats
+#define EPISODE_IMAGE1 episode_kernel_stats_r128
+#define EPISODE_FN(name) name##_stats
+#define STATS_ARG , *stats
+#endif
+
+// Launchers: stats == nullptr launches the images without statistics (kernel 2's unit), otherwise the statistics images
+// (kernel 3's unit), so that every launch of one evaluation uses the same image.
+void EPISODE_FN(rem2d_launch_episode)(const Layout& L, int image, int gs, int max_gs, int grid, cudaStream_t st, float* slots, const int* order,
+                                      int n_order, int* queue, DevPop p, const Terrain* ter, const Consts* k, int max_ticks, double* fitness,
+                                      int* ticks, int* alive, int* status, unsigned long long* counters, ParkPolicy park, float* park_state,
+                                      int* park_creature, int* park_count, const EpisodeStats* stats) {
+#ifndef REM2D_STATS
+    if (stats) {
+        rem2d_launch_episode_stats(L, image, gs, max_gs, grid, st, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive,
+                                   status, counters, park, park_state, park_creature, park_count, stats);
+        return;
+    }
+#endif
+    const int smem = make_hot_layout(L, gs).rows * 128;
+    if (image) EPISODE_IMAGE1<<<grid, 32, smem, st>>>(L, gs, max_gs, 0, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive,
+                                                      status, counters, park, park_state, park_creature, park_count, 0, 0 STATS_ARG);
+    else EPISODE_IMAGE0<<<grid, 32, smem, st>>>(L, gs, max_gs, 0, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive, status,
+                                                counters, park, park_state, park_creature, park_count, 0, 0 STATS_ARG);
+}
+// resident CTAs (= warps) of the episode kernel per SM for a given dynamic shared-memory size: registers AND shared memory.
+// image 0 / 1: the images without statistics, 2 / 3: the statistics images of the same register caps.
+int EPISODE_FN(rem2d_episode_blocks_per_sm)(int image, int dyn_smem_bytes) {
+#ifndef REM2D_STATS
+    if (image >= 2) return rem2d_episode_blocks_per_sm_stats(image - 2, dyn_smem_bytes);
+#endif
     int n = 0;
-    cudaError_t e = image ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, episode_kernel_r128, 32, (size_t)dyn_smem_bytes)
-                          : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, episode_kernel, 32, (size_t)dyn_smem_bytes);
+    cudaError_t e = image ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, EPISODE_IMAGE1, 32, (size_t)dyn_smem_bytes)
+                          : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, EPISODE_IMAGE0, 32, (size_t)dyn_smem_bytes);
     if (e != cudaSuccess) { cudaGetLastError(); return 0; }
     return n;
 }
-void rem2d_launch_tail(const Layout& L, int image, int gs, int max_gs, cudaStream_t st, float* park_state, int* park_creature, int first_slot, int n_parked,
-                       const Terrain* ter, const Consts* k, int max_ticks, double* fitness, int* ticks, int* alive, int* status,
-                       unsigned long long* counters, unsigned int* tail_trace) {
+void EPISODE_FN(rem2d_launch_tail)(const Layout& L, int image, int gs, int max_gs, cudaStream_t st, float* park_state, int* park_creature,
+                                   int first_slot, int n_parked, const Terrain* ter, const Consts* k, int max_ticks, double* fitness, int* ticks,
+                                   int* alive, int* status, unsigned long long* counters, unsigned int* tail_trace, const EpisodeStats* stats) {
+#ifndef REM2D_STATS
+    if (stats) {
+        rem2d_launch_tail_stats(L, image, gs, max_gs, st, park_state, park_creature, first_slot, n_parked, ter, k, max_ticks, fitness, ticks,
+                                alive, status, counters, tail_trace, stats);
+        return;
+    }
+#endif
     ParkPolicy none = {0, 0, 0.0f, 0, 0, 0, nullptr, tail_trace, 0};
     const int per = 32 >> gs, grid = (n_parked + per - 1) / per, smem = make_hot_layout(L, gs).rows * 128;
-    if (image) episode_kernel_r128<<<grid, 32, smem, st>>>(L, gs, max_gs, 1, nullptr, nullptr, 0, nullptr, DevPop(), ter, k, max_ticks, fitness, ticks,
-                                                            alive, status, counters, none, park_state, park_creature, nullptr, first_slot,
-                                                            n_parked);
-    else episode_kernel<<<grid, 32, smem, st>>>(L, gs, max_gs, 1, nullptr, nullptr, 0, nullptr, DevPop(), ter, k, max_ticks, fitness, ticks, alive, status,
-                                                counters, none, park_state, park_creature, nullptr, first_slot, n_parked);
+    if (image) EPISODE_IMAGE1<<<grid, 32, smem, st>>>(L, gs, max_gs, 1, nullptr, nullptr, 0, nullptr, DevPop(), ter, k, max_ticks, fitness, ticks,
+                                                      alive, status, counters, none, park_state, park_creature, nullptr, first_slot,
+                                                      n_parked STATS_ARG);
+    else EPISODE_IMAGE0<<<grid, 32, smem, st>>>(L, gs, max_gs, 1, nullptr, nullptr, 0, nullptr, DevPop(), ter, k, max_ticks, fitness, ticks, alive,
+                                                status, counters, none, park_state, park_creature, nullptr, first_slot, n_parked STATS_ARG);
 }
 #endif
 
@@ -232,11 +283,13 @@ void rem2d_launch_tail(const Layout& L, int image, int gs, int max_gs, cudaStrea
 // (measured: 1.4x slower whole run when a tail kernel was resident next to the episode kernels).
 cudaError_t rem2d_attr_step(int max_hot_bytes);
 cudaError_t rem2d_attr_episode(int max_hot_bytes);
+cudaError_t rem2d_attr_episode_stats(int max_hot_bytes);
 #if REM2D_KERNEL_ID == 0
 cudaError_t rem2d_set_kernel_attributes(int max_hot_bytes) {
     cudaError_t e = rem2d_attr_step(max_hot_bytes);
     if (e != cudaSuccess) return e;
-    return rem2d_attr_episode(max_hot_bytes);
+    if ((e = rem2d_attr_episode(max_hot_bytes)) != cudaSuccess) return e;
+    return rem2d_attr_episode_stats(max_hot_bytes);
 }
 #elif REM2D_KERNEL_ID == 1
 cudaError_t rem2d_attr_step(int max_hot_bytes) {
@@ -244,12 +297,12 @@ cudaError_t rem2d_attr_step(int max_hot_bytes) {
     if (e != cudaSuccess) return e;
     return cudaFuncSetAttribute(step_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
 }
-#elif REM2D_KERNEL_ID == 2
-cudaError_t rem2d_attr_episode(int max_hot_bytes) {
-    cudaError_t e = cudaFuncSetAttribute(episode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes);
+#elif REM2D_KERNEL_ID == 2 || REM2D_KERNEL_ID == 3
+cudaError_t EPISODE_FN(rem2d_attr_episode)(int max_hot_bytes) {
+    cudaError_t e = cudaFuncSetAttribute(EPISODE_IMAGE0, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes);
     if (e != cudaSuccess) return e;
-    if ((e = cudaFuncSetAttribute(episode_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)) != cudaSuccess) return e;
-    if ((e = cudaFuncSetAttribute(episode_kernel_r128, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes)) != cudaSuccess) return e;
-    return cudaFuncSetAttribute(episode_kernel_r128, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    if ((e = cudaFuncSetAttribute(EPISODE_IMAGE0, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)) != cudaSuccess) return e;
+    if ((e = cudaFuncSetAttribute(EPISODE_IMAGE1, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes)) != cudaSuccess) return e;
+    return cudaFuncSetAttribute(EPISODE_IMAGE1, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
 }
 #endif

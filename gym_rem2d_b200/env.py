@@ -32,12 +32,17 @@ class _Box:
 
 
 class BatchedModular2D:
-    """A whole population of creatures, each in its own world, stepped together on one GPU."""
+    """A whole population of creatures, each in its own world, stepped together on one GPU. With ``stats=True`` every
+    ``evaluate`` also leaves the episode statistics of the population in ``last_stats`` (``Engine.read_stats``)."""
 
-    def __init__(self, device=0, stream=None, max_perturbance=K.MAX_PERTURBANCE_TERRAIN, lib_path=None, precision="exact", **config):
+    def __init__(self, device=0, stream=None, max_perturbance=K.MAX_PERTURBANCE_TERRAIN, lib_path=None, precision="exact", stats=False,
+                 **config):
         self.engine = Engine(lib_path=lib_path, device=device, stream=stream, precision=precision, **config)
         self.max_perturbance = max_perturbance
         self.table = None
+        self.stats = bool(stats)
+        self._engine_stats = False
+        self.last_stats = None
         self.seed(K.TERRAIN_SEED)
 
     def seed(self, seed=None):
@@ -68,13 +73,19 @@ class BatchedModular2D:
     def fitness(self):
         return self.engine.fitness()
 
-    def evaluate(self, individuals=None, table=None, steps=K.EVALUATION_STEPS, tree_depth=None):
-        """Whole episodes for the whole population: float64 fitness per individual, as ``evaluate`` returns."""
+    def evaluate(self, individuals=None, table=None, steps=K.EVALUATION_STEPS, tree_depth=None, stats=None):
+        """Whole episodes for the whole population: float64 fitness per individual, as ``evaluate`` returns. ``stats``
+        (default: the constructor's) also records the episode statistics, left in ``last_stats``; they never change results."""
         if table is None:
             table = flatten_population(individuals, tree_depth)
         self.table = table
+        stats = self.stats if stats is None else bool(stats)
+        if stats != self._engine_stats:
+            self.engine.set_stats(stats)
+            self._engine_stats = stats
         fit, ticks = self.engine.evaluate(table, steps)
         self.last_ticks = ticks
+        self.last_stats = self.engine.read_stats() if stats else None
         return fit
 
     def close(self):
@@ -161,12 +172,14 @@ def evaluate(individual, EVALUATION_STEPS=10000, HEADLESS=True, INTERVAL=100, EN
     return float(env.evaluate([individual], steps=EVALUATION_STEPS, tree_depth=TREE_DEPTH)[0])
 
 
-def evaluate_population(individuals, EVALUATION_STEPS=10000, TREE_DEPTH=None, env=None, as_torch=True):
-    """Batched evaluate: fitness of every individual (torch.float32 tensor on the host by default)."""
+def evaluate_population(individuals, EVALUATION_STEPS=10000, TREE_DEPTH=None, env=None, as_torch=True, return_stats=False):
+    """Batched evaluate: fitness of every individual (torch.float32 tensor on the host by default). With ``return_stats``,
+    ``(fitness, stats)``: the episode statistics of ``Engine.read_stats`` (numpy arrays; ground_ticks per body of the
+    flattened table)."""
     env = env or getEnv()
     env.seed(K.TERRAIN_SEED)
-    fit = env.evaluate(individuals, steps=EVALUATION_STEPS, tree_depth=TREE_DEPTH)
+    fit = env.evaluate(individuals, steps=EVALUATION_STEPS, tree_depth=TREE_DEPTH, stats=True if return_stats else None)
     if as_torch:
         import torch
-        return torch.from_numpy(fit.astype(np.float32))
-    return fit
+        fit = torch.from_numpy(fit.astype(np.float32))
+    return (fit, env.last_stats) if return_stats else fit
