@@ -60,6 +60,10 @@ END_RUNNING, END_ORIGIN, END_WALL, END_GOAL, END_STEPS = 0, 1, 2, 3, 4
 END_REASONS = {END_RUNNING: "running", END_ORIGIN: "origin", END_WALL: "wall", END_GOAL: "goal", END_STEPS: "steps"}
 
 
+class Observation(C.Structure):
+    _fields_ = [("joint_angle", C.c_void_p), ("joint_speed", C.c_void_p), ("root", C.c_void_p), ("ground", C.c_void_p)]
+
+
 class Rem2dError(RuntimeError):
     pass
 
@@ -106,6 +110,9 @@ def load_library(path=None):
     if hasattr(lib, "rem2d_read_stats"):          # the episode statistics extension (include/rem2d_stats.h)
         lib.rem2d_set_stats.argtypes = [H, C.c_int32]
         lib.rem2d_read_stats.argtypes = [H, C.POINTER(EpisodeStats)]
+    if hasattr(lib, "rem2d_step_targets"):        # the closed-loop control extension (include/rem2d_control.h)
+        lib.rem2d_step_targets.argtypes = [H, C.c_void_p, C.c_int32]
+        lib.rem2d_read_observations.argtypes = [H, C.POINTER(Observation)]
     _LIBS[path] = lib
     return lib
 
@@ -294,3 +301,37 @@ class Engine:
             setattr(v, k, a.ctypes.data)
         self._check(self.lib.rem2d_read_stats(self.h, C.byref(v)), "rem2d_read_stats")
         return st
+
+    def _require_control(self):
+        if not hasattr(self.lib, "rem2d_step_targets"):
+            raise Rem2dError("%s does not take joint targets (include/rem2d_control.h)" % self.backend)
+
+    def step_targets(self, targets, n_ticks=1):
+        """Advances every living creature by up to ``n_ticks`` ticks with the P-controller driven to ``targets`` (float64
+        [n_joints], target angles in radians in table order, held for all ticks) instead of the sine controllers, which are
+        not advanced. Semantics: include/rem2d_control.h."""
+        self._require_control()
+        if self.pop is None:
+            raise Rem2dError("rem2d_step_targets: no population uploaded")
+        nj = self.pop.n_bodies - self.pop.n_creatures
+        t = np.ascontiguousarray(targets, np.float64)
+        if t.shape != (nj,):
+            raise ValueError("targets must have shape (%d,) (one per joint), got %s" % (nj, t.shape))
+        self._check(self.lib.rem2d_step_targets(self.h, _ptr(t), int(n_ticks)), "rem2d_step_targets")
+
+    def read_observations(self):
+        """End-of-tick observations of the uploaded population: a dict of joint_angle float32[n_joints] (the angle the next
+        tick's P-controller uses), joint_speed float32[n_joints], root float32[n, 6] (x, y, angle, vx, vy, omega of body 0)
+        and ground int32[n_bodies] (1: touching terrain). Definitions: include/rem2d_control.h."""
+        self._require_control()
+        pop = self.pop
+        if pop is None:
+            raise Rem2dError("rem2d_read_observations: no population uploaded")
+        nc, nb = pop.n_creatures, pop.n_bodies
+        ob = dict(joint_angle=np.zeros(nb - nc, np.float32), joint_speed=np.zeros(nb - nc, np.float32),
+                  root=np.zeros((nc, 6), np.float32), ground=np.zeros(nb, np.int32))
+        v = Observation()
+        for k, a in ob.items():
+            setattr(v, k, a.ctypes.data)
+        self._check(self.lib.rem2d_read_observations(self.h, C.byref(v)), "rem2d_read_observations")
+        return ob

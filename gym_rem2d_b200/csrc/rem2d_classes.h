@@ -1,5 +1,5 @@
 // rem2d_classes.h — the launch interface of the three kernels (rem2d_kernels.cu; one translation unit per kernel so that
-// they compile in parallel, and one more for the episode kernel with statistics) and the host's per-class view of it. All classes run the SAME code: the class only selects a
+// they compile in parallel, one more for the episode kernel with statistics and one for the step kernel with joint targets) and the host's per-class view of it. All classes run the SAME code: the class only selects a
 // Layout (the capacity classes themselves are in rem2d_host_util.h).
 #pragma once
 #include <cuda_runtime.h>
@@ -16,6 +16,10 @@ int rem2d_episode_blocks_per_sm_stats(int image, int dyn_smem_bytes);
 void rem2d_launch_reset(const rem2d::Layout& L, int gs, int n_batches, cudaStream_t st, float* state, const int* lane_creature, rem2d::DevPop p);
 void rem2d_launch_step(const rem2d::Layout& L, int gs, int n_batches, cudaStream_t st, float* state, int n_ticks, const rem2d::Terrain* ter,
                        const rem2d::Consts* k, unsigned long long* counters);
+// the step kernel with caller-supplied joint targets (include/rem2d_control.h): targets[j] for global joint j, held for n_ticks
+void rem2d_launch_step_targets(const rem2d::Layout& L, int gs, int n_batches, cudaStream_t st, float* state, int n_ticks,
+                               const rem2d::Terrain* ter, const rem2d::Consts* k, unsigned long long* counters, const int* lane_creature,
+                               const int32_t* body_off, const double* targets);
 void rem2d_launch_episode(const rem2d::Layout& L, int image, int gs, int max_gs, int grid, cudaStream_t st, float* slots, const int* order, int n_order, int* queue,
                           rem2d::DevPop p, const rem2d::Terrain* ter, const rem2d::Consts* k, int max_ticks, double* fitness,
                           int* ticks, int* alive, int* status, unsigned long long* counters, ParkPolicy park, float* park_state,
@@ -42,6 +46,7 @@ struct ClassOps {
     }
     template <class... A> void reset(A... a) const { rem2d_launch_reset(L, a...); }
     template <class... A> void step(A... a) const { rem2d_launch_step(L, a...); }
+    template <class... A> void step_targets(A... a) const { rem2d_launch_step_targets(L, a...); }
     template <class... A> void episode(A... a) const { rem2d_launch_episode(L, a...); }
     template <class... A> void tail(A... a) const { rem2d_launch_tail(L, a...); }
 };

@@ -1,4 +1,4 @@
-// rem2d_cuda.cu — host side + C-ABI (include/rem2d.h, include/rem2d_stats.h) of the CUDA build, sm_100a only (kernels: rem2d_kernels.cu).
+// rem2d_cuda.cu — host side + C-ABI (include/rem2d.h, include/rem2d_stats.h, include/rem2d_control.h) of the CUDA build, sm_100a only (kernels: rem2d_kernels.cu).
 //
 // Sorts creatures into capacity classes (by body count), keeps one lane-interleaved state block per 32 creatures in
 // HBM, and runs every class on its own stream so small and large classes overlap on the 148 SMs: rem2d_step on a
@@ -18,6 +18,7 @@
 
 #include "rem2d_classes.h"
 #include "rem2d_host_util.h"
+#include "../../include/rem2d_control.h"
 
 using namespace rem2d;
 
@@ -49,6 +50,19 @@ __global__ void roots_kernel(const float* state, const int* __restrict__ lane_cr
     root_x[c] = g[(S_COUNT + BF_CX) * 32];
     wod[c] = __hiloint2double(__float_as_int(g[S_WOD_HI * 32]), __float_as_int(g[S_WOD_LO * 32]));
     alive[c] = __float_as_int(g[S_ALIVE * 32]);
+}
+
+// joint angles / joint speeds / root state / ground flags of every creature of a class -> table-indexed outputs
+// (rem2d_read_observations; rem2d::observe_column)
+__global__ void observations_kernel(const float* state, const int* __restrict__ lane_creature, int n_lanes, const __grid_constant__ Layout L,
+                                    const int32_t* __restrict__ body_off, float* joint_angle, float* joint_speed, float* root, int32_t* ground) {
+    int gl = blockIdx.x * blockDim.x + threadIdx.x;
+    if (gl >= n_lanes) return;
+    int c = lane_creature[gl];
+    if (c < 0) return;
+    const float* g = state + (size_t)(gl >> 5) * L.words * 32 + (gl & 31);
+    const int b0 = body_off[c], j0 = b0 - c;
+    observe_column(g, L, body_off[c + 1] - b0, joint_angle + j0, joint_speed + j0, root + (size_t)c * 6, ground + b0);
 }
 
 // FP32 issue-rate microbenchmark: 8 independent multiply / add chains per thread. The step kernel is built with
@@ -135,6 +149,7 @@ struct rem2d_handle {
     std::vector<int> creature_class, creature_lane;     // lane index within the class (batch*32+lane)
     Buf d_pop_mem[16];
     Buf b_results, b_roots;
+    Buf b_targets, b_obs;               // rem2d_step_targets / rem2d_read_observations (grow-only)
     DevPop dpop{};
     ClassState cls[N_CLASSES];
     double* d_fitness = nullptr; int *d_ticks = nullptr, *d_alive = nullptr, *d_status = nullptr;
@@ -204,6 +219,7 @@ static void release_buffers(rem2d_handle* h) {
     h->b_roots = Buf();
     if (h->b_stats.p) cudaFree(h->b_stats.p);
     h->b_stats = Buf();
+    for (Buf* b : {&h->b_targets, &h->b_obs}) { if (b->p) cudaFree(b->p); *b = Buf(); }
 }
 
 extern "C" {
@@ -730,21 +746,30 @@ static int gather(rem2d_handle* h) {
     return REM2D_OK;
 }
 
-extern "C" {
-
-int rem2d_step(rem2d_handle* h, int32_t n_ticks) {
-    if (!h) return REM2D_E_INVALID;
+// The stepping path: every class on its own stream, from the static creature -> column mapping. targets == nullptr: the sine
+// controllers (step_kernel); otherwise the host array of n_joints target angles (step_kernel_targets, include/rem2d_control.h).
+static int launch_step(rem2d_handle* h, int32_t n_ticks, const double* targets) {
     if (!h->have_pop || n_ticks < 0) { h->err = "step: no population / negative tick count"; return REM2D_E_INVALID; }
     if (!h->state_valid) { h->err = "step: per-creature state was consumed by rem2d_run_episodes/rem2d_evaluate; call rem2d_reset first"; return REM2D_E_INVALID; }
     cudaSetDevice(h->cfg.device);
     h->stats_valid = false;                      // the stepping path records no statistics
     CK(cudaEventRecord(h->ev_start, h->user_stream));
+    const double* d_targets = nullptr;
+    if (targets) {
+        CK(ensure(h->b_targets, sizeof(double) * (size_t)std::max(h->n_joints, 1)));
+        d_targets = (const double*)h->b_targets.p;
+        if (h->n_joints) CK(cudaMemcpyAsync(h->b_targets.p, targets, sizeof(double) * h->n_joints, cudaMemcpyHostToDevice, h->user_stream));
+    }
     int rc = fork_streams(h);
     if (rc) return rc;
     for (int k = N_CLASSES - 1; k >= 0; --k) {        // most expensive class first
         ClassState& cs = h->cls[k];
         if (!cs.n_batches) continue;
-        g_classes(k).step(step_group_shift(h->load, k, h->opt), cs.n_batches, cs.stream, cs.d_state, n_ticks, h->d_ter, h->d_consts, h->d_counters);
+        if (targets)
+            g_classes(k).step_targets(step_group_shift(h->load, k, h->opt), cs.n_batches, cs.stream, cs.d_state, n_ticks, h->d_ter, h->d_consts,
+                                      h->d_counters, cs.d_lane_creature, h->dpop.body_off, d_targets);
+        else
+            g_classes(k).step(step_group_shift(h->load, k, h->opt), cs.n_batches, cs.stream, cs.d_state, n_ticks, h->d_ter, h->d_consts, h->d_counters);
         h->launches++;
     }
     CK(cudaGetLastError());
@@ -754,6 +779,22 @@ int rem2d_step(rem2d_handle* h, int32_t n_ticks) {
     CK(cudaEventSynchronize(h->ev_stop));
     CK(cudaEventElapsedTime(&h->last_ms, h->ev_start, h->ev_stop));
     return REM2D_OK;
+}
+
+extern "C" {
+
+int rem2d_step(rem2d_handle* h, int32_t n_ticks) {
+    if (!h) return REM2D_E_INVALID;
+    return launch_step(h, n_ticks, nullptr);
+}
+
+int rem2d_step_targets(rem2d_handle* h, const double* targets, int32_t n_ticks) {
+    if (!h) return REM2D_E_INVALID;
+    if (!targets) { h->err = "step_targets: NULL targets"; return REM2D_E_INVALID; }
+    if (h->have_pop)
+        for (int j = 0; j < h->n_joints; ++j)
+            if (!std::isfinite(targets[j])) { h->err = "step_targets: target " + std::to_string(j) + " is not finite"; return REM2D_E_INVALID; }
+    return launch_step(h, n_ticks, targets);
 }
 
 int rem2d_fitness(rem2d_handle* h, double* out) {
@@ -942,6 +983,37 @@ int rem2d_read_roots(rem2d_handle* h, float* root_x, double* wod, int32_t* alive
     if (root_x) CK(cudaMemcpyAsync(root_x, d_x, sizeof(float) * h->n_creatures, cudaMemcpyDeviceToHost, h->user_stream));
     if (wod) CK(cudaMemcpyAsync(wod, d_wod, sizeof(double) * h->n_creatures, cudaMemcpyDeviceToHost, h->user_stream));
     if (alive) CK(cudaMemcpyAsync(alive, d_alive, sizeof(int) * h->n_creatures, cudaMemcpyDeviceToHost, h->user_stream));
+    CK(cudaStreamSynchronize(h->user_stream));
+    return REM2D_OK;
+}
+
+int rem2d_read_observations(rem2d_handle* h, rem2d_observation* out) {
+    if (!h || !out) return REM2D_E_INVALID;
+    if (!h->have_pop) { h->err = "read_observations: no population uploaded"; return REM2D_E_INVALID; }
+    if (!h->state_valid) { h->err = "read_observations: per-creature state was consumed by rem2d_run_episodes; call rem2d_reset first"; return REM2D_E_INVALID; }
+    cudaSetDevice(h->cfg.device);
+    const size_t n = (size_t)h->n_creatures, nb = (size_t)h->n_bodies, nj = (size_t)h->n_joints;
+    CK(ensure(h->b_obs, sizeof(float) * (2 * nj + 6 * n) + sizeof(int32_t) * nb + 64));
+    float* d_angle = (float*)h->b_obs.p;
+    float* d_speed = d_angle + nj;
+    float* d_root = d_speed + nj;
+    int32_t* d_ground = (int32_t*)(d_root + 6 * n);
+    for (int k = 0; k < N_CLASSES; ++k) {
+        ClassState& cs = h->cls[k];
+        if (!cs.n_batches) continue;
+        const int n_lanes = cs.n_batches * 32;
+        observations_kernel<<<(n_lanes + 127) / 128, 128, 0, h->user_stream>>>(cs.d_state, cs.d_lane_creature, n_lanes, g_classes(k).L,
+                                                                               h->dpop.body_off, d_angle, d_speed, d_root, d_ground);
+        h->launches++;
+    }
+    CK(cudaGetLastError());
+    auto copy = [&](void* dst, const void* src, size_t bytes) {
+        return dst && bytes ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, h->user_stream) : cudaSuccess;
+    };
+    CK(copy(out->joint_angle, d_angle, nj * sizeof(float)));
+    CK(copy(out->joint_speed, d_speed, nj * sizeof(float)));
+    CK(copy(out->root, d_root, 6 * n * sizeof(float)));
+    CK(copy(out->ground, d_ground, nb * sizeof(int32_t)));
     CK(cudaStreamSynchronize(h->user_stream));
     return REM2D_OK;
 }

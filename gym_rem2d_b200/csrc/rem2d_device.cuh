@@ -284,6 +284,28 @@ __host__ __device__ inline HotLayout make_hot_layout(const Layout& L, int gs) {
     return H;
 }
 
+// Observation of one creature at the end of a tick (include/rem2d_control.h, rem2d_read_observations) from its cold column g,
+// nb bodies: the outputs are already offset to the creature's first joint (joint_angle, joint_speed), its root row (root[6])
+// and its first body (ground). The values are those rem2d_read_state decodes from the same column.
+__device__ __forceinline__ void observe_column(const float* g, const Layout& L, int nb, float* joint_angle, float* joint_speed,
+                                               float* root, int32_t* ground) {
+    auto B = [&](int f, int i) { return g[(S_COUNT + i * BF_COUNT + f) * 32]; };
+    for (int j = 0; j < nb - 1; ++j) {
+        const int a = __float_as_int(g[(L.off_joint + j * JF_COUNT + JF_META) * 32]) & 0xff, b = j + 1;
+        joint_angle[j] = B(BF_A, b) - B(BF_A, a) - 0.0f;          // the currentAngle of Sim::tick_pre
+        joint_speed[j] = B(BF_W, b) - B(BF_W, a);
+    }
+    root[0] = B(BF_CX, 0); root[1] = B(BF_CY, 0); root[2] = B(BF_A, 0);
+    root[3] = B(BF_VX, 0); root[4] = B(BF_VY, 0); root[5] = B(BF_W, 0);
+    unsigned long long m = 0ull;                                   // bodies with a touching terrain contact
+    const int n_pool = __float_as_int(g[S_NC * 32]);
+    for (int q = 0; q < n_pool; ++q) {
+        const int key = __float_as_int(g[(L.off_cont + q * CF_COUNT + CF_KEY) * 32]);
+        if (((key >> 16) & 0xff) & CK_TOUCHING) m |= 1ull << (key & 0xff);
+    }
+    for (int b = 0; b < nb; ++b) ground[b] = (int32_t)((m >> b) & 1ull);
+}
+
 // One creature. All G lanes of the creature's group hold the same Sim (same cold column `g`, same hot column base `h`) and call
 // every member function TOGETHER; functions marked "leader" are executed by sub == 0 only and everything the other lanes need
 // afterwards is broadcast or read after a group barrier. With G == 1 the code degenerates to the sequential per-lane form.
@@ -319,6 +341,9 @@ public:
 #ifdef REM2D_STATS
     EpisodeStats st;          // where the statistics go, and the creature this group is ticking (set before every tick)
     int st_c;
+#endif
+#ifdef REM2D_TARGETS
+    const double* tgt;        // caller-supplied target angles of this creature's joints (step_kernel_targets, include/rem2d_control.h)
 #endif
 
     // ---- accessors
@@ -2145,11 +2170,16 @@ public:
             setSd(S_WOD_LO, wod);
         }
         for (int j = sub; j < nj; j += G) {
+#ifdef REM2D_TARGETS
+            // the controller output is the caller's target; the sine controller is not advanced (i_state unchanged)
+            const double out = tgt[j];
+#else
             double ist = Jd(JF_ISTATE, j) + Jd(JF_FREQ, j);
             setJd(JF_ISTATE, j, ist);
             double s, c;
             sincos_kernel(ist + (Jd(JF_PHASE, j) + 0.0), s, c);
             double out = Jd(JF_AMP, j) * s + Jd(JF_OFFS, j);
+#endif
             int a = Ji(JF_META, j) & 0xff, b = j + 1;
             float currentAngle = B(BF_A, b) - B(BF_A, a) - 0.0f;
             double speed = (out - (double)currentAngle) * k->p_gain;

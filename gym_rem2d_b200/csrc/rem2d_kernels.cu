@@ -2,13 +2,18 @@
 // kernel (-DREM2D_KERNEL_ID=0..2) so the translation units build in parallel; every capacity class and every group size runs the
 // same code with its own Layout and group shift (kernel parameters). REM2D_KERNEL_ID=3 compiles the episode kernel once more
 // with the episode statistics (REM2D_STATS): two more images, launched only by evaluations that record statistics, so that
-// the images of every other evaluation stay exactly what they are without them.
+// the images of every other evaluation stay exactly what they are without them. REM2D_KERNEL_ID=4 compiles the step kernel once
+// more with caller-supplied joint targets (REM2D_TARGETS, include/rem2d_control.h): step_kernel_targets, launched only by
+// rem2d_step_targets, so that step_kernel stays exactly what it is.
 //
 // Lane mapping (all kernels): a warp holds 32 >> gs creatures, each owned by a group of G = 1 << gs lanes (rem2d_device.cuh).
 // Cold state: blocks of 32 creature columns; creature column q lives in block q >> 5, column q & 31.
 #include <cstdlib>
 #if REM2D_KERNEL_ID == 3
 #define REM2D_STATS 1
+#endif
+#if REM2D_KERNEL_ID == 4
+#define REM2D_TARGETS 1
 #endif
 #include "rem2d_classes.h"
 
@@ -40,11 +45,22 @@ void rem2d_launch_reset(const Layout& L, int gs, int n_batches, cudaStream_t st,
 }
 #endif
 
-#if REM2D_KERNEL_ID == 1
-// Each group advances its creature by up to n_ticks ticks.
-__global__ void __launch_bounds__(32, 1) step_kernel(const __grid_constant__ Layout L, int gs, float* state, int n_ticks,
+#if REM2D_KERNEL_ID == 1 || REM2D_KERNEL_ID == 4
+#ifndef REM2D_TARGETS
+#define STEP_KERNEL step_kernel
+#else
+#define STEP_KERNEL step_kernel_targets
+#endif
+// Each group advances its creature by up to n_ticks ticks. The targets image takes the controller output of global joint j from
+// targets[j]; lane_creature and body_off locate the creature's first joint.
+__global__ void __launch_bounds__(32, 1) STEP_KERNEL(const __grid_constant__ Layout L, int gs, float* state, int n_ticks,
                                                      const Terrain* __restrict__ ter, const Consts* __restrict__ k,
-                                                     unsigned long long* counters) {
+                                                     unsigned long long* counters
+#ifdef REM2D_TARGETS
+                                                     , const int* __restrict__ lane_creature, const int32_t* __restrict__ body_off,
+                                                     const double* __restrict__ targets
+#endif
+                                                     ) {
     extern __shared__ float hot[];
     const int lane = threadIdx.x;
     const int q = blockIdx.x * (32 >> gs) + (lane >> gs);
@@ -55,6 +71,9 @@ __global__ void __launch_bounds__(32, 1) step_kernel(const __grid_constant__ Lay
 #pragma unroll
     for (int i = 0; i < REM2D_N_COUNTERS; ++i) sim.cnt.c[i] = 0u;
     sim.nb = sim.Si(S_NB); sim.nj = sim.nb - 1;
+#ifdef REM2D_TARGETS
+    if (sim.nb > 0) { const int c = lane_creature[q]; sim.tgt = targets + (body_off[c] - c); }   // (padding columns: nb = 0)
+#endif
 #ifdef REM2D_PHASE_TIMING
     for (int i = 0; i < REM2D_N_PHASES; ++i) sim.ph[i] = 0;
     sim.phase_t0 = clock64(); sim.phase_cur = PH_LOOP;
@@ -73,10 +92,19 @@ __global__ void __launch_bounds__(32, 1) step_kernel(const __grid_constant__ Lay
         if (lane == 0 && v) atomicAdd(&counters[i], v);
     }
 }
+#ifndef REM2D_TARGETS
 void rem2d_launch_step(const Layout& L, int gs, int n_batches, cudaStream_t st, float* state, int n_ticks, const Terrain* ter, const Consts* k,
                        unsigned long long* counters) {
     step_kernel<<<n_batches << gs, 32, make_hot_layout(L, gs).rows * 128, st>>>(L, gs, state, n_ticks, ter, k, counters);
 }
+#else
+void rem2d_launch_step_targets(const Layout& L, int gs, int n_batches, cudaStream_t st, float* state, int n_ticks, const Terrain* ter,
+                               const Consts* k, unsigned long long* counters, const int* lane_creature, const int32_t* body_off,
+                               const double* targets) {
+    step_kernel_targets<<<n_batches << gs, 32, make_hot_layout(L, gs).rows * 128, st>>>(L, gs, state, n_ticks, ter, k, counters, lane_creature,
+                                                                                        body_off, targets);
+}
+#endif
 #endif
 
 #if REM2D_KERNEL_ID == 2 || REM2D_KERNEL_ID == 3
@@ -284,18 +312,24 @@ void EPISODE_FN(rem2d_launch_tail)(const Layout& L, int image, int gs, int max_g
 cudaError_t rem2d_attr_step(int max_hot_bytes);
 cudaError_t rem2d_attr_episode(int max_hot_bytes);
 cudaError_t rem2d_attr_episode_stats(int max_hot_bytes);
+cudaError_t rem2d_attr_step_targets(int max_hot_bytes);
 #if REM2D_KERNEL_ID == 0
 cudaError_t rem2d_set_kernel_attributes(int max_hot_bytes) {
     cudaError_t e = rem2d_attr_step(max_hot_bytes);
     if (e != cudaSuccess) return e;
+    if ((e = rem2d_attr_step_targets(max_hot_bytes)) != cudaSuccess) return e;
     if ((e = rem2d_attr_episode(max_hot_bytes)) != cudaSuccess) return e;
     return rem2d_attr_episode_stats(max_hot_bytes);
 }
-#elif REM2D_KERNEL_ID == 1
+#elif REM2D_KERNEL_ID == 1 || REM2D_KERNEL_ID == 4
+#ifndef REM2D_TARGETS
 cudaError_t rem2d_attr_step(int max_hot_bytes) {
-    cudaError_t e = cudaFuncSetAttribute(step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes);
+#else
+cudaError_t rem2d_attr_step_targets(int max_hot_bytes) {
+#endif
+    cudaError_t e = cudaFuncSetAttribute(STEP_KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes);
     if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(step_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    return cudaFuncSetAttribute(STEP_KERNEL, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
 }
 #elif REM2D_KERNEL_ID == 2 || REM2D_KERNEL_ID == 3
 cudaError_t EPISODE_FN(rem2d_attr_episode)(int max_hot_bytes) {

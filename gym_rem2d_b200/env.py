@@ -59,16 +59,33 @@ class BatchedModular2D:
         self.table = table
         self.engine.upload(table)
 
-    def step(self, n_ticks=1):
+    def step(self, n_ticks=1, targets=None):
         """Advances every living creature by ``n_ticks`` ticks. Returns (reward, done) arrays formed like ``Modular2D.step``
         (Modular2DEnv.py:642-649): reward = root x, or -100 with done = True when the root is left of the origin or behind the
         wall of death. A creature whose episode ended with success (x > ENV_LENGTH) or at the step limit keeps reporting its
-        x — only the two death rules give -100, as in the reference."""
-        self.engine.step(n_ticks)
+        x — only the two death rules give -100, as in the reference.
+
+        ``targets`` (numpy array or CPU torch tensor of shape (n_joints,), radians, table joint order) drives every joint's
+        P-controller to its target for these ticks instead of the genome's sine oscillators, which pause
+        (``Engine.step_targets``; include/rem2d_control.h). ``observe()`` gives the feedback for the next call."""
+        if targets is None:
+            self.engine.step(n_ticks)
+        else:
+            if hasattr(targets, "detach"):            # torch tensor: host memory only
+                if targets.device.type != "cpu":
+                    raise ValueError("targets must be on the host (a numpy array or a CPU tensor)")
+                targets = targets.detach().numpy()
+            self.engine.step_targets(targets, n_ticks)
         x, wod, _alive = self.engine.read_roots()          # 16 bytes per creature, not the whole state block
         x = x.astype(np.float64)
         dead = (x < 0.0) | (wod > x)
         return np.where(dead, -100.0, x), dead
+
+    def observe(self):
+        """End-of-tick observations for closed-loop control: a dict of joint_angle float32[n_joints], joint_speed
+        float32[n_joints], root float32[n, 6] (x, y, angle, vx, vy, omega) and ground int32[n_bodies]
+        (``Engine.read_observations``)."""
+        return self.engine.read_observations()
 
     def fitness(self):
         return self.engine.fitness()
@@ -115,6 +132,8 @@ class Modular2D:
         return
 
     def step(self, action):
+        """Like the reference, ignores ``action``: the genome's controllers drive the joints (closed-loop control:
+        ``BatchedModular2D.step(targets=...)``)."""
         if self.tree_morphology is None:
             raise Exception("no tree_morphology")
         reward, done = self._batched.step(1)
