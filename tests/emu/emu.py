@@ -1,40 +1,41 @@
-"""ctypes handle on the CPU emulation of the CUDA device code (tests/emu/librem2d_emu.so). TEST INFRASTRUCTURE ONLY."""
+"""ctypes handle on the CPU emulation of the CUDA device code (tests/emu: librem2d_emu.so, and librem2d_emu_stats.so /
+librem2d_emu_targets.so for the statistics and joint-target variants). TEST INFRASTRUCTURE ONLY."""
 import ctypes as C
 import os
 import subprocess
 
 import numpy as np
 
+from gym_rem2d_b200 import constants as K
 from gym_rem2d_b200.capi import Config, Engine, Population, load_library, N_COUNTERS, COUNTER_NAMES
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB = os.path.join(HERE, "librem2d_emu.so")
+VARIANTS = {"plain": "librem2d_emu.so", "stats": "librem2d_emu_stats.so", "targets": "librem2d_emu_targets.so"}
+STATS = ("end_reason", "max_x", "joint_work", "airborne_ticks", "ground_ticks")
+OBS = ("joint_angle", "joint_speed", "root", "ground")
 
 
 class EmuOut(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("pose", "vel", "joint_impulse", "limit_state", "motor_speed", "alive", "ticks", "fitness",
-                                          "wod", "n_contacts", "n_touching", "touching_pairs", "touching_impulse")] + \
-               [("max_pairs", C.c_int32), ("sched_P", C.c_void_p), ("sched_smax", C.c_void_p), ("counters", C.c_void_p),
-                ("n_syncs", C.c_void_p)]
+                                          "wod", "n_contacts", "n_touching", "touching_pairs", "touching_impulse", "sched_P",
+                                          "sched_smax", "counters", "n_syncs", "status", "finish_gs", "gs_seq", "n_seq") + OBS + STATS] + \
+               [("max_pairs", C.c_int32), ("max_seq", C.c_int32)]
 
 
-def build():
-    subprocess.check_call(["make", "-s", "-C", HERE])
-    return LIB
+_libs = {}
 
 
-_lib = None
-
-
-def lib():
-    global _lib
-    if _lib is None:
-        _lib = C.CDLL(build())
-        _lib.rem2d_emu_run.argtypes = [C.POINTER(Population), C.c_void_p, C.c_int, C.c_double, C.POINTER(Config), C.c_int, C.c_int,
-                                       C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.POINTER(EmuOut)]
-        _lib.rem2d_emu_classes.argtypes = [C.c_void_p]
-        _lib.rem2d_emu_plan.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
-    return _lib
+def lib(variant="plain"):
+    if variant not in _libs:
+        subprocess.check_call(["make", "-s", "-C", HERE, VARIANTS[variant]])
+        L = C.CDLL(os.path.join(HERE, VARIANTS[variant]))
+        common = [C.POINTER(Population), C.c_void_p, C.c_int, C.c_double, C.POINTER(Config), C.c_int, C.c_int, C.c_int, C.c_int]
+        L.rem2d_emu_step.argtypes = common + [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.POINTER(EmuOut)]
+        L.rem2d_emu_queue.argtypes = common + [C.c_int, C.c_void_p, C.c_int, C.c_int, C.POINTER(EmuOut)]
+        L.rem2d_emu_classes.argtypes = [C.c_void_p]
+        L.rem2d_emu_plan.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+        _libs[variant] = L
+    return _libs[variant]
 
 
 _classes = None
@@ -82,34 +83,61 @@ def plan(members, work, options=None, max_ticks=10000, n_sms=148, max_warps_per_
                 **{k: cols[i].tolist() for i, k in enumerate(("gs", "grid", "grid2", "park_cap", "order", "step_gs"))})
 
 
-def run(pop, ys, step, creatures, gs, n_ticks, max_pairs=24, klass=None, **cfg_over):
-    """One emulated warp: `creatures` (<= 32 >> gs) of `pop`, reset + n_ticks ticks with groups of 1 << gs lanes."""
-    L = lib()
+def _run(entry, variant, pop, ys, terrain_step, klass, gs, cfg_over, max_pairs, args):
+    """Calls `entry` of the `variant` library on one warp. Every output is indexed like the table of `pop` (creature, body,
+    joint); the entries of creatures the warp did not run keep -1 (NaN for floats)."""
     binder = Engine.__new__(Engine)                      # only for _pop_struct (no native handle)
     s, keep = Engine._pop_struct(binder, pop)
     cfg = Config()
     load_library().rem2d_default_config(C.byref(cfg))
     for k, v in cfg_over.items():
         setattr(cfg, k, v)
-    creatures = np.ascontiguousarray(creatures, np.int32)
-    nbs = np.diff(pop.body_off)[creatures]
-    klass = klass or class_of(int(nbs.max()))
-    n, nb, nj = len(creatures), int(nbs.sum()), int(nbs.sum()) - len(creatures)
-    ys = np.ascontiguousarray(ys, np.float64)
-    st = dict(pose=np.zeros((nb, 3), np.float32), vel=np.zeros((nb, 3), np.float32), joint_impulse=np.zeros((nj, 4), np.float32),
-              limit_state=np.zeros(nj, np.int32), motor_speed=np.zeros(nj, np.float32), alive=np.zeros(n, np.int32),
-              ticks=np.zeros(n, np.int32), fitness=np.zeros(n, np.float64), wod=np.zeros(n, np.float64),
-              n_contacts=np.zeros(n, np.int32), n_touching=np.zeros(n, np.int32),
-              touching_pairs=np.full((n, max_pairs, 2), -1, np.int32), touching_impulse=np.zeros((n, max_pairs, 4), np.float32),
-              sched_P=np.zeros(n, np.int32), sched_smax=np.zeros(n, np.int32), counters=np.zeros(N_COUNTERS, np.uint64),
-              n_syncs=np.zeros(1, np.int64))
-    o = EmuOut()
+    n, nb, nj = pop.n_creatures, pop.n_bodies, pop.n_bodies - pop.n_creatures
+    shapes = dict(pose=((nb, 3), np.float32), vel=((nb, 3), np.float32), joint_impulse=((nj, 4), np.float32),
+                  limit_state=(nj, np.int32), motor_speed=(nj, np.float32), alive=(n, np.int32), ticks=(n, np.int32),
+                  fitness=(n, np.float64), wod=(n, np.float64), n_contacts=(n, np.int32), n_touching=(n, np.int32),
+                  touching_pairs=((n, max_pairs, 2), np.int32), touching_impulse=((n, max_pairs, 4), np.float32),
+                  sched_P=(n, np.int32), sched_smax=(n, np.int32), status=(n, np.int32), finish_gs=(n, np.int32),
+                  joint_angle=(nj, np.float32), joint_speed=(nj, np.float32), root=((n, 6), np.float32), ground=(nb, np.int32))
+    if variant == "stats":
+        shapes.update(end_reason=(n, np.int32), max_x=(n, np.float32), joint_work=(n, np.float64), airborne_ticks=(n, np.int32),
+                      ground_ticks=(nb, np.int32))
+    st = {k: np.full(shape, np.nan if np.dtype(dt).kind == "f" else -1, dt) for k, (shape, dt) in shapes.items()}
+    st.update(counters=np.zeros(N_COUNTERS, np.uint64), n_syncs=np.zeros(1, np.int64), gs_seq=np.zeros(64, np.int32),
+              n_seq=np.zeros(1, np.int32))
+    o = EmuOut(max_pairs=max_pairs, max_seq=len(st["gs_seq"]))
     for k, a in st.items():
         setattr(o, k, a.ctypes.data)
-    o.max_pairs = max_pairs
-    rc = L.rem2d_emu_run(C.byref(s), ys.ctypes.data, len(ys), float(step), C.byref(cfg), klass[0], klass[1], klass[2], gs,
-                         creatures.ctypes.data, n, int(n_ticks), C.byref(o))
+    ys = np.ascontiguousarray(ys, np.float64)
+    rc = getattr(lib(variant), entry)(C.byref(s), ys.ctypes.data, len(ys), float(terrain_step), C.byref(cfg), klass[0], klass[1],
+                                      klass[2], gs, *args, C.byref(o))
     if rc != 0:
-        raise RuntimeError("rem2d_emu_run failed: %d" % rc)
+        raise RuntimeError("%s (%s) failed: %d" % (entry, variant, rc))
     st["counters"] = dict(zip(COUNTER_NAMES, (int(v) for v in st["counters"])))
+    st["gs_seq"] = st.pop("gs_seq")[:int(st.pop("n_seq")[0])].tolist()
     return st
+
+
+def step(pop, ys, creatures, gs, n_ticks, variant="plain", targets=None, klass=None, terrain_step=K.TERRAIN_STEP, max_pairs=24,
+         **cfg_over):
+    """One emulated warp of the stepping kernel: `creatures` (<= 32 >> gs) of `pop`, a group of 1 << gs lanes each, reset and
+    then n_ticks ticks. variant "targets" takes targets[n_calls, n_joints of the table]: call i holds targets[i] for n_ticks
+    ticks, as rem2d_step_targets does. `klass` = (bodies, pool slots, staged contacts); the class of the largest creature by
+    default."""
+    creatures = np.ascontiguousarray(creatures, np.int32)
+    klass = klass or class_of(int(np.diff(pop.body_off)[creatures].max()))
+    n_calls, t = 1, None
+    if targets is not None:
+        t = np.ascontiguousarray(targets, np.float64)
+        n_calls = len(t)
+    return _run("rem2d_emu_step", variant, pop, ys, terrain_step, klass, gs, cfg_over, max_pairs,
+                (creatures.ctypes.data, len(creatures), None if t is None else t.ctypes.data, n_calls, int(n_ticks)))
+
+
+def queue(pop, ys, order, gs, max_gs, max_ticks, klass, variant="plain", terrain_step=K.TERRAIN_STEP, max_pairs=24, **cfg_over):
+    """One emulated warp of the queue-mode episode kernel, parking off: the creatures `order` of `pop` are pulled in that order
+    by groups of 1 << gs lanes, which widen up to max_gs as the warp drains. Each creature's outputs are its state at the end of
+    its episode; gs_seq lists the group shifts the warp ran at."""
+    order = np.ascontiguousarray(order, np.int32)
+    return _run("rem2d_emu_queue", variant, pop, ys, terrain_step, klass, gs, cfg_over, max_pairs,
+                (int(max_gs), order.ctypes.data, len(order), int(max_ticks)))

@@ -1,29 +1,29 @@
 """Closed-loop control of stepping runs (rem2d_step_targets / rem2d_read_observations, include/rem2d_control.h) on the CPU: the
-oracle with joint targets (tests/control_oracle) against plain oracle stepping and against the stated control rule, the frozen sine
-controllers, the observations against read_state, the call contract, the Python layer, and the device code of step_kernel_targets
-and of the observation gather (-DREM2D_TARGETS, through the emulation shim of tests/emu) against the oracle, bit for bit."""
+oracle with the extension headers (tests/oracle_ext) against plain oracle stepping and against the stated control rule, the
+frozen sine controllers, the observations against read_state, the call contract, the Python layer, and the device code of
+step_kernel_targets and of the observation gather (-DREM2D_TARGETS, the targets build of the emulation in tests/emu) against the
+oracle, bit for bit."""
 import ctypes as C
 import os
 import random
-import subprocess
 import sys
 
 import numpy as np
 import pytest
 
 from gym_rem2d_b200 import Individual, constants as K, terrain
-from gym_rem2d_b200.capi import Config, Engine, Observation, Population, Rem2dError, load_library
+from gym_rem2d_b200.capi import Observation, Rem2dError
 from gym_rem2d_b200.env import BatchedModular2D
 from gym_rem2d_b200.flatten import flatten_population
 from oracle.oracle import OracleEngine
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "emu"))
-sys.path.insert(0, os.path.join(HERE, "control_oracle"))
+sys.path.insert(0, os.path.join(HERE, "oracle_ext"))
 import emu  # noqa: E402
-from control_oracle import ControlOracleEngine, LIB as CONTROL_LIB  # noqa: E402
+import oracle_ext  # noqa: E402
+from oracle_ext import OracleExtEngine  # noqa: E402
 
-EMU_DIR = os.path.join(HERE, "control_emu")
 STATE = ("pose", "vel", "joint_impulse", "limit_state", "motor_speed", "alive", "ticks", "awake", "wod", "n_contacts",
          "n_touching", "touching_pairs", "touching_impulse")
 OBS = ("joint_angle", "joint_speed", "root", "ground")
@@ -79,7 +79,7 @@ def observations_from_state(pop, st):
 def test_sine_outputs_as_targets_reproduce_plain_stepping(enc):
     pop = population(enc, 64, 40 + len(enc))
     xs, ys = terrain.generate_terrain()
-    plain, ctl = engine(OracleEngine, ys, pop), engine(ControlOracleEngine, ys, pop)
+    plain, ctl = engine(OracleEngine, ys, pop), engine(OracleExtEngine, ys, pop)
     T = 150
     sine = ctl.sine_outputs(T)
     for t in range(T):
@@ -95,7 +95,7 @@ def test_sine_outputs_as_targets_reproduce_plain_stepping(enc):
 def test_the_control_rule():
     pop = population("lsystem", 64, 3)
     xs, ys = terrain.generate_terrain()
-    ctl = engine(ControlOracleEngine, ys, pop)
+    ctl = engine(OracleExtEngine, ys, pop)
     A, B = joints(pop)
     creature = np.repeat(np.arange(pop.n_creatures), np.diff(pop.body_off) - 1)
     rng = np.random.default_rng(0)
@@ -120,7 +120,7 @@ def test_sine_controllers_are_frozen_during_target_ticks():
     """A plain tick after k target ticks uses the sine output indexed by plain ticks only."""
     pop = population("ce", 48, 5)
     xs, ys = terrain.generate_terrain()
-    ctl = engine(ControlOracleEngine, ys, pop)
+    ctl = engine(OracleExtEngine, ys, pop)
     sine = ctl.sine_outputs(4)
     A, B = joints(pop)
     creature = np.repeat(np.arange(pop.n_creatures), np.diff(pop.body_off) - 1)
@@ -142,7 +142,7 @@ def test_sine_controllers_are_frozen_during_target_ticks():
 def test_sine_outputs_follow_plain_ticks_only():
     pop = population("direct", 32, 6)
     xs, ys = terrain.generate_terrain()
-    ctl = engine(ControlOracleEngine, ys, pop)
+    ctl = engine(OracleExtEngine, ys, pop)
     sine = ctl.sine_outputs(6)
     ctl.step(2)
     assert same(ctl.sine_outputs(4), sine[2:6])
@@ -156,7 +156,7 @@ def test_sine_outputs_follow_plain_ticks_only():
 def test_observations_equal_read_state(flat):
     pop = population("lsystem", 96, 8 + flat)
     xs, ys = terrain.flat_terrain() if flat else terrain.generate_terrain()
-    ctl = engine(ControlOracleEngine, ys, pop)
+    ctl = engine(OracleExtEngine, ys, pop)
     rng = np.random.default_rng(2)
     for t in range(60):
         if t % 3:
@@ -175,7 +175,7 @@ def test_contract():
     pop = population("direct", 16, 3)
     xs, ys = terrain.generate_terrain()
     nj = pop.n_bodies - pop.n_creatures
-    ctl = engine(ControlOracleEngine, ys)
+    ctl = engine(OracleExtEngine, ys)
     lib = ctl.lib
     zeros = np.zeros(nj)
     assert lib.rem2d_step_targets(ctl.h, zeros.ctypes.data, 1) != 0          # no population uploaded
@@ -233,9 +233,9 @@ def test_batched_env_takes_targets_and_observes():
     import torch
     random.seed(11)
     individuals = [Individual.random(encoding="lsystem") for _ in range(12)]
-    env = BatchedModular2D(lib_path=CONTROL_LIB)
+    env = BatchedModular2D(lib_path=oracle_ext.build())
     env.reset(individuals)
-    ref = ControlOracleEngine()
+    ref = OracleExtEngine()
     ref.set_terrain(env.terrain_y, K.TERRAIN_STEP)
     ref.upload(env.table)
     nj = env.table.n_bodies - env.table.n_creatures
@@ -257,50 +257,6 @@ def test_batched_env_takes_targets_and_observes():
 
 # ------------------------------------------------------------------ device code of step_kernel_targets on the CPU
 
-class EmuControlOut(C.Structure):
-    _fields_ = [(k, C.c_void_p) for k in ("fitness", "ticks", "alive", "pose", "vel", "joint_impulse", "motor_speed") + OBS +
-                ("counters",)]
-
-
-_elib = None
-
-
-def elib():
-    global _elib
-    if _elib is None:
-        subprocess.check_call(["make", "-s", "-C", EMU_DIR])
-        _elib = C.CDLL(os.path.join(EMU_DIR, "librem2d_emu_control.so"))
-        _elib.rem2d_emu_control_step.argtypes = [C.POINTER(Population), C.c_void_p, C.c_int, C.c_double, C.POINTER(Config), C.c_int,
-                                                 C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int,
-                                                 C.POINTER(EmuControlOut)]
-    return _elib
-
-
-def emu_control(pop, ys, klass, gs, creatures, targets, ticks_per_call):
-    """One emulated warp of step_kernel_targets: `creatures` (1 << gs lanes each) from tick 0, call i holding targets[i] (table
-    joint order) for ticks_per_call ticks. Returns the state and the observations indexed like the table."""
-    binder = Engine.__new__(Engine)
-    s, keep = Engine._pop_struct(binder, pop)
-    cfg = Config()
-    load_library().rem2d_default_config(C.byref(cfg))
-    n, nb, nj = pop.n_creatures, pop.n_bodies, pop.n_bodies - pop.n_creatures
-    out = dict(fitness=np.zeros(n), ticks=np.zeros(n, np.int32), alive=np.zeros(n, np.int32), pose=np.zeros((nb, 3), np.float32),
-               vel=np.zeros((nb, 3), np.float32), joint_impulse=np.zeros((nj, 4), np.float32), motor_speed=np.zeros(nj, np.float32),
-               joint_angle=np.zeros(nj, np.float32), joint_speed=np.zeros(nj, np.float32), root=np.zeros((n, 6), np.float32),
-               ground=np.zeros(nb, np.int32), counters=np.zeros(12, np.uint64))
-    o = EmuControlOut()
-    for k, a in out.items():
-        setattr(o, k, a.ctypes.data)
-    creatures = np.ascontiguousarray(creatures, np.int32)
-    targets = np.ascontiguousarray(targets, np.float64)
-    ys = np.ascontiguousarray(ys, np.float64)
-    rc = elib().rem2d_emu_control_step(C.byref(s), ys.ctypes.data, len(ys), float(K.TERRAIN_STEP), C.byref(cfg), klass[0], klass[1],
-                                       klass[2], gs, creatures.ctypes.data, len(creatures), targets.ctypes.data, len(targets),
-                                       int(ticks_per_call), C.byref(o))
-    assert rc == 0, rc
-    return out
-
-
 @pytest.fixture(scope="module")
 def lsystem_world():
     random.seed(5)
@@ -320,12 +276,12 @@ def test_emulated_targets_kernel_equals_the_oracle(lsystem_world, gs, ticks_per_
     rng = np.random.default_rng(gs * 10 + ticks_per_call)
     nj = pop.n_bodies - pop.n_creatures
     targets = rng.uniform(-np.pi / 2, np.pi / 2, (n_calls, nj))
-    r = emu_control(pop, ys, klass, gs, creatures, targets, ticks_per_call)
+    r = emu.step(pop, ys, creatures, gs, ticks_per_call, variant="targets", targets=targets, klass=klass)
     sub = pop.select(creatures)
     j0 = np.asarray(pop.body_off[:-1], np.int64) - np.arange(pop.n_creatures)
     jsel = np.concatenate([np.arange(j0[c], j0[c] + nbs[c] - 1) for c in creatures])
     bsel = np.concatenate([np.arange(pop.body_off[c], pop.body_off[c + 1]) for c in creatures])
-    o = engine(ControlOracleEngine, ys, sub)
+    o = engine(OracleExtEngine, ys, sub)
     for i in range(n_calls):
         o.step_targets(targets[i, jsel], ticks_per_call)
     st, ob = o.read_state(), o.read_observations()
@@ -338,4 +294,4 @@ def test_emulated_targets_kernel_equals_the_oracle(lsystem_world, gs, ticks_per_
         assert same(r[k][jsel], st[k]), (what, k)
     assert same(r["joint_angle"][jsel], ob["joint_angle"]) and same(r["joint_speed"][jsel], ob["joint_speed"]), what
     assert same(r["root"][creatures], ob["root"]) and same(r["ground"][bsel], ob["ground"]), what
-    assert dict(zip(o.counters(), (int(v) for v in r["counters"]))) == o.counters(), what
+    assert r["counters"] == o.counters(), what

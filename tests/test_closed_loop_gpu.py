@@ -1,5 +1,5 @@
 """Closed-loop control on the CUDA library (step_kernel_targets and observations_kernel) against the oracle with joint targets
-(tests/control_oracle), bit for bit: state, observations, fitness, ticks and counters, over three encodings, every forced group
+(tests/oracle_ext), bit for bit: state, observations, fitness, ticks and counters, over three encodings, every forced group
 shift, mixed plain and target calls, held targets, the 33-44-body class, sine outputs fed back as targets, and a 300-tick
 feedback loop over 4096 creatures. The fast library exports the functions and runs them. Needs a GPU; tests/test_closed_loop.py
 checks the oracle and the device code on the CPU."""
@@ -17,8 +17,8 @@ from gym_rem2d_b200.flatten import flatten_population
 from gym_rem2d_b200.population import random_population
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, os.path.join(HERE, "control_oracle"))
-from control_oracle import ControlOracleEngine  # noqa: E402
+sys.path.insert(0, os.path.join(HERE, "oracle_ext"))
+from oracle_ext import OracleExtEngine  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -35,7 +35,7 @@ def same(a, b):
 
 def pair(pop, ys, precision="exact", **options):
     g = Engine(device=0, precision=precision)
-    o = ControlOracleEngine(threads=THREADS)
+    o = OracleExtEngine(threads=THREADS)
     for e in (g, o):
         e.set_terrain(ys, K.TERRAIN_STEP)
     for k, v in options.items():
@@ -107,7 +107,7 @@ def test_sine_outputs_as_targets_reproduce_plain_stepping_on_cuda(enc):
     pop = flatten_population([Individual.random(encoding=enc) for _ in range(256)])
     xs, ys = terrain.generate_terrain()
     plain, ctl = Engine(device=0), Engine(device=0)
-    o = ControlOracleEngine()
+    o = OracleExtEngine()
     for e in (plain, ctl, o):
         e.set_terrain(ys, K.TERRAIN_STEP)
         e.upload(pop)
@@ -151,7 +151,7 @@ def test_batched_env_on_cuda():
     individuals = [Individual.random(encoding="lsystem") for _ in range(64)]
     env = BatchedModular2D(device=0)
     env.reset(individuals)
-    o = ControlOracleEngine()
+    o = OracleExtEngine()
     o.set_terrain(env.terrain_y, K.TERRAIN_STEP)
     o.upload(env.table)
     for t in range(40):

@@ -34,20 +34,20 @@ def oracle_state(sub, ys, step, n_ticks, **cfg):
 def check(sub, ys, gs, n_ticks, step=K.TERRAIN_STEP, **cfg):
     so, co, fo = oracle_state(sub, ys, step, n_ticks, **cfg)
     per = 32 >> gs
-    out = []
+    out, total = [], dict.fromkeys(co, 0)
     for first in range(0, sub.n_creatures, per):          # one emulated warp per `per` creatures
         idx = np.arange(first, min(first + per, sub.n_creatures))
-        se = emu.run(sub, ys, step, idx, gs, n_ticks, **cfg)
+        se = emu.step(sub, ys, idx, gs, n_ticks, terrain_step=step, **cfg)
         b0, b1 = sub.body_off[idx[0]], sub.body_off[idx[-1] + 1]
         j0, j1 = b0 - idx[0], b1 - idx[-1] - 1
         sl = {"pose": slice(b0, b1), "vel": slice(b0, b1), "joint_impulse": slice(j0, j1), "limit_state": slice(j0, j1),
               "motor_speed": slice(j0, j1)}
         for k in INT_KEYS + FLT_KEYS:
-            ref = so[k][sl.get(k, slice(idx[0], idx[-1] + 1))]
-            assert np.array_equal(se[k], ref), "gs=%d creatures %s: %s differs" % (gs, idx, k)
-        assert np.array_equal(se["fitness"], fo[idx])
-        out.append(se)
-    total = {k: sum(s["counters"][k] for s in out) for k in co}
+            s = sl.get(k, slice(idx[0], idx[-1] + 1))
+            assert np.array_equal(se[k][s], so[k][s]), "gs=%d creatures %s: %s differs" % (gs, idx, k)
+        assert np.array_equal(se["fitness"][idx], fo[idx])
+        out.append(se["sched_P"][idx])
+        total = {k: v + se["counters"][k] for k, v in total.items()}
     assert total == co
     return out
 
@@ -67,8 +67,8 @@ def test_every_group_size_matches_the_oracle_on_large_creatures(lsystem_pop, gs)
     out = check(sub, ys, gs, 45)
     if gs >= 2:
         # the schedule really pipelines: period well below the number of constraints of a 17-21 body creature
-        assert max(int(s["sched_P"].max()) for s in out) <= 8
-        assert min(int(s["sched_P"].min()) for s in out) >= 3
+        assert max(int(p.max()) for p in out) <= 8
+        assert min(int(p.min()) for p in out) >= 3
 
 
 @pytest.mark.parametrize("gs", [1, 2, 3])
@@ -107,7 +107,7 @@ def test_spilled_hot_contacts_fall_back_to_the_sequential_sweep():
     nbs = np.diff(pop.body_off)
     ok = np.nonzero(nbs >= 3)[0][:4]
     so, _, _ = oracle_state(pop.select(ok), ys, 0.15, 50)
-    se = emu.run(pop.select(ok), ys, 0.15, np.arange(len(ok)), 2, 50, klass=(12, 64, 1))
+    se = emu.step(pop.select(ok), ys, np.arange(len(ok)), 2, 50, klass=(12, 64, 1), terrain_step=0.15)
     for k in INT_KEYS + FLT_KEYS:
         assert np.array_equal(se[k], so[k]), k
     assert so["n_touching"].max() > 1

@@ -1,29 +1,26 @@
 """Episode statistics of whole-episode runs (rem2d_set_stats / rem2d_read_stats, include/rem2d_stats.h) on the CPU: the oracle
-with statistics (tests/stats_oracle) against the definitions recomputed from a stepping run of the plain oracle, every end
-reason, the call contract, and the device code of the statistics images (-DREM2D_STATS, through the emulation shim of
-tests/emu) against the oracle, bit for bit."""
+with the extension headers (tests/oracle_ext) against the definitions recomputed from a stepping run of the plain oracle, every
+end reason, the call contract, and the device code of the statistics images (-DREM2D_STATS, the statistics build of the
+emulation in tests/emu) against the oracle, bit for bit."""
 import ctypes as C
 import os
 import random
-import subprocess
 import sys
 
 import numpy as np
 import pytest
 
 from gym_rem2d_b200 import Individual, constants as K, terrain
-from gym_rem2d_b200.capi import (Config, Engine, Population, Rem2dError, load_library, END_RUNNING, END_ORIGIN, END_WALL, END_GOAL,
-                                 END_STEPS)
+from gym_rem2d_b200.capi import Rem2dError, END_RUNNING, END_ORIGIN, END_WALL, END_GOAL, END_STEPS
 from gym_rem2d_b200.flatten import flatten_population
 from oracle.oracle import OracleEngine
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "emu"))
-sys.path.insert(0, os.path.join(HERE, "stats_oracle"))
+sys.path.insert(0, os.path.join(HERE, "oracle_ext"))
 import emu  # noqa: E402
-from stats_oracle import StatsOracleEngine  # noqa: E402
+from oracle_ext import OracleExtEngine  # noqa: E402
 
-STATS_DIR = os.path.join(HERE, "stats_emu")
 NAMES = ("end_reason", "max_x", "joint_work", "airborne_ticks", "ground_ticks")
 ENCODINGS = ("direct", "lsystem", "ce", "cppn")
 
@@ -34,7 +31,7 @@ def population(enc, n, seed):
 
 
 def oracle(ys, stats=True, **cfg):
-    o = StatsOracleEngine(threads=8, **cfg)
+    o = OracleExtEngine(threads=8, **cfg)
     o.set_terrain(ys, K.TERRAIN_STEP)
     o.set_stats(stats)
     return o
@@ -184,10 +181,9 @@ def test_plain_oracle_has_no_statistics():
         o.set_stats(True)
 
 
-def test_contract():
-    pop = population("direct", 16, 3)
-    xs, ys = terrain.generate_terrain()
-    o = oracle(ys, stats=False)
+def check_contract(o, pop):
+    """The call contract of the statistics on engine `o`, terrain set, statistics off and nothing uploaded: the oracle's here,
+    the CUDA library's in tests/test_episode_stats_gpu.py."""
     with pytest.raises(Rem2dError):
         o.read_stats()                          # no population
     o.upload(pop)
@@ -211,6 +207,13 @@ def test_contract():
     assert np.array_equal(jw, full["joint_work"])
     o.run_episodes(200)
     assert_stats_equal(o.read_stats(), full, "re-run")
+    # the run consumed the per-creature state: stepping is refused and leaves the statistics readable
+    with pytest.raises(Rem2dError):
+        o.step(1)
+    with pytest.raises(Rem2dError):
+        o.step_targets(np.zeros(pop.n_bodies - pop.n_creatures), 1)
+    assert_stats_equal(o.read_stats(), full, "after a refused step")
+    o.reset()
     o.step(1)
     with pytest.raises(Rem2dError):
         o.read_stats()                          # the stepping path records none
@@ -224,51 +227,12 @@ def test_contract():
         o.read_stats()
 
 
+def test_contract():
+    xs, ys = terrain.generate_terrain()
+    check_contract(oracle(ys, stats=False), population("direct", 16, 3))
+
+
 # ------------------------------------------------------------------ device code of the statistics images on the CPU
-
-class EmuStatsOut(C.Structure):
-    _fields_ = [(k, C.c_void_p) for k in ("fitness", "ticks", "status") + NAMES]
-
-
-_slib = None
-
-
-def slib():
-    global _slib
-    if _slib is None:
-        subprocess.check_call(["make", "-s", "-C", STATS_DIR])
-        _slib = C.CDLL(os.path.join(STATS_DIR, "librem2d_emu_stats.so"))
-        common = [C.POINTER(Population), C.c_void_p, C.c_int, C.c_double, C.POINTER(Config), C.c_int, C.c_int, C.c_int, C.c_int]
-        _slib.rem2d_emu_stats_step.argtypes = common + [C.c_void_p, C.c_int, C.c_int, C.POINTER(EmuStatsOut)]
-        _slib.rem2d_emu_stats_queue.argtypes = common + [C.c_int, C.c_void_p, C.c_int, C.c_int, C.POINTER(EmuStatsOut)]
-    return _slib
-
-
-def emu_stats(entry, pop, ys, klass, gs, creatures, n_ticks, max_gs=None):
-    """Runs one emulated warp of the statistics image: entry "step" (creatures from tick 0, 1 << gs lanes each) or "queue"
-    (queue-mode episode loop with regrouping up to max_gs). Returns fitness, ticks and the statistics, indexed by creature
-    (ground_ticks by body)."""
-    binder = Engine.__new__(Engine)
-    s, keep = Engine._pop_struct(binder, pop)
-    cfg = Config()
-    load_library().rem2d_default_config(C.byref(cfg))
-    n = pop.n_creatures
-    out = dict(fitness=np.zeros(n), ticks=np.zeros(n, np.int32), status=np.zeros(n, np.int32), end_reason=np.zeros(n, np.int32),
-               max_x=np.zeros(n, np.float32), joint_work=np.zeros(n), airborne_ticks=np.zeros(n, np.int32),
-               ground_ticks=np.zeros(pop.n_bodies, np.int32))
-    o = EmuStatsOut()
-    for k, a in out.items():
-        setattr(o, k, a.ctypes.data)
-    creatures = np.ascontiguousarray(creatures, np.int32)
-    ys = np.ascontiguousarray(ys, np.float64)
-    args = (C.byref(s), ys.ctypes.data, len(ys), float(K.TERRAIN_STEP), C.byref(cfg), klass[0], klass[1], klass[2], gs)
-    if entry == "step":
-        rc = slib().rem2d_emu_stats_step(*args, creatures.ctypes.data, len(creatures), int(n_ticks), C.byref(o))
-    else:
-        rc = slib().rem2d_emu_stats_queue(*args, int(max_gs), creatures.ctypes.data, len(creatures), int(n_ticks), C.byref(o))
-    assert rc == 0, rc
-    return out
-
 
 def subset(stats, pop, creatures):
     """The statistics of `creatures` only (ground_ticks of their bodies)."""
@@ -293,7 +257,7 @@ def test_emulated_stepping_entry_equals_the_oracle(world, gs):
     nbs = np.diff(pop.body_off)
     creatures = np.nonzero((nbs >= 3) & (nbs <= 22))[0][7 * gs:7 * gs + (32 >> gs)]
     n_ticks = 300
-    r = emu_stats("step", pop, ys, klass, gs, creatures, n_ticks)
+    r = emu.step(pop, ys, creatures, gs, n_ticks, variant="stats", klass=klass)
     o = oracle(ys)
     fc, tc = o.evaluate(pop.select(creatures), n_ticks)
     assert np.array_equal(r["ticks"][creatures], tc) and np.array_equal(r["fitness"][creatures], fc)
@@ -307,6 +271,6 @@ def test_emulated_queue_with_regrouping_equals_the_oracle(world, nb):
     nbs = np.diff(pop.body_off)
     fit = np.nonzero((nbs >= 3) & (nbs <= nb))[0]
     order = fit[np.argsort(-nbs[fit], kind="stable")][:40]          # the largest creatures of the class first, as the host queues
-    r = emu_stats("queue", pop, ys, klass, 0, order, K.EVALUATION_STEPS, max_gs=klass[3])
+    r = emu.queue(pop, ys, order, 0, klass[3], K.EVALUATION_STEPS, klass, variant="stats")
     assert np.array_equal(r["ticks"][order], to[order]) and np.array_equal(r["fitness"][order], fo[order])
     assert_stats_equal(subset(r, pop, order), subset(so, pop, order), "NB %d" % nb)

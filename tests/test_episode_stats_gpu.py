@@ -1,7 +1,8 @@
 """Episode statistics of the CUDA library (the statistics images of the episode kernel) against the oracle, bit for bit, under
 every execution strategy: bulk and warp mode, parking and tail launches, forced group widths, refill rounds, the overflow wave,
 the 128-register image, re-runs after a capacity overflow and regrouping of draining warps (reference: the oracle with
-statistics, tests/stats_oracle). Statistics never change results, in the exact and in the fast build. Needs a GPU; tests/test_episode_stats.py checks the oracle and the device code on the CPU."""
+statistics, tests/oracle_ext). Statistics never change results, in the exact and in the fast build, and the call contract is the
+oracle's. Needs a GPU; tests/test_episode_stats.py checks the oracle and the device code on the CPU."""
 import os
 import random
 import sys
@@ -15,8 +16,9 @@ from gym_rem2d_b200.flatten import flatten_population
 from gym_rem2d_b200.population import random_population
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, os.path.join(HERE, "stats_oracle"))
-from stats_oracle import StatsOracleEngine  # noqa: E402
+sys.path.insert(0, os.path.join(HERE, "oracle_ext"))
+from oracle_ext import OracleExtEngine  # noqa: E402
+from tests.test_episode_stats import check_contract, population  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -32,7 +34,7 @@ def assert_stats_equal(a, b, what=""):
 
 
 def oracle_eval(pop, ys, max_ticks=K.EVALUATION_STEPS, step=K.TERRAIN_STEP):
-    o = StatsOracleEngine(threads=max(8, os.cpu_count() or 8))
+    o = OracleExtEngine(threads=max(8, os.cpu_count() or 8))
     o.set_terrain(ys, step)
     o.set_stats(True)
     f, t = o.evaluate(pop, max_ticks)
@@ -173,3 +175,12 @@ def test_python_interfaces():
     env2.evaluate(table=table)
     assert_stats_equal(env2.last_stats, so, "BatchedModular2D(stats=True)")
     env.close(); env2.close()
+
+
+def test_contract_equals_the_oracle():
+    """The statistics' call contract that tests/test_episode_stats.py checks on the oracle, on the CUDA library."""
+    xs, ys = terrain.generate_terrain()
+    g = Engine(device=0)
+    g.set_terrain(ys, K.TERRAIN_STEP)
+    check_contract(g, population("direct", 16, 3))
+    g.close()

@@ -1,11 +1,9 @@
-"""Regrouping of a draining episode warp, on the CPU emulation of the device code (tests/emu, tests/regroup_emu): once the class queue is empty,
-Sim::episodes (rem2d_device.cuh, the loop of the episode kernel) packs the surviving creatures of the warp into wider lane
-groups, up to the class's widest group shift. Results must equal the oracle bit for bit, and the work counters must be
-those of the creatures' whole episodes, also when a creature overflows its class after a regroup."""
-import ctypes as C
+"""Regrouping of a draining episode warp, on the CPU emulation of the device code (tests/emu, its queue entry): once the class
+queue is empty, Sim::episodes (rem2d_device.cuh, the loop of the episode kernel) packs the surviving creatures of the warp into
+wider lane groups, up to the class's widest group shift. Results must equal the oracle bit for bit, and the work counters must
+be those of the creatures' whole episodes, also when a creature overflows its class after a regroup."""
 import os
 import random
-import subprocess
 import sys
 
 import numpy as np
@@ -15,59 +13,8 @@ from gym_rem2d_b200 import Individual, constants as K, terrain
 from gym_rem2d_b200.flatten import flatten_population
 from oracle.oracle import OracleEngine
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, os.path.join(HERE, "emu"))
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "emu"))
 import emu  # noqa: E402
-from gym_rem2d_b200.capi import Config, Engine, Population, load_library, N_COUNTERS, COUNTER_NAMES  # noqa: E402
-
-QUEUE_DIR = os.path.join(HERE, "regroup_emu")
-
-
-class EmuQueueOut(C.Structure):
-    _fields_ = [(k, C.c_void_p) for k in ("fitness", "ticks", "alive", "status", "finish_gs", "counters", "gs_seq")] + \
-               [("max_seq", C.c_int32), ("n_seq", C.c_void_p)]
-
-
-_qlib = None
-
-
-def qlib():
-    global _qlib
-    if _qlib is None:
-        subprocess.check_call(["make", "-s", "-C", QUEUE_DIR])
-        _qlib = C.CDLL(os.path.join(QUEUE_DIR, "librem2d_emu_queue.so"))
-        _qlib.rem2d_emu_queue.argtypes = [C.POINTER(Population), C.c_void_p, C.c_int, C.c_double, C.POINTER(Config), C.c_int,
-                                          C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.POINTER(EmuQueueOut)]
-    return _qlib
-
-
-def emu_queue(pop, ys, step, order, gs, max_gs, max_ticks, klass):
-    """One emulated warp of the queue-mode episode kernel, parking off: the creatures `order` of `pop` are pulled in that order
-    by groups of 1 << gs lanes, which widen up to max_gs as the warp drains. `klass` = (bodies, pool slots, staged contacts).
-    Returns the per-creature fitness, ticks, alive, status and finishing group shift (indexed by creature; -1 / NaN for
-    creatures not in `order`), the work counters and the group shifts the warp ran at."""
-    binder = Engine.__new__(Engine)                      # only for _pop_struct (no native handle)
-    s, keep = Engine._pop_struct(binder, pop)
-    cfg = Config()
-    load_library().rem2d_default_config(C.byref(cfg))
-    order = np.ascontiguousarray(order, np.int32)
-    n = pop.n_creatures
-    st = dict(fitness=np.full(n, np.nan), ticks=np.full(n, -1, np.int32), alive=np.full(n, -1, np.int32),
-              status=np.full(n, -1, np.int32), finish_gs=np.full(n, -1, np.int32), counters=np.zeros(N_COUNTERS, np.uint64),
-              gs_seq=np.zeros(64, np.int32))
-    n_seq = np.zeros(1, np.int32)
-    o = EmuQueueOut()
-    for k, a in st.items():
-        setattr(o, k, a.ctypes.data)
-    o.max_seq, o.n_seq = len(st["gs_seq"]), n_seq.ctypes.data
-    ys = np.ascontiguousarray(ys, np.float64)
-    rc = qlib().rem2d_emu_queue(C.byref(s), ys.ctypes.data, len(ys), float(step), C.byref(cfg), klass[0], klass[1], klass[2], gs,
-                                max_gs, order.ctypes.data, len(order), int(max_ticks), C.byref(o))
-    if rc != 0:
-        raise RuntimeError("rem2d_emu_queue failed: %d" % rc)
-    st["counters"] = dict(zip(COUNTER_NAMES, (int(v) for v in st["counters"])))
-    st["gs_seq"] = st["gs_seq"][:int(n_seq[0])].tolist()
-    return st
 
 
 @pytest.fixture(scope="module")
@@ -90,7 +37,7 @@ def oracle_counters(pop, ys, creatures):
 
 def queue(world, order, gs, klass, max_gs=None):
     pop, ys, _, _ = world
-    return emu_queue(pop, ys, K.TERRAIN_STEP, order, gs, klass[3] if max_gs is None else max_gs, K.EVALUATION_STEPS, klass[:3])
+    return emu.queue(pop, ys, order, gs, klass[3] if max_gs is None else max_gs, K.EVALUATION_STEPS, klass[:3])
 
 
 @pytest.mark.parametrize("gs", [0, 2])
@@ -122,7 +69,7 @@ def test_counters_equal_the_stepping_entry(world):
     r = queue(world, order, 0, klass)
     total = {}
     for first in range(0, len(order), 32):
-        se = emu.run(pop, ys, K.TERRAIN_STEP, order[first:first + 32], 0, K.EVALUATION_STEPS, klass=klass[:3])
+        se = emu.step(pop, ys, order[first:first + 32], 0, K.EVALUATION_STEPS, klass=klass[:3])
         for k, v in se["counters"].items():
             total[k] = total.get(k, 0) + v
     assert r["counters"] == total
