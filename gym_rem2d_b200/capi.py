@@ -113,6 +113,8 @@ def load_library(path=None):
     if hasattr(lib, "rem2d_step_targets"):        # the closed-loop control extension (include/rem2d_control.h)
         lib.rem2d_step_targets.argtypes = [H, C.c_void_p, C.c_int32]
         lib.rem2d_read_observations.argtypes = [H, C.POINTER(Observation)]
+    if hasattr(lib, "rem2d_set_policy"):          # the feedback policy extension (include/rem2d_policy.h)
+        lib.rem2d_set_policy.argtypes = [H, C.c_void_p, C.c_int32, C.c_int32]
     _LIBS[path] = lib
     return lib
 
@@ -335,3 +337,23 @@ class Engine:
             setattr(v, k, a.ctypes.data)
         self._check(self.lib.rem2d_read_observations(self.h, C.byref(v)), "rem2d_read_observations")
         return ob
+
+    def set_policy(self, weights):
+        """Per-joint feedback policy for every later upload / evaluate (include/rem2d_policy.h): float64 weights of shape
+        (n_joints, 10 * H + 1), a numpy array or a CPU tensor, one row per joint in table order (gym_rem2d_b200.policy); None
+        clears it. The upload takes a snapshot; an upload with another joint count is refused while a policy is set."""
+        if not hasattr(self.lib, "rem2d_set_policy"):
+            raise Rem2dError("%s does not run feedback policies (include/rem2d_policy.h)" % self.backend)
+        if weights is None:
+            self._check(self.lib.rem2d_set_policy(self.h, None, 0, 0), "rem2d_set_policy")
+            return
+        from .policy import hidden_size
+        if hasattr(weights, "detach"):                # torch tensor: host memory only
+            if weights.device.type != "cpu":
+                raise ValueError("policy weights must be on the host (a numpy array or a CPU tensor)")
+            weights = weights.detach().numpy()
+        w = np.ascontiguousarray(weights, np.float64)
+        if w.ndim != 2:
+            raise ValueError("policy weights must have shape (n_joints, 10 * H + 1), got %s" % (w.shape,))
+        H = hidden_size(w.shape[1])
+        self._check(self.lib.rem2d_set_policy(self.h, _ptr(w), w.shape[0], H), "rem2d_set_policy")

@@ -1,4 +1,4 @@
-// rem2d_cuda.cu — host side + C-ABI (include/rem2d.h, include/rem2d_stats.h, include/rem2d_control.h) of the CUDA build, sm_100a only (kernels: rem2d_kernels.cu).
+// rem2d_cuda.cu — host side + C-ABI (include/rem2d.h, include/rem2d_stats.h, include/rem2d_control.h, include/rem2d_policy.h) of the CUDA build, sm_100a only (kernels: rem2d_kernels.cu).
 //
 // Sorts creatures into capacity classes (by body count), keeps one lane-interleaved state block per 32 creatures in
 // HBM, and runs every class on its own stream so small and large classes overlap on the 148 SMs: rem2d_step on a
@@ -19,6 +19,7 @@
 #include "rem2d_classes.h"
 #include "rem2d_host_util.h"
 #include "../../include/rem2d_control.h"
+#include "../../include/rem2d_policy.h"
 
 using namespace rem2d;
 
@@ -139,7 +140,14 @@ struct rem2d_handle {
     bool stats_on = false, upload_stats = false, stats_valid = false;
     Buf b_stats;
     EpisodeStats dstats{};
-    int warps_per_sm[4] = {};           // rem2d_episode_blocks_per_sm of the four episode images (plan_upload input)
+    // feedback policy (rem2d_set_policy): the caller's weights for later uploads, and the snapshot the current upload took on
+    // the device (selects the policy images for every run of that upload; the statistics then always point somewhere, b_stats)
+    std::vector<double> policy_w;
+    int policy_nj = 0, policy_hidden = 0;
+    bool policy_on = false, upload_policy = false;
+    Buf b_policy;
+    PolicyWeights dpolicy{};
+    int warps_per_sm[6] = {};           // rem2d_episode_blocks_per_sm of the six episode images (plan_upload input)
     int prio_high = 0;                  // greatest stream priority of the device (tail pool)
     int n_edges = 0;
     // population
@@ -219,7 +227,7 @@ static void release_buffers(rem2d_handle* h) {
     h->b_roots = Buf();
     if (h->b_stats.p) cudaFree(h->b_stats.p);
     h->b_stats = Buf();
-    for (Buf* b : {&h->b_targets, &h->b_obs}) { if (b->p) cudaFree(b->p); *b = Buf(); }
+    for (Buf* b : {&h->b_targets, &h->b_obs, &h->b_policy}) { if (b->p) cudaFree(b->p); *b = Buf(); }
 }
 
 extern "C" {
@@ -297,7 +305,7 @@ int rem2d_create(const rem2d_config* cfg, rem2d_handle** out) {
         for (int q = 0; q < N_CLASSES; ++q)
             for (int gs = 0; gs <= 5; ++gs) max_hot = std::max(max_hot, class_hot_bytes(q, gs));
         if ((e = rem2d_set_kernel_attributes(max_hot)) != cudaSuccess) return fail("cudaFuncSetAttribute", e);
-        for (int im = 0; im < 4; ++im) h->warps_per_sm[im] = std::max(1, rem2d_episode_blocks_per_sm(im, 1024));
+        for (int im = 0; im < 6; ++im) h->warps_per_sm[im] = std::max(1, rem2d_episode_blocks_per_sm(im, 1024));
         for (int im = 0; im < 2; ++im) h->load.max_warps_per_sm[im] = h->warps_per_sm[im];
     }
     *out = h;
@@ -372,6 +380,11 @@ static int launch_reset(rem2d_handle* h);
 static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_reset) {
     if (!h || !pop) return REM2D_E_INVALID;
     if (pop->n_creatures < 0 || pop->n_joints != pop->n_bodies - pop->n_creatures) { h->err = "upload: inconsistent counts"; return REM2D_E_INVALID; }
+    if (h->policy_on && pop->n_joints != h->policy_nj) {
+        h->err = "upload: the policy set with rem2d_set_policy has " + std::to_string(h->policy_nj) + " joints, the population " +
+                 std::to_string(pop->n_joints);
+        return REM2D_E_INVALID;
+    }
     cudaSetDevice(h->cfg.device);
     free_population(h);
     const int n = pop->n_creatures;
@@ -414,6 +427,14 @@ static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_res
     CK(upload_array(h, 12, pop->max_torque, nj, &h->dpop.max_torque));
     CK(upload_array(h, 13, pop->ctrl, nbod * 5, &h->dpop.ctrl));
     CK(upload_array(h, 14, (const uint8_t*)order.data(), nj, &h->dpop.joint_order));
+    // the policy's snapshot (rem2d_set_policy): later calls change h->policy_w, never this copy
+    h->upload_policy = h->policy_on;
+    if (h->upload_policy) {
+        CK(ensure(h->b_policy, sizeof(double) * std::max<size_t>(h->policy_w.size(), 1)));
+        if (!h->policy_w.empty())
+            CK(cudaMemcpyAsync(h->b_policy.p, h->policy_w.data(), sizeof(double) * h->policy_w.size(), cudaMemcpyHostToDevice, h->user_stream));
+        h->dpolicy = PolicyWeights{(const double*)h->b_policy.p, h->dpop.body_off, h->policy_hidden};
+    }
     // the pageable source buffers (order, caller arrays) must stay valid until the copies ran
     CK(cudaStreamSynchronize(h->user_stream));
     for (int k = 0; k < N_CLASSES; ++k) {
@@ -461,11 +482,11 @@ static int upload_impl(rem2d_handle* h, const rem2d_population* pop, bool do_res
         h->load.work[k] = 0.0;
         for (int c : members[k]) { int nbc = pop->body_off[c + 1] - pop->body_off[c]; h->load.work[k] += nbc == 1 ? 1.0 : 3.5 + nbc; }
     }
-    // statistics runs launch the statistics images: the planner sees their occupancy
+    // statistics runs launch the statistics images, policy runs the policy images: the planner sees their occupancy
     h->upload_stats = h->stats_on;
-    for (int im = 0; im < 2; ++im) h->load.max_warps_per_sm[im] = h->warps_per_sm[im + (h->upload_stats ? 2 : 0)];
+    for (int im = 0; im < 2; ++im) h->load.max_warps_per_sm[im] = h->warps_per_sm[im + (h->upload_policy ? 4 : h->upload_stats ? 2 : 0)];
     h->plan = plan_upload(h->load, h->opt);
-    if (h->upload_stats) {
+    if (h->upload_stats || h->upload_policy) {      // (the policy images always accumulate: without statistics into scratch)
         const size_t nn = (size_t)std::max(n, 1), nbod = (size_t)std::max(pop->n_bodies, 1);
         CK(ensure(h->b_stats, nn * (sizeof(double) + sizeof(float) + 2 * sizeof(int32_t)) + nbod * sizeof(int32_t) + 64));
         EpisodeStats& d = h->dstats;
@@ -526,8 +547,11 @@ static int launch_reset(rem2d_handle* h) {
 
 // Promotion: creatures that exceeded a capacity of their class (contact pool) are re-run from tick 0 on the refill
 // episode kernel of the next larger class until they fit. Rare (very fine terrains, pile-ups).
-// destinations of the episode statistics of the uploaded population (nullptr: it was uploaded with statistics off)
-static const EpisodeStats* stats_dest(const rem2d_handle* h) { return h->upload_stats ? &h->dstats : nullptr; }
+// destinations of the episode statistics of the uploaded population (nullptr: it was uploaded with statistics off and without a
+// policy; the policy images accumulate them anyway, into b_stats, which read_stats then refuses)
+static const EpisodeStats* stats_dest(const rem2d_handle* h) { return h->upload_stats || h->upload_policy ? &h->dstats : nullptr; }
+// the policy of the uploaded population (nullptr: none)
+static const PolicyWeights* policy_of(const rem2d_handle* h) { return h->upload_policy ? &h->dpolicy : nullptr; }
 
 static int promote_overflowed(rem2d_handle* h, int max_ticks) {
     const int n = h->n_creatures;
@@ -563,7 +587,7 @@ static int promote_overflowed(rem2d_handle* h, int max_ticks) {
             CK(cudaMemsetAsync(d_queue, 0, sizeof(int), h->user_stream));
             g_classes(k).episode(h->plan.image, gs, widest_group_shift(k, gs), grid, h->user_stream, (float*)cs.b_redo_slots.p, d_order, (int)redo[k].size(), d_queue, h->dpop, h->d_ter,
                                  h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr, 0}, nullptr, nullptr, nullptr, stats_dest(h));
+                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr, 0}, nullptr, nullptr, nullptr, stats_dest(h), policy_of(h));
             h->launches++;
             CK(cudaGetLastError());
             CK(cudaStreamSynchronize(h->user_stream));      // redo[] (pageable source of the copy) goes out of scope
@@ -595,7 +619,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         if (lp.warp_mode) {      // queue mode with a whole warp per creature and one warp for every creature
             g_classes(k).episode(1, 5, 5, cs.n_members, cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop, h->d_ter,
                                  h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr, 0}, nullptr, nullptr, nullptr, stats_dest(h));
+                                 ParkPolicy{0, 0, 0.0f, 0, 0, 0, nullptr, nullptr, 0}, nullptr, nullptr, nullptr, stats_dest(h), policy_of(h));
             CK(cudaEventRecord(cs.t_end, cs.stream));
             h->launches++;
             continue;
@@ -615,7 +639,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         if (h->plan.grid2[k] > 0) { CK(cudaEventRecord(cs.done2, cs.stream)); CK(cudaStreamWaitEvent(cs.stream2, cs.done2, 0)); }   // queue / park counters are reset
         g_classes(k).episode(h->plan.image, h->plan.gs[k], widest_group_shift(k, h->plan.gs[k]), h->plan.grid[k], cs.stream, cs.d_state, cs.d_lane_creature, cs.n_members, cs.d_queue, h->dpop,
                              h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                             park, cs.d_park_state, cs.d_park_creature, cs.d_park_count, stats_dest(h));
+                             park, cs.d_park_state, cs.d_park_creature, cs.d_park_count, stats_dest(h), policy_of(h));
         // Nothing reads this copy, but it shapes the tail launches: without it the bench population gets twice the tail
         // launches and the second EA generation evaluates 40 % slower (3.1 s against 2.2 s; B200 at 1000 W).
         CK(cudaMemcpyAsync(cs.h_park_count, cs.d_park_count, sizeof(int), cudaMemcpyDeviceToHost, cs.stream));
@@ -632,7 +656,8 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
         const size_t first_block = ((size_t)h->plan.grid[k] * (32 >> gs) + 31) / 32;
         g_classes(k).episode(h->plan.image, gs, widest_group_shift(k, gs), h->plan.grid2[k], cs.stream2, cs.d_state + first_block * g_classes(k).words * 32, cs.d_lane_creature, cs.n_members,
                              cs.d_queue, h->dpop, h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status,
-                             h->d_counters, park_policy(k), cs.d_park_state, cs.d_park_creature, cs.d_park_count, stats_dest(h));
+                             h->d_counters, park_policy(k), cs.d_park_state, cs.d_park_creature, cs.d_park_count, stats_dest(h),
+                             policy_of(h));
         h->launches++;
     }
     CK(cudaGetLastError());
@@ -688,7 +713,7 @@ static int launch_episodes(rem2d_handle* h, int max_ticks) {
                     const int tail_gs = (cnt - launched[k] >= 32) ? std::min(3, h->opt.tail_group_shift) : h->opt.tail_group_shift;
                     g_classes(k).tail(h->plan.image, tail_gs, widest_group_shift(k, tail_gs), idle_stream(), cs.d_park_state, cs.d_park_creature, launched[k], cnt - launched[k],
                                       h->d_ter, h->d_consts, max_ticks, h->d_fitness, h->d_ticks, h->d_alive, h->d_status, h->d_counters,
-                                      trace ? (unsigned int*)cs.b_ttrace.p : nullptr, stats_dest(h));
+                                      trace ? (unsigned int*)cs.b_ttrace.p : nullptr, stats_dest(h), policy_of(h));
                     CK(cudaGetLastError());
                     h->launches++;
                     launched[k] = cnt;
@@ -747,7 +772,8 @@ static int gather(rem2d_handle* h) {
 }
 
 // The stepping path: every class on its own stream, from the static creature -> column mapping. targets == nullptr: the sine
-// controllers (step_kernel); otherwise the host array of n_joints target angles (step_kernel_targets, include/rem2d_control.h).
+// controllers (step_kernel), or the policy of a population uploaded with one (step_kernel_policy, include/rem2d_policy.h);
+// otherwise the host array of n_joints target angles (step_kernel_targets, include/rem2d_control.h), which overrides both.
 static int launch_step(rem2d_handle* h, int32_t n_ticks, const double* targets) {
     if (!h->have_pop || n_ticks < 0) { h->err = "step: no population / negative tick count"; return REM2D_E_INVALID; }
     if (!h->state_valid) { h->err = "step: per-creature state was consumed by rem2d_run_episodes/rem2d_evaluate; call rem2d_reset first"; return REM2D_E_INVALID; }
@@ -768,6 +794,9 @@ static int launch_step(rem2d_handle* h, int32_t n_ticks, const double* targets) 
         if (targets)
             g_classes(k).step_targets(step_group_shift(h->load, k, h->opt), cs.n_batches, cs.stream, cs.d_state, n_ticks, h->d_ter, h->d_consts,
                                       h->d_counters, cs.d_lane_creature, h->dpop.body_off, d_targets);
+        else if (h->upload_policy)
+            g_classes(k).step_policy(step_group_shift(h->load, k, h->opt), cs.n_batches, cs.stream, cs.d_state, n_ticks, h->d_ter, h->d_consts,
+                                     h->d_counters, cs.d_lane_creature, h->dpolicy);
         else
             g_classes(k).step(step_group_shift(h->load, k, h->opt), cs.n_batches, cs.stream, cs.d_state, n_ticks, h->d_ter, h->d_consts, h->d_counters);
         h->launches++;
@@ -952,6 +981,21 @@ int rem2d_read_stats(rem2d_handle* h, rem2d_episode_stats* out) {
     CK(copy(out->airborne_ticks, d.airborne_ticks, n * sizeof(int32_t)));
     CK(copy(out->ground_ticks, d.ground_ticks, nb * sizeof(int32_t)));
     CK(cudaStreamSynchronize(h->user_stream));
+    return REM2D_OK;
+}
+
+int rem2d_set_policy(rem2d_handle* h, const double* weights, int32_t n_joints, int32_t n_hidden) {
+    if (!h) return REM2D_E_INVALID;
+    if (!weights) { h->policy_on = false; h->policy_w.clear(); h->policy_nj = h->policy_hidden = 0; return REM2D_OK; }
+    if (n_hidden < 1 || n_hidden > REM2D_POLICY_MAX_HIDDEN || n_joints < 0) {
+        h->err = "set_policy: need 1 <= n_hidden <= 16 and n_joints >= 0";
+        return REM2D_E_INVALID;
+    }
+    const size_t n = (size_t)n_joints * (size_t)(10 * n_hidden + 1);
+    for (size_t i = 0; i < n; ++i)
+        if (!std::isfinite(weights[i])) { h->err = "set_policy: weight " + std::to_string(i) + " is not finite"; return REM2D_E_INVALID; }
+    h->policy_w.assign(weights, weights + n);
+    h->policy_nj = n_joints; h->policy_hidden = n_hidden; h->policy_on = true;
     return REM2D_OK;
 }
 

@@ -36,6 +36,7 @@ inline int atomicExch(int* p, int v) { return __atomic_exchange_n(p, v, __ATOMIC
 
 #include "../../include/rem2d.h"
 #include "../../include/rem2d_stats.h"
+#include "../../include/rem2d_policy.h"
 
 namespace rem2d {
 
@@ -244,6 +245,12 @@ struct EpisodeStats {
     const int32_t* body_off;
 };
 
+// Per-joint feedback policy (include/rem2d_policy.h), evaluated by the policy images only (-DREM2D_POLICY): the weights of global
+// joint j start at w + j * (10 * n_hidden + 1); body_off locates a creature's first joint (body_off[c] - c).
+struct PolicyWeights {
+    const double* w; const int32_t* body_off; int n_hidden;
+};
+
 // Capacities and section offsets of one capacity class. The layout is a RUN-TIME value (kernel parameter, i.e. constant
 // bank): all classes execute the SAME code image. With one template instantiation per class, warps of 7 different
 // 365 KB kernels shared each SM's instruction cache and every class ran 1.4-5x slower than alone (measured, DESIGN.md).
@@ -344,6 +351,11 @@ public:
 #endif
 #ifdef REM2D_TARGETS
     const double* tgt;        // caller-supplied target angles of this creature's joints (step_kernel_targets, include/rem2d_control.h)
+#endif
+#ifdef REM2D_POLICY
+    PolicyWeights pol;        // the population's policy, and the weights of this creature's first joint (set before every tick)
+    const double* __restrict__ pw;
+    __device__ __forceinline__ void set_policy_creature(int c) { pw = pol.w + (size_t)(pol.body_off[c] - c) * (10 * pol.n_hidden + 1); }
 #endif
 
     // ---- accessors
@@ -2169,6 +2181,19 @@ public:
             double wod = Sd(S_WOD_LO) + k->wod_speed;
             setSd(S_WOD_LO, wod);
         }
+#ifdef REM2D_POLICY
+        // the policy's inputs are the state at the start of the tick (rem2d_read_observations): first the bodies with a
+        // touching terrain contact, a mask over the pool (order-free, strided over the group)
+        unsigned long long ground = 0ull;
+        const int n_pool = Si(S_NC);
+        for (int q = sub; q < n_pool; q += G) {
+            const int key = Ci(CF_KEY, q);
+            if (key_flags(key) & CK_TOUCHING) ground |= 1ull << key_body(key);
+        }
+        for (int o = G >> 1; o > 0; o >>= 1) ground |= __shfl_xor_sync(gmask, ground, o);
+        const int H = pol.n_hidden, P = 10 * H + 1;
+        const double root_a = (double)B(BF_A, 0), root_vx = (double)B(BF_VX, 0), root_vy = (double)B(BF_VY, 0);
+#endif
         for (int j = sub; j < nj; j += G) {
 #ifdef REM2D_TARGETS
             // the controller output is the caller's target; the sine controller is not advanced (i_state unchanged)
@@ -2182,6 +2207,22 @@ public:
 #endif
             int a = Ji(JF_META, j) & 0xff, b = j + 1;
             float currentAngle = B(BF_A, b) - B(BF_A, a) - 0.0f;
+#ifdef REM2D_POLICY
+            {   // the joint's network (include/rem2d_policy.h): target = sine output + u, in this order of operations
+                const double* __restrict__ w = pw + (size_t)j * P;
+                const double x[REM2D_POLICY_FEATURES] = {out, (double)currentAngle, (double)(B(BF_W, b) - B(BF_W, a)),
+                                                         (double)((ground >> b) & 1ull), (double)((ground >> a) & 1ull),
+                                                         root_a, root_vx, root_vy};
+                double u = __ldg(w + 10 * H);
+                for (int k = 0; k < H; ++k) {
+                    double acc = __ldg(w + 8 * H + k);
+#pragma unroll
+                    for (int i = 0; i < REM2D_POLICY_FEATURES; ++i) acc = acc + __ldg(w + 8 * k + i) * x[i];
+                    u = u + __ldg(w + 9 * H + k) * (acc / (1.0 + fabs(acc)));
+                }
+                out = out + u;
+            }
+#endif
             double speed = (out - (double)currentAngle) * k->p_gain;
             set_awake(a, true); set_awake(b, true);       // (lanes may wake the same body: identical idempotent writes)
             J(JF_MSPEED, j) = (float)speed;
@@ -2348,6 +2389,9 @@ public:
             if (my >= 0) {                                            // group-uniform
 #ifdef REM2D_STATS
                 st_c = my;
+#endif
+#ifdef REM2D_POLICY
+                set_policy_creature(my);
 #endif
                 tick();
                 PHASE(PH_PARK);

@@ -4,7 +4,10 @@
 // with the episode statistics (REM2D_STATS): two more images, launched only by evaluations that record statistics, so that
 // the images of every other evaluation stay exactly what they are without them. REM2D_KERNEL_ID=4 compiles the step kernel once
 // more with caller-supplied joint targets (REM2D_TARGETS, include/rem2d_control.h): step_kernel_targets, launched only by
-// rem2d_step_targets, so that step_kernel stays exactly what it is.
+// rem2d_step_targets, so that step_kernel stays exactly what it is. REM2D_KERNEL_ID=5 compiles the episode kernel with the
+// per-joint feedback policy and the statistics (REM2D_POLICY, include/rem2d_policy.h): episode_kernel_policy and its
+// 128-register twin, launched only by evaluations of a population uploaded with a policy (with statistics off, the host points
+// the statistics at scratch); REM2D_KERNEL_ID=6 compiles the step kernel with the policy: step_kernel_policy.
 //
 // Lane mapping (all kernels): a warp holds 32 >> gs creatures, each owned by a group of G = 1 << gs lanes (rem2d_device.cuh).
 // Cold state: blocks of 32 creature columns; creature column q lives in block q >> 5, column q & 31.
@@ -14,6 +17,13 @@
 #endif
 #if REM2D_KERNEL_ID == 4
 #define REM2D_TARGETS 1
+#endif
+#if REM2D_KERNEL_ID == 5
+#define REM2D_STATS 1
+#define REM2D_POLICY 1
+#endif
+#if REM2D_KERNEL_ID == 6
+#define REM2D_POLICY 1
 #endif
 #include "rem2d_classes.h"
 
@@ -45,20 +55,26 @@ void rem2d_launch_reset(const Layout& L, int gs, int n_batches, cudaStream_t st,
 }
 #endif
 
-#if REM2D_KERNEL_ID == 1 || REM2D_KERNEL_ID == 4
-#ifndef REM2D_TARGETS
-#define STEP_KERNEL step_kernel
-#else
+#if REM2D_KERNEL_ID == 1 || REM2D_KERNEL_ID == 4 || REM2D_KERNEL_ID == 6
+#if defined(REM2D_TARGETS)
 #define STEP_KERNEL step_kernel_targets
+#elif defined(REM2D_POLICY)
+#define STEP_KERNEL step_kernel_policy
+#else
+#define STEP_KERNEL step_kernel
 #endif
 // Each group advances its creature by up to n_ticks ticks. The targets image takes the controller output of global joint j from
-// targets[j]; lane_creature and body_off locate the creature's first joint.
+// targets[j]; lane_creature and body_off locate the creature's first joint. The policy image locates the weights of the
+// creature's joints through lane_creature and the policy's body_off.
 __global__ void __launch_bounds__(32, 1) STEP_KERNEL(const __grid_constant__ Layout L, int gs, float* state, int n_ticks,
                                                      const Terrain* __restrict__ ter, const Consts* __restrict__ k,
                                                      unsigned long long* counters
 #ifdef REM2D_TARGETS
                                                      , const int* __restrict__ lane_creature, const int32_t* __restrict__ body_off,
                                                      const double* __restrict__ targets
+#endif
+#ifdef REM2D_POLICY
+                                                     , const int* __restrict__ lane_creature, const __grid_constant__ PolicyWeights pol
 #endif
                                                      ) {
     extern __shared__ float hot[];
@@ -73,6 +89,10 @@ __global__ void __launch_bounds__(32, 1) STEP_KERNEL(const __grid_constant__ Lay
     sim.nb = sim.Si(S_NB); sim.nj = sim.nb - 1;
 #ifdef REM2D_TARGETS
     if (sim.nb > 0) { const int c = lane_creature[q]; sim.tgt = targets + (body_off[c] - c); }   // (padding columns: nb = 0)
+#endif
+#ifdef REM2D_POLICY
+    sim.pol = pol;
+    if (sim.nb > 0) sim.set_policy_creature(lane_creature[q]);                                  // (padding columns: nb = 0)
 #endif
 #ifdef REM2D_PHASE_TIMING
     for (int i = 0; i < REM2D_N_PHASES; ++i) sim.ph[i] = 0;
@@ -92,22 +112,28 @@ __global__ void __launch_bounds__(32, 1) STEP_KERNEL(const __grid_constant__ Lay
         if (lane == 0 && v) atomicAdd(&counters[i], v);
     }
 }
-#ifndef REM2D_TARGETS
+#if REM2D_KERNEL_ID == 1
 void rem2d_launch_step(const Layout& L, int gs, int n_batches, cudaStream_t st, float* state, int n_ticks, const Terrain* ter, const Consts* k,
                        unsigned long long* counters) {
     step_kernel<<<n_batches << gs, 32, make_hot_layout(L, gs).rows * 128, st>>>(L, gs, state, n_ticks, ter, k, counters);
 }
-#else
+#elif REM2D_KERNEL_ID == 4
 void rem2d_launch_step_targets(const Layout& L, int gs, int n_batches, cudaStream_t st, float* state, int n_ticks, const Terrain* ter,
                                const Consts* k, unsigned long long* counters, const int* lane_creature, const int32_t* body_off,
                                const double* targets) {
     step_kernel_targets<<<n_batches << gs, 32, make_hot_layout(L, gs).rows * 128, st>>>(L, gs, state, n_ticks, ter, k, counters, lane_creature,
                                                                                         body_off, targets);
 }
+#else
+void rem2d_launch_step_policy(const Layout& L, int gs, int n_batches, cudaStream_t st, float* state, int n_ticks, const Terrain* ter,
+                              const Consts* k, unsigned long long* counters, const int* lane_creature, const PolicyWeights& pol) {
+    step_kernel_policy<<<n_batches << gs, 32, make_hot_layout(L, gs).rows * 128, st>>>(L, gs, state, n_ticks, ter, k, counters, lane_creature,
+                                                                                       pol);
+}
 #endif
 #endif
 
-#if REM2D_KERNEL_ID == 2 || REM2D_KERNEL_ID == 3
+#if REM2D_KERNEL_ID == 2 || REM2D_KERNEL_ID == 3 || REM2D_KERNEL_ID == 5
 // Whole episodes, two modes of ONE kernel (one code image: co-resident warps of both modes share the instruction cache).
 //
 // mode 0, queue: every group pulls the next creature of its class from a queue (big creatures first), builds its world in
@@ -178,6 +204,9 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
 #ifdef REM2D_STATS
                                                         , const EpisodeStats& stats
 #endif
+#ifdef REM2D_POLICY
+                                                        , const PolicyWeights& pol
+#endif
                                                         ) {
     extern __shared__ float hot[];
     const int lane = threadIdx.x;
@@ -187,6 +216,9 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
     sim.ter = ter; sim.k = k;
 #ifdef REM2D_STATS
     sim.st = stats; sim.st_c = -1;
+#endif
+#ifdef REM2D_POLICY
+    sim.pol = pol;
 #endif
 #pragma unroll
     for (int i = 0; i < REM2D_N_COUNTERS; ++i) sim.cnt.c[i] = 0u;
@@ -233,14 +265,14 @@ static __device__ __forceinline__ void episode_body(const Layout& L, int gs, int
                        int* park_count, int first_slot, int n_slots
 #define EPISODE_ARGS L, gs, max_gs, mode, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive, status, counters, park, park_state, \
                      park_creature, park_count, first_slot, n_slots
-#ifndef REM2D_STATS
+#if REM2D_KERNEL_ID == 2
 __global__ void __launch_bounds__(32, 1) episode_kernel(EPISODE_PARAMS) { episode_body(EPISODE_ARGS); }
 __global__ void __launch_bounds__(32, 16) episode_kernel_r128(EPISODE_PARAMS) { episode_body(EPISODE_ARGS); }
 #define EPISODE_IMAGE0 episode_kernel
 #define EPISODE_IMAGE1 episode_kernel_r128
 #define EPISODE_FN(name) name
 #define STATS_ARG
-#else
+#elif REM2D_KERNEL_ID == 3
 // the statistics images: the same code and register caps, the statistics' destinations as a trailing parameter
 __global__ void __launch_bounds__(32, 1) episode_kernel_stats(EPISODE_PARAMS, const __grid_constant__ EpisodeStats stats) {
     episode_body(EPISODE_ARGS, stats);
@@ -252,18 +284,38 @@ __global__ void __launch_bounds__(32, 16) episode_kernel_stats_r128(EPISODE_PARA
 #define EPISODE_IMAGE1 episode_kernel_stats_r128
 #define EPISODE_FN(name) name##_stats
 #define STATS_ARG , *stats
+#else
+// the policy images: the same code and register caps, the statistics' destinations and the policy as trailing parameters
+__global__ void __launch_bounds__(32, 1) episode_kernel_policy(EPISODE_PARAMS, const __grid_constant__ EpisodeStats stats,
+                                                               const __grid_constant__ PolicyWeights pol) {
+    episode_body(EPISODE_ARGS, stats, pol);
+}
+__global__ void __launch_bounds__(32, 16) episode_kernel_policy_r128(EPISODE_PARAMS, const __grid_constant__ EpisodeStats stats,
+                                                                     const __grid_constant__ PolicyWeights pol) {
+    episode_body(EPISODE_ARGS, stats, pol);
+}
+#define EPISODE_IMAGE0 episode_kernel_policy
+#define EPISODE_IMAGE1 episode_kernel_policy_r128
+#define EPISODE_FN(name) name##_policy
+#define STATS_ARG , *stats, *policy
 #endif
 
-// Launchers: stats == nullptr launches the images without statistics (kernel 2's unit), otherwise the statistics images
-// (kernel 3's unit), so that every launch of one evaluation uses the same image.
+// Launchers: policy != nullptr launches the policy images (kernel 5's unit; stats must then point somewhere), otherwise stats ==
+// nullptr launches the images without statistics (kernel 2's unit) and anything else the statistics images (kernel 3's unit), so
+// that every launch of one evaluation uses the same image.
 void EPISODE_FN(rem2d_launch_episode)(const Layout& L, int image, int gs, int max_gs, int grid, cudaStream_t st, float* slots, const int* order,
                                       int n_order, int* queue, DevPop p, const Terrain* ter, const Consts* k, int max_ticks, double* fitness,
                                       int* ticks, int* alive, int* status, unsigned long long* counters, ParkPolicy park, float* park_state,
-                                      int* park_creature, int* park_count, const EpisodeStats* stats) {
-#ifndef REM2D_STATS
+                                      int* park_creature, int* park_count, const EpisodeStats* stats, const PolicyWeights* policy) {
+#if REM2D_KERNEL_ID == 2
+    if (policy) {
+        rem2d_launch_episode_policy(L, image, gs, max_gs, grid, st, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive,
+                                    status, counters, park, park_state, park_creature, park_count, stats, policy);
+        return;
+    }
     if (stats) {
         rem2d_launch_episode_stats(L, image, gs, max_gs, grid, st, slots, order, n_order, queue, p, ter, k, max_ticks, fitness, ticks, alive,
-                                   status, counters, park, park_state, park_creature, park_count, stats);
+                                   status, counters, park, park_state, park_creature, park_count, stats, nullptr);
         return;
     }
 #endif
@@ -274,9 +326,10 @@ void EPISODE_FN(rem2d_launch_episode)(const Layout& L, int image, int gs, int ma
                                                 counters, park, park_state, park_creature, park_count, 0, 0 STATS_ARG);
 }
 // resident CTAs (= warps) of the episode kernel per SM for a given dynamic shared-memory size: registers AND shared memory.
-// image 0 / 1: the images without statistics, 2 / 3: the statistics images of the same register caps.
+// image 0 / 1: the images without statistics, 2 / 3: the statistics images, 4 / 5: the policy images of the same register caps.
 int EPISODE_FN(rem2d_episode_blocks_per_sm)(int image, int dyn_smem_bytes) {
-#ifndef REM2D_STATS
+#if REM2D_KERNEL_ID == 2
+    if (image >= 4) return rem2d_episode_blocks_per_sm_policy(image - 4, dyn_smem_bytes);
     if (image >= 2) return rem2d_episode_blocks_per_sm_stats(image - 2, dyn_smem_bytes);
 #endif
     int n = 0;
@@ -287,11 +340,17 @@ int EPISODE_FN(rem2d_episode_blocks_per_sm)(int image, int dyn_smem_bytes) {
 }
 void EPISODE_FN(rem2d_launch_tail)(const Layout& L, int image, int gs, int max_gs, cudaStream_t st, float* park_state, int* park_creature,
                                    int first_slot, int n_parked, const Terrain* ter, const Consts* k, int max_ticks, double* fitness, int* ticks,
-                                   int* alive, int* status, unsigned long long* counters, unsigned int* tail_trace, const EpisodeStats* stats) {
-#ifndef REM2D_STATS
+                                   int* alive, int* status, unsigned long long* counters, unsigned int* tail_trace, const EpisodeStats* stats,
+                                   const PolicyWeights* policy) {
+#if REM2D_KERNEL_ID == 2
+    if (policy) {
+        rem2d_launch_tail_policy(L, image, gs, max_gs, st, park_state, park_creature, first_slot, n_parked, ter, k, max_ticks, fitness, ticks,
+                                 alive, status, counters, tail_trace, stats, policy);
+        return;
+    }
     if (stats) {
         rem2d_launch_tail_stats(L, image, gs, max_gs, st, park_state, park_creature, first_slot, n_parked, ter, k, max_ticks, fitness, ticks,
-                                alive, status, counters, tail_trace, stats);
+                                alive, status, counters, tail_trace, stats, nullptr);
         return;
     }
 #endif
@@ -313,25 +372,31 @@ cudaError_t rem2d_attr_step(int max_hot_bytes);
 cudaError_t rem2d_attr_episode(int max_hot_bytes);
 cudaError_t rem2d_attr_episode_stats(int max_hot_bytes);
 cudaError_t rem2d_attr_step_targets(int max_hot_bytes);
+cudaError_t rem2d_attr_episode_policy(int max_hot_bytes);
+cudaError_t rem2d_attr_step_policy(int max_hot_bytes);
 #if REM2D_KERNEL_ID == 0
 cudaError_t rem2d_set_kernel_attributes(int max_hot_bytes) {
     cudaError_t e = rem2d_attr_step(max_hot_bytes);
     if (e != cudaSuccess) return e;
     if ((e = rem2d_attr_step_targets(max_hot_bytes)) != cudaSuccess) return e;
+    if ((e = rem2d_attr_step_policy(max_hot_bytes)) != cudaSuccess) return e;
     if ((e = rem2d_attr_episode(max_hot_bytes)) != cudaSuccess) return e;
-    return rem2d_attr_episode_stats(max_hot_bytes);
+    if ((e = rem2d_attr_episode_stats(max_hot_bytes)) != cudaSuccess) return e;
+    return rem2d_attr_episode_policy(max_hot_bytes);
 }
-#elif REM2D_KERNEL_ID == 1 || REM2D_KERNEL_ID == 4
-#ifndef REM2D_TARGETS
+#elif REM2D_KERNEL_ID == 1 || REM2D_KERNEL_ID == 4 || REM2D_KERNEL_ID == 6
+#if REM2D_KERNEL_ID == 1
 cudaError_t rem2d_attr_step(int max_hot_bytes) {
-#else
+#elif REM2D_KERNEL_ID == 4
 cudaError_t rem2d_attr_step_targets(int max_hot_bytes) {
+#else
+cudaError_t rem2d_attr_step_policy(int max_hot_bytes) {
 #endif
     cudaError_t e = cudaFuncSetAttribute(STEP_KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes);
     if (e != cudaSuccess) return e;
     return cudaFuncSetAttribute(STEP_KERNEL, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
 }
-#elif REM2D_KERNEL_ID == 2 || REM2D_KERNEL_ID == 3
+#elif REM2D_KERNEL_ID == 2 || REM2D_KERNEL_ID == 3 || REM2D_KERNEL_ID == 5
 cudaError_t EPISODE_FN(rem2d_attr_episode)(int max_hot_bytes) {
     cudaError_t e = cudaFuncSetAttribute(EPISODE_IMAGE0, cudaFuncAttributeMaxDynamicSharedMemorySize, max_hot_bytes);
     if (e != cudaSuccess) return e;

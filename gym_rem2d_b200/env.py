@@ -42,6 +42,7 @@ class BatchedModular2D:
         self.table = None
         self.stats = bool(stats)
         self._engine_stats = False
+        self._engine_policy = False
         self.last_stats = None
         self.seed(K.TERRAIN_SEED)
 
@@ -52,11 +53,20 @@ class BatchedModular2D:
         self.engine.set_terrain(self.terrain_y, K.TERRAIN_STEP)
         return [self._seed]
 
-    def reset(self, individuals=None, table=None, tree_depth=None):
-        """Builds one world per individual (genome.create -> flatten -> upload)."""
+    def _set_policy(self, policy):
+        """The policy of the next upload: the given weights, or none (open loop), clearing one set by an earlier call."""
+        if policy is not None or self._engine_policy:
+            self.engine.set_policy(policy)
+            self._engine_policy = policy is not None
+
+    def reset(self, individuals=None, table=None, tree_depth=None, policy=None):
+        """Builds one world per individual (genome.create -> flatten -> upload). ``policy``: float64 weights of a per-joint
+        feedback policy, shape (n_joints, 10 * H + 1) (``Engine.set_policy``; gym_rem2d_b200.policy); later ``step`` calls
+        without targets run it. None: the genome's open-loop sine controllers."""
         if table is None:
             table = flatten_population(individuals, tree_depth)
         self.table = table
+        self._set_policy(policy)
         self.engine.upload(table)
 
     def step(self, n_ticks=1, targets=None):
@@ -90,9 +100,11 @@ class BatchedModular2D:
     def fitness(self):
         return self.engine.fitness()
 
-    def evaluate(self, individuals=None, table=None, steps=K.EVALUATION_STEPS, tree_depth=None, stats=None):
+    def evaluate(self, individuals=None, table=None, steps=K.EVALUATION_STEPS, tree_depth=None, stats=None, policy=None):
         """Whole episodes for the whole population: float64 fitness per individual, as ``evaluate`` returns. ``stats``
-        (default: the constructor's) also records the episode statistics, left in ``last_stats``; they never change results."""
+        (default: the constructor's) also records the episode statistics, left in ``last_stats``; they never change results.
+        ``policy``: per-joint feedback policy weights for this population, shape (n_joints, 10 * H + 1) (``reset``); None:
+        open loop."""
         if table is None:
             table = flatten_population(individuals, tree_depth)
         self.table = table
@@ -100,6 +112,7 @@ class BatchedModular2D:
         if stats != self._engine_stats:
             self.engine.set_stats(stats)
             self._engine_stats = stats
+        self._set_policy(policy)
         fit, ticks = self.engine.evaluate(table, steps)
         self.last_ticks = ticks
         self.last_stats = self.engine.read_stats() if stats else None
@@ -191,13 +204,15 @@ def evaluate(individual, EVALUATION_STEPS=10000, HEADLESS=True, INTERVAL=100, EN
     return float(env.evaluate([individual], steps=EVALUATION_STEPS, tree_depth=TREE_DEPTH)[0])
 
 
-def evaluate_population(individuals, EVALUATION_STEPS=10000, TREE_DEPTH=None, env=None, as_torch=True, return_stats=False):
+def evaluate_population(individuals, EVALUATION_STEPS=10000, TREE_DEPTH=None, env=None, as_torch=True, return_stats=False,
+                        policy=None):
     """Batched evaluate: fitness of every individual (torch.float32 tensor on the host by default). With ``return_stats``,
     ``(fitness, stats)``: the episode statistics of ``Engine.read_stats`` (numpy arrays; ground_ticks per body of the
-    flattened table)."""
+    flattened table). ``policy``: per-joint feedback policy weights for the flattened population (``BatchedModular2D.reset``)."""
     env = env or getEnv()
     env.seed(K.TERRAIN_SEED)
-    fit = env.evaluate(individuals, steps=EVALUATION_STEPS, tree_depth=TREE_DEPTH, stats=True if return_stats else None)
+    fit = env.evaluate(individuals, steps=EVALUATION_STEPS, tree_depth=TREE_DEPTH, stats=True if return_stats else None,
+                       policy=policy)
     if as_torch:
         import torch
         fit = torch.from_numpy(fit.astype(np.float32))

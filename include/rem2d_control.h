@@ -1,7 +1,7 @@
 /* rem2d_control.h — closed-loop control of stepping runs: an extension of the C-ABI in rem2d.h.
  *
- * Exported by gym_rem2d_b200/csrc/librem2d_cuda.so (both precisions) and by the test oracle with joint targets
- * (tests/control_oracle/librem2d_oracle_control.so: the CPU oracle, unchanged, plus the two functions below).
+ * Exported by gym_rem2d_b200/csrc/librem2d_cuda.so (both precisions) and by the test oracle with the extension headers
+ * (tests/oracle_ext/librem2d_oracle_ext.so: the CPU oracle, unchanged, plus the two functions below).
  * The plain oracle (oracle/librem2d_oracle.so) exports rem2d.h only.
  *
  * rem2d_step_targets(h, targets, n_ticks):

@@ -1,7 +1,7 @@
 /* rem2d_stats.h — episode statistics of whole-episode runs: an extension of the C-ABI in rem2d.h.
  *
- * Exported by gym_rem2d_b200/csrc/librem2d_cuda.so (both precisions) and by the test oracle with statistics
- * (tests/stats_oracle/librem2d_oracle_stats.so: the CPU oracle, unchanged, plus the accumulation below after every tick).
+ * Exported by gym_rem2d_b200/csrc/librem2d_cuda.so (both precisions) and by the test oracle with the extension headers
+ * (tests/oracle_ext/librem2d_oracle_ext.so: the CPU oracle, unchanged, plus the accumulation below after every tick).
  * The plain oracle (oracle/librem2d_oracle.so) exports rem2d.h only.
  *
  * Every value is defined by the state at the end of a tick (after Collide, Solve, SolveTOI and the termination rule) as
